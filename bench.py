@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the BreaKmer per-target k-mer assembly hot path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload C2]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload C2] [--dump-outputs DIR]
 
 A "step" is one pass of the whole hot path (target.compare_kmers: k-mer counting, sample-only selection, read
 grouping, init_assembly) over the workload's regions.  The default workload is BASELINE.json configs[1], the
@@ -18,6 +18,9 @@ The default line also carries `c5_strong` and `c3_sharded`: the same measurement
 One JSON line is printed by rank 0.  `value` is whole-job regions/s with the inputs already resident in HBM; `e2e`
 is the same metric through the C-ABI calls bk_batch_submit / bk_batch_wait with HOST buffers (host->device copies and
 the result read-back inside the timed region).  Each rank drives its GPU from ONE host thread.
+
+--dump-outputs DIR writes what the last timed step of `value` returned as DIR/<name>.npy (see result_arrays).  The
+inputs are generated from fixed seeds, so two builds run with the same arguments can be compared file by file.
 """
 import argparse
 import json
@@ -26,6 +29,8 @@ import statistics
 import sys
 import threading
 import time
+
+import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
@@ -42,6 +47,7 @@ WORKLOADS = {
 METRIC = "target_regions_assembled_per_sec"
 UNIT = "regions/s"
 CALL_REGIONS = 2500          # regions per C-ABI call
+DUMP_LIMIT = 60 << 20        # bytes of --dump-outputs array data; with the .npy headers the files stay under 64 MB
 
 
 def config_dict(workload, world, regions_override=0):
@@ -525,6 +531,87 @@ def sharded_summary(D, workload, total, args, steps):
         run.close()
 
 
+def _segments(a, start, length):
+    """a[start[i]:start[i] + length[i]] for every i, concatenated"""
+    length = np.asarray(length, np.int64)
+    ends = np.cumsum(length)
+    if not len(ends) or not ends[-1]:
+        return a[:0]
+    return a[np.arange(ends[-1]) - np.repeat(ends - length - np.asarray(start, np.int64), length)]
+
+
+def result_arrays(outs, calls, packed, limit=DUMP_LIMIT):
+    """The results of one step ({call: batch.BatchOutput}) as flat float64 arrays, region by region in workload order.
+
+    Per region: `region` (index in the workload), `region_status`, `so_len` / `uniq_len` / `ctg_len` (its number of
+    sample-only k-mers, unique reads and contigs).  Per contig, in acceptance order: `ctg_seq_len`, `ctg_cnt_len`,
+    `ctg_reads_len`, `ctg_kmers_len`.  The payloads `so_mers`, `so_counts`, `uniq_rec`, `uniq_mult`, `ctg_seq`,
+    `ctg_kmer_locs`, `ctg_indel_only`, `ctg_others`, `ctg_reads`, `ctg_kmer_mer`, `ctg_kmer_pos`, `ctg_kmer_lth`,
+    `ctg_kmer_dist`, `ctg_kmer_order` follow in that order.  The library leaves contig payloads in completion order,
+    which changes from run to run; gathered in this order they do not.  Read indices count from the region's first
+    read, so they do not depend on how regions are packed into calls.  Every value is an integer below 2**53 (k-mer
+    codes need k <= 26), so float64 holds it exactly.  Above `limit` bytes, a fixed seeded sample of whole regions is
+    kept."""
+    items = []                                  # (region in the workload, call, region in the call, elements to write)
+    for c in sorted(outs):
+        o = outs[c]
+        per_ctg = 4 + 2 * o.seq_off[:, 1] + 2 * o.cnt_off[:, 1] + o.reads_off[:, 1] + 5 * o.kmers_off[:, 1]
+        cum = np.concatenate([[0], np.cumsum(per_ctg)])
+        size = 5 + 2 * np.diff(o.so_off) + 2 * np.diff(o.uniq_reg_off) + cum[o.ctg_reg_off[1:]] - cum[o.ctg_reg_off[:-1]]
+        items += [(calls[c][r], c, r, int(size[r])) for r in range(o.n_regions)]
+    items.sort()
+    elems = np.array([it[3] for it in items], np.int64)
+    if 8 * int(elems.sum()) > limit:
+        order = np.random.default_rng(0).permutation(len(items))
+        items = [items[i] for i in np.sort(order[np.cumsum(elems[order]) <= limit // 8])]
+    cols = {}
+
+    def add(name, a):
+        cols.setdefault(name, []).append(np.asarray(a))
+
+    for g, c, r, _n in items:
+        o, base = outs[c], int(packed[c].read_reg_off[r])
+        add("region", [g])
+        add("region_status", o.region_status[r:r + 1])
+        a, b = o.so_off[r], o.so_off[r + 1]
+        add("so_len", [b - a])
+        add("so_mers", o.so_mers[a:b])
+        add("so_counts", o.so_counts[a:b])
+        a, b = o.uniq_reg_off[r], o.uniq_reg_off[r + 1]
+        add("uniq_len", [b - a])
+        add("uniq_rec", o.uniq_rec[a:b].astype(np.int64) - base)
+        add("uniq_mult", o.uniq_mult[a:b])
+        cs = slice(o.ctg_reg_off[r], o.ctg_reg_off[r + 1])
+        add("ctg_len", [cs.stop - cs.start])
+        for name, tab in (("ctg_seq_len", o.seq_off), ("ctg_cnt_len", o.cnt_off), ("ctg_reads_len", o.reads_off),
+                          ("ctg_kmers_len", o.kmers_off)):
+            add(name, tab[cs, 1])
+        for name, arr, tab in (("ctg_seq", o.seq, o.seq_off), ("ctg_kmer_locs", o.kmer_locs, o.seq_off),
+                               ("ctg_indel_only", o.indel_only, o.cnt_off), ("ctg_others", o.others, o.cnt_off),
+                               ("ctg_reads", o.reads, o.reads_off), ("ctg_kmer_mer", o.kmer_mer, o.kmers_off),
+                               ("ctg_kmer_pos", o.kmer_pos, o.kmers_off), ("ctg_kmer_lth", o.kmer_lth, o.kmers_off),
+                               ("ctg_kmer_dist", o.kmer_dist, o.kmers_off), ("ctg_kmer_order", o.kmer_order, o.kmers_off)):
+            seg = _segments(arr, tab[cs, 0], tab[cs, 1])
+            add(name, seg.astype(np.int64) - base if name == "ctg_reads" else seg)
+    res = {}
+    for name, parts in cols.items():
+        a = np.concatenate(parts)
+        if a.size and int(a.max()) >= 1 << 53:
+            raise ValueError("%s: values from 2**53 up are not exact in float64" % name)
+        res[name] = a.astype(np.float64)
+    return res
+
+
+def dump_outputs(out_dir, run, prefix=""):
+    """--dump-outputs: the results of the last pass `run` timed, one .npy per array of result_arrays"""
+    from breakmer_b200 import batch
+    outs = {c: batch.BatchOutput(res, run.packed[c]) for c, (_j, res) in run.last.items()}
+    arrays = result_arrays(outs, run.calls, run.packed, DUMP_LIMIT // run.D.world)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, prefix + name + ".npy"), a)
+
+
 def gpu_arm(args):
     D = Dist(args)
     torch = D.torch
@@ -563,6 +650,8 @@ def gpu_arm(args):
     dev_s, wall_s = run.timed(args.steps, True, flush)
     host_resident = run.host_ms
     clocks = sampler.stop()
+    if args.dump_outputs:             # before any other call reuses the handles' result buffers
+        dump_outputs(args.dump_outputs, run, "rank%d_" % D.rank if D.world > 1 else "")
     rank_ms = D.gather_floats(1000.0 * run.last_local_dev_s / args.steps)
     calls_by_rank = [int(v) for v in D.gather_floats(float(run.items_run))]
     gpu_launches = 0
@@ -934,7 +1023,12 @@ def main():
     ap.add_argument("--no-dropin-leg", action="store_true")
     ap.add_argument("--no-extra-workloads", action="store_true", help="skip the c5_strong / c3_sharded keys")
     ap.add_argument("--extra-workloads", default="c5,c3", help="which of the two extra workloads to run (default both)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the results of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     if args.impl == "reference":

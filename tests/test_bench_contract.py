@@ -52,3 +52,94 @@ def test_gpu_arm_line():
     assert d["sharding_check"]["equal_to_single_gpu_run"] is True and d["sharding_check"]["regions"] == 60
     assert d["e2e_dropin"]["value"] > 0 and d["run"]["host_threads_per_rank"] == 1
     assert all(v["frac"] is None or v["frac"] >= 0 for v in d["roofline_per_kernel"].values())
+
+
+def _dumped_records(A, g, k):
+    """region g of result_arrays(...) -> (sample-only {mer: count}, unique records, contig records with region-local
+    read indices)"""
+    import numpy as np
+    from breakmer_b200 import _lib, batch
+    off = {n: np.concatenate([[0], np.cumsum(A[n + "_len"])]).astype(np.int64)
+           for n in ("so", "uniq", "ctg", "ctg_seq", "ctg_cnt", "ctg_reads", "ctg_kmers")}
+    i = list(A["region"]).index(g)
+    s = slice(off["so"][i], off["so"][i + 1])
+    only = dict(zip(_lib.codes_to_mers(A["so_mers"][s].astype(np.uint64), k), A["so_counts"][s].astype(int).tolist()))
+    s = slice(off["uniq"][i], off["uniq"][i + 1])
+    uniq = list(zip(A["uniq_rec"][s].astype(int).tolist(), A["uniq_mult"][s].astype(int).tolist()))
+    ctgs = []
+    for c in range(off["ctg"][i], off["ctg"][i + 1]):
+        sq, cn, rd, km = (slice(off[n][c], off[n][c + 1]) for n in ("ctg_seq", "ctg_cnt", "ctg_reads", "ctg_kmers"))
+        ctgs.append({"seq": A["ctg_seq"][sq].astype(np.uint8).tobytes().decode(),
+                     "indel_only": A["ctg_indel_only"][cn].astype(int).tolist(), "others": A["ctg_others"][cn].astype(int).tolist(),
+                     "reads": A["ctg_reads"][rd].astype(int).tolist(),
+                     "kmers": [list(t) for t in zip(_lib.codes_to_mers(A["ctg_kmer_mer"][km].astype(np.uint64), k),
+                                                    A["ctg_kmer_pos"][km].astype(int).tolist(),
+                                                    A["ctg_kmer_lth"][km].astype(int).tolist(),
+                                                    A["ctg_kmer_dist"][km].astype(int).tolist(),
+                                                    [batch.ORDER_NAMES[int(o)] for o in A["ctg_kmer_order"][km]])],
+                     "kmer_locs": A["ctg_kmer_locs"][sq].astype(int).tolist()})
+    return only, uniq, ctgs
+
+
+@pytest.mark.gpu
+def test_dumped_arrays_hold_the_batch_records():
+    """result_arrays (what --dump-outputs writes) decodes to the records the library returned, and does not depend on
+    how the regions were packed into calls; above its size limit it keeps the same seeded sample of whole regions"""
+    import bench
+    import numpy as np
+    from breakmer_b200 import _lib, batch, synth
+    regions = list(synth.config_regions("C2", 4, start=8)) + list(synth.config_regions("C5", 4, start=40))
+    calls = [[0, 2, 4, 6], [1, 3, 5, 7]]
+    h = _lib.Handle(0)
+    try:
+        packed = {c: batch.PackedBatch([regions[i] for i in calls[c]]) for c in range(2)}
+        outs = {c: batch.run(h, packed[c]) for c in range(2)}
+        A = bench.result_arrays(outs, calls, packed)
+        assert A["region"].tolist() == list(range(8)) and all(a.dtype == np.float64 for a in A.values())
+        for c in range(2):
+            o, pk = outs[c], packed[c]
+            for r, g in enumerate(calls[c]):
+                base = int(pk.read_reg_off[r])
+                a, b = o.uniq_reg_off[r], o.uniq_reg_off[r + 1]
+                only, uniq, ctgs = _dumped_records(A, g, pk.k)
+                assert only == o.sample_only(r)
+                assert uniq == list(zip((o.uniq_rec[a:b] - base).tolist(), o.uniq_mult[a:b].tolist()))
+                want = o.contig_records(r)
+                assert len(ctgs) == len(want)
+                for got, exp in zip(ctgs, want):
+                    assert sorted(pk.read_ids[base + i] for i in got.pop("reads")) == exp.pop("reads")
+                    assert got == exp
+        one = {0: batch.PackedBatch(regions)}
+        B = bench.result_arrays({0: batch.run(h, one[0])}, [list(range(8))], one)
+    finally:
+        h.close()
+    assert A.keys() == B.keys() and all(np.array_equal(A[n], B[n]) for n in A)
+    limit = sum(a.nbytes for a in A.values()) // 2
+    S = bench.result_arrays(outs, calls, packed, limit)
+    assert sum(a.nbytes for a in S.values()) <= limit and 0 < len(S["region"]) < 8
+    for g in S["region"].astype(int):
+        assert _dumped_records(S, g, 15) == _dumped_records(A, g, 15)
+    S2 = bench.result_arrays(outs, calls, packed, limit)
+    assert all(np.array_equal(S[n], S2[n]) for n in S)
+
+
+@pytest.mark.gpu
+def test_gpu_arm_dumps_the_outputs_of_its_last_step(tmp_path):
+    import bench
+    import numpy as np
+    from breakmer_b200 import _lib, batch, synth
+    d = _run(["--regions", "24", "--steps", "2", "--warmup", "3", "--no-cpu-baseline", "--no-ref-cache-leg", "--no-ingest-leg",
+              "--no-dropin-leg", "--dump-outputs", str(tmp_path)])
+    assert d["steps"] == 2
+    got = {fn[:-4]: np.load(os.path.join(str(tmp_path), fn)) for fn in os.listdir(str(tmp_path))}
+    assert sum(a.nbytes for a in got.values()) <= bench.DUMP_LIMIT
+    packed = {0: batch.PackedBatch(list(synth.config_regions("C2", 24)))}
+    h = _lib.Handle(0)
+    try:
+        want = bench.result_arrays({0: batch.run(h, packed[0])}, [list(range(24))], packed)
+    finally:
+        h.close()
+    assert got.keys() == want.keys()
+    for n in want:
+        assert got[n].dtype == np.float64 and np.array_equal(got[n], want[n]), n
+    assert got["ctg_len"].sum() > 0
