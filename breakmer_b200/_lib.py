@@ -104,6 +104,7 @@ def load():
                                    c_void_p, c_int64,
                                    POINTER(POINTER(c_uint64)), POINTER(POINTER(c_uint32)), POINTER(c_int64)]
     lib.bk_compare_kmers_batch.argtypes = [H, POINTER(BatchInput), POINTER(BatchResult)]
+    lib.bk_compare_kmers_long.argtypes = [H, POINTER(BatchInput), POINTER(BatchResult)]
     lib.bk_batch_submit.argtypes = [H, POINTER(BatchInput)]
     lib.bk_batch_wait.argtypes = [H, POINTER(BatchResult)]
     lib.bk_batch_upload.argtypes = [H, POINTER(BatchInput)]
@@ -129,8 +130,9 @@ def load():
                  "bk_write_sample_kmers"):
         getattr(lib, name).restype = c_int
     for name in ("bk_create", "bk_destroy", "bk_nw_batch", "bk_dedup_reads", "bk_count_kmers", "bk_sample_only",
-                 "bk_compare_kmers_batch", "bk_batch_submit", "bk_batch_wait", "bk_batch_upload", "bk_compare_kmers_resident", "bk_kernel_times",
-                 "bk_kernel_times_reset", "bk_set_option", "bk_ref_cache_build", "bk_ref_cache_clear"):
+                 "bk_compare_kmers_batch", "bk_compare_kmers_long", "bk_batch_submit", "bk_batch_wait", "bk_batch_upload",
+                 "bk_compare_kmers_resident", "bk_kernel_times", "bk_kernel_times_reset", "bk_set_option", "bk_ref_cache_build",
+                 "bk_ref_cache_clear"):
         getattr(lib, name).restype = c_int
     _lib = lib
     return lib
@@ -138,7 +140,7 @@ def load():
 
 EXPORTED_SYMBOLS = (
     "bk_version", "bk_device_count", "bk_create", "bk_destroy", "bk_last_error", "bk_nw_batch", "bk_dedup_reads",
-    "bk_count_kmers", "bk_sample_only", "bk_compare_kmers_batch", "bk_batch_submit", "bk_batch_wait", "bk_batch_upload", "bk_compare_kmers_resident", "bk_kernel_times",
+    "bk_count_kmers", "bk_sample_only", "bk_compare_kmers_batch", "bk_compare_kmers_long", "bk_batch_submit", "bk_batch_wait", "bk_batch_upload", "bk_compare_kmers_resident", "bk_kernel_times",
     "bk_kernel_times_reset", "bk_set_option", "bk_ref_cache_build", "bk_ref_cache_clear",
     "bk_ingest_create", "bk_ingest_destroy", "bk_ingest_last_error", "bk_ingest_buffers", "bk_ingest_files",
     "bk_write_contigs", "bk_write_sample_kmers")

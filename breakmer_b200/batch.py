@@ -14,6 +14,8 @@ import numpy as np
 from . import _lib
 
 ORDER_NAMES = ("for", "rev", "mid")
+MAX_LEN = 4095             # longest read / contig of bk_compare_kmers_batch's assembler
+LONG_MAX_LEN = 65535       # ... and of bk_compare_kmers_long's (run(..., long=True))
 
 
 def _concat(seqs):
@@ -195,10 +197,16 @@ class BatchOutput:
         return out
 
 
-def run(handle, packed, resident=False, decode=True):
-    """bk_compare_kmers_batch (or the resident variant after `upload`)."""
+def run(handle, packed, resident=False, decode=True, long=False):
+    """bk_compare_kmers_batch (or the resident variant after `upload`).  long=True: bk_compare_kmers_long, for regions
+    with reads or contigs above MAX_LEN (up to LONG_MAX_LEN) bases, which the batched call reports as BK_ERR_CAPACITY."""
     res = _lib.BatchResult()
-    if resident:
+    if long:
+        if resident:
+            raise ValueError("the long entry takes its inputs in the call (no resident form)")
+        s = packed.struct()
+        handle._check(handle.lib.bk_compare_kmers_long(handle.h, ctypes.byref(s), ctypes.byref(res)))
+    elif resident:
         handle._check(handle.lib.bk_compare_kmers_resident(handle.h, ctypes.byref(res)))
     else:
         s = packed.struct()

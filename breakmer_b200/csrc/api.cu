@@ -15,6 +15,7 @@
 #include "radix_sort.cuh"
 #include "scan.cuh"
 #include "pipeline.cuh"
+#include "assemble_long.cuh"
 #include "ingest.cuh"
 #include "dedup.cuh"
 
@@ -541,12 +542,12 @@ int bk_sample_only(bk_handle_t h, int k, const uint64_t* case_mers, const uint32
 }
 
 // On a failed submit the stream may hold work that uses the arenas: drain it so that the handle is reusable.
-static int submit_guarded(bk_handle_t h, const bk_batch_input* in) {
+static int submit_guarded(bk_handle_t h, const bk_batch_input* in, bool long_path = false) {
   if (h && h->pending.active) {                     // refused without touching the batch that is in flight
     h->err = "a batch is already in flight on this handle (call bk_batch_wait first)";
     return BK_ERR_ARG;
   }
-  const int rc = guarded(h, [&] { pipeline_submit(h, in); });
+  const int rc = guarded(h, [&] { pipeline_submit(h, in, long_path); });
   if (rc != BK_OK && h) { cudaStreamSynchronize(h->st); cudaGetLastError(); h->pending.active = false; }
   return rc;
 }
@@ -570,6 +571,12 @@ int bk_batch_wait(bk_handle_t h, bk_batch_result* out) {
 int bk_compare_kmers_batch(bk_handle_t h, const bk_batch_input* in, bk_batch_result* out) {
   if (h && (!in || !out)) { h->err = "bk_compare_kmers_batch: null argument"; return BK_ERR_ARG; }
   const int rc = submit_guarded(h, in);
+  return rc != BK_OK ? rc : wait_guarded(h, out);
+}
+
+int bk_compare_kmers_long(bk_handle_t h, const bk_batch_input* in, bk_batch_result* out) {
+  if (h && (!in || !out)) { h->err = "bk_compare_kmers_long: null argument"; return BK_ERR_ARG; }
+  const int rc = submit_guarded(h, in, true);
   return rc != BK_OK ? rc : wait_guarded(h, out);
 }
 

@@ -21,6 +21,9 @@
 #pragma once
 #include "common.cuh"
 #include "nw.cuh"
+#ifndef BK_SIM
+#include "nw_sweep.cuh"
+#endif
 
 namespace bk {
 
@@ -29,6 +32,33 @@ constexpr int ASM_BUF = 3 * ASM_CAP;   // gap buffers: data starts at ASM_CAP, m
 constexpr int ASM_KCAP = 2 * ASM_CAP;  // contig k-mer tuple list capacity
 constexpr int ASM_LASTCOL = ASM_CAP / 2 + 1;   // row pairs of one sweep
 constexpr int ORDER_FOR = 0, ORDER_REV = 1, ORDER_MID = 2;
+
+// Capacity of the state machine, a template argument of everything below that touches a contig.  BITS is the width of
+// a position in the packed keys: find_reads sorts [pos : BITS | CAP - 1 - len : BITS], m_first holds
+// [contig serial : 32 - BITS | CAP - 1 - window : BITS].
+//   AsmCap      assemble_kernel: reads and contigs up to 4,095 bases (the warp DP's limit, NW_MAX_LEN), contig and
+//               staged reads in shared memory, 2^20 contigs per region
+//   AsmCapLong  assemble_long_kernel: reads and contigs up to 65,535 bases, contig and staged read in global scratch,
+//               2^16 contigs per region
+struct AsmCap {
+  static constexpr int BITS = 12;
+  static constexpr int CAP = 1 << BITS;        // as ASM_CAP
+  static constexpr int MAX_LEN = CAP - 1;       // longest read / contig
+  static constexpr int BUF = 3 * CAP;           // as ASM_BUF
+  static constexpr int KCAP = 2 * CAP;          // as ASM_KCAP
+  static constexpr bool LONG = false;
+  using Key = int;
+};
+struct AsmCapLong {
+  static constexpr int BITS = 16;
+  static constexpr int CAP = 1 << BITS;
+  static constexpr int MAX_LEN = CAP - 1;
+  static constexpr int BUF = 3 * CAP;
+  static constexpr int KCAP = 2 * CAP;
+  static constexpr bool LONG = true;
+  using Key = unsigned;
+};
+constexpr int ASM_LONG_MAX_LEN = AsmCapLong::CAP - 1;                          // 65,535
 
 // Speculation width: the next ASM_SPEC_W reads of a contig's read stream are aligned
 // concurrently, one warp each (the CTA has up to ASM_SPEC_W warps per region; warp 0
@@ -104,7 +134,7 @@ struct AsmParams {
   uint8_t* m_used;                 // buffer.used_mers
   uint32_t* m_checked;             // contig serial in whose checked_kmers the mer is
   uint32_t* m_taken;               // finalize serial (check_alt_reads' mer_set)
-  uint32_t* m_first;               // [contig serial : 20 | 4095 - first window : 12] of the mer in the contig being emitted
+  uint32_t* m_first;               // [contig serial : 32 - BITS | CAP - 1 - first window : BITS] of the mer in the contig being emitted
   uint8_t* r_used;                 // fq_read.used
   uint8_t* r_deleted;              // key removed from fq_recs
   uint8_t* r_queued;               // 1: contig pending in buffer.contigs, 2: left it
@@ -117,7 +147,7 @@ struct AsmParams {
   int32_t* hit_u; int32_t* hit_pos; int32_t* hit2_u; int32_t* hit2_pos;
   uint64_t* sort_a; uint64_t* sort_b;  // size U each: sort buffers of find_reads
   int32_t* l_mused;                    // size S: list form of buffer.used_mers
-  // per-warp scratch, slot = global warp index
+  // per-warp scratch, slot = global warp index; sizes for AsmCap (AsmCapLong: the same formulas with its CAP)
   uint8_t* w_cseq;                 // ASM_BUF bytes
   int32_t* w_cnt;                  // 4 * ASM_BUF ints: io[2], ot[2]
   int32_t* w_K;                    // 4 * ASM_KCAP ints: s, x, meta, buffer coordinate of the window
@@ -223,7 +253,8 @@ BK_DEV bool window_code(const uint8_t* seq, int x, int k, uint64_t& code) {
   return ok;
 }
 
-struct RegionCtx {
+template <class T>
+struct RegionCtxT {
   const AsmParams* P;
   int region, k;
   // mers
@@ -256,6 +287,7 @@ struct RegionCtx {
   int2* edge_all;                 // ASM_SPEC_W x (2 * ASM_CAP) int2 or null
   uint2* lastcol;                 // warp 0's last-column scratch
   uint8_t* tab;                   // warp 0's score-table scratch
+  int32_t* nwl_diag;              // AsmCapLong: diagonals of the CTA's anti-diagonal sweep (nw_long.cuh), 9 * (CAP + 1) ints
   // contig under construction
   uint8_t* cseq; int c0, clen;
   int32_t* cnt_buf; int cur, k0, klen;
@@ -272,14 +304,15 @@ struct RegionCtx {
 #if defined(BK_PHASE_PROF) && !defined(BK_SIM)
   long long ph_cycles[PH_COUNT_];
 #endif
-  // staging (shared memory on the device)
+  // staging (shared memory on the device; global scratch in the long kernel)
   uint8_t* s_read; uint8_t* s_contig;
 
-  BK_DEV int32_t* io_vec(int which) const { return cnt_buf + (size_t)which * ASM_BUF; }
-  BK_DEV int32_t* ot_vec(int which) const { return cnt_buf + (size_t)(2 + which) * ASM_BUF; }
+  BK_DEV int32_t* io_vec(int which) const { return cnt_buf + (size_t)which * T::BUF; }
+  BK_DEV int32_t* ot_vec(int which) const { return cnt_buf + (size_t)(2 + which) * T::BUF; }
   BK_DEV int read_len_of(int u) const { return u_len[u]; }
   BK_DEV const uint8_t* read_ptr(int u) const { return P->rbases + P->roff[u_rec[u]]; }
 };
+using RegionCtx = RegionCtxT<AsmCap>;
 
 // lookup of a code in the region's ascending mer table; -1 if absent.  Regions with up
 // to MER_HASH_MAX mers use an open-addressed table in shared memory (entry =
@@ -289,7 +322,8 @@ constexpr int MER_HASH_MAX = 1400;
 BK_DEV unsigned mer_hash(uint64_t code) { return (unsigned)((code * 0x9E3779B97F4A7C15ull) >> 53); }        // 11 bits
 BK_DEV int mer_tag(uint64_t code) { return (int)((code * 0xC2B2AE3D27D4EB4Full) >> 49); }                 // 15 bits
 
-BK_DEV void build_mer_hash(RegionCtx& c) {
+template <class T>
+BK_DEV void build_mer_hash(RegionCtxT<T>& c) {
   c.hash_on = c.S > 0 && c.S <= MER_HASH_MAX;
   if (!c.hash_on) return;
   syncwarp();
@@ -304,7 +338,8 @@ BK_DEV void build_mer_hash(RegionCtx& c) {
   syncwarp();
 }
 
-BK_DEV int find_mer(const RegionCtx& c, uint64_t code) {
+template <class T>
+BK_DEV int find_mer(const RegionCtxT<T>& c, uint64_t code) {
   if (c.hash_on) {
     const int tag = mer_tag(code);
     unsigned slot = mer_hash(code);
@@ -327,7 +362,8 @@ BK_DEV int find_mer(const RegionCtx& c, uint64_t code) {
   return (lo < c.S && c.mer[lo] == code) ? lo : -1;
 }
 
-BK_DEV int stage_read(RegionCtx& c, int u) {
+template <class T>
+BK_DEV int stage_read(RegionCtxT<T>& c, int u) {
   const int n = c.read_len_of(u);
   const uint8_t* src = c.read_ptr(u);
   syncwarp();
@@ -335,7 +371,8 @@ BK_DEV int stage_read(RegionCtx& c, int u) {
   syncwarp();
   return n;
 }
-BK_DEV void sync_contig_to_smem(RegionCtx& c) {
+template <class T>
+BK_DEV void sync_contig_to_smem(RegionCtxT<T>& c) {
   syncwarp();
   for (int x = lane(); x < c.clen; x += WARP) c.s_contig[x] = c.cseq[c.c0 + x];
   syncwarp();
@@ -347,7 +384,8 @@ BK_DEV void sync_contig_to_smem(RegionCtx& c) {
 // pass A of every "which windows are live sample-only mers" question: lane l owns a
 // contiguous run of windows and rolls the 2-bit code along it (k loads for the first
 // window, one per further window); win[x] = local mer index or -1
-BK_DEV void lookup_windows(RegionCtx& c, const uint8_t* seq, int nwin, int32_t* win) {
+template <class T>
+BK_DEV void lookup_windows(RegionCtxT<T>& c, const uint8_t* seq, int nwin, int32_t* win) {
   const int k = c.k;
   const int per = (nwin + WARP - 1) / WARP;
   const int x0 = lane() * per;
@@ -374,14 +412,16 @@ BK_DEV void lookup_windows(RegionCtx& c, const uint8_t* seq, int nwin, int32_t* 
   syncwarp();
 }
 
-BK_DEV void append_kmers(RegionCtx& c, const uint8_t* seq, int base, int nlen, int order) {
+template <class T>
+BK_DEV void append_kmers(RegionCtxT<T>& c, const uint8_t* seq, int base, int nlen, int order) {
   const int k = c.k;
   const int nwin = nlen - k;              // range(0, len - l)
   if (nwin <= 0) return;
   BK_PH_BEGIN
   const int m = nlen / 2;
   const unsigned lt = lane_lt_mask();
-  int32_t* Ks = c.K; int32_t* Kx = c.K + ASM_KCAP; int32_t* Km = c.K + 2 * ASM_KCAP; int32_t* Kb = c.K + 3 * ASM_KCAP;
+  constexpr int KCAP = T::KCAP;
+  int32_t* Ks = c.K; int32_t* Kx = c.K + KCAP; int32_t* Km = c.K + 2 * KCAP; int32_t* Kb = c.K + 3 * KCAP;
   int32_t* win = reinterpret_cast<int32_t*>(c.wcode);
   lookup_windows(c, seq + base, nwin, win);
   // pass 0: ascending x over [lo0, hi0) ; pass 1: descending x over [lo1, hi1)
@@ -402,7 +442,7 @@ BK_DEV void append_kmers(RegionCtx& c, const uint8_t* seq, int base, int nlen, i
       const unsigned mk = ballot(sidx >= 0);
       if (sidx >= 0) {
         const int dst = c.nK + popc(mk & lt);
-        if (dst < ASM_KCAP) {
+        if (dst < KCAP) {
           Ks[dst] = sidx; Kx[dst] = x;
           const int lth = x < m ? 1 : 0, dist = x < m ? m - x : x - m;
           Km[dst] = lth | (order << 1) | (dist << 3);
@@ -412,25 +452,28 @@ BK_DEV void append_kmers(RegionCtx& c, const uint8_t* seq, int base, int nlen, i
       c.nK += popc(mk);
     }
   }
-  if (c.nK > ASM_KCAP) { c.nK = ASM_KCAP; c.status = ST_CAPACITY; }
+  if (c.nK > KCAP) { c.nK = KCAP; c.status = ST_CAPACITY; }
   syncwarp();
   BK_PH_END(c, PH_KMERS)
 }
 
-BK_DEV void set_kmers(RegionCtx& c) {                               // :548-550
+template <class T>
+BK_DEV void set_kmers(RegionCtxT<T>& c) {                               // :548-550
   c.ct_setup = true;
   c.nK = 0;
   append_kmers(c, c.s_contig, 0, c.clen, ORDER_MID);
 }
 
 // ---- assembly_counts (:160-221) ---------------------------------------------------
-BK_DEV void set_counts(RegionCtx& c, int start, int end, int n, bool io) {      // :195-199
+template <class T>
+BK_DEV void set_counts(RegionCtxT<T>& c, int start, int end, int n, bool io) {      // :195-199
   int32_t* v = (io ? c.io_vec(c.cur) : c.ot_vec(c.cur)) + c.k0;
   if (end > c.klen) end = c.klen;                                   // python slice clipping
   for (int x = start + lane(); x < end; x += WARP) v[x] += n;
   syncwarp();
 }
-BK_DEV void extend_counts(RegionCtx& c, int l, int n, bool io, bool post) {     // :201-221
+template <class T>
+BK_DEV void extend_counts(RegionCtxT<T>& c, int l, int n, bool io, bool post) {     // :201-221
   int32_t* vi = c.io_vec(c.cur);
   int32_t* vo = c.ot_vec(c.cur);
   const int at = post ? c.k0 + c.klen : c.k0 - l;
@@ -441,14 +484,15 @@ BK_DEV void extend_counts(RegionCtx& c, int l, int n, bool io, bool post) {     
 }
 // contig replaced by read u; old counts re-added at [start, end) with python's
 // zip-truncate / slice-assign semantics (:181-193, Q17).  s_read holds read u.
-BK_DEV void set_superseq(RegionCtx& c, int u, const uint8_t* rd, int lr, int start, int end) {
+template <class T>
+BK_DEV void set_superseq(RegionCtxT<T>& c, int u, const uint8_t* rd, int lr, int start, int end) {
   const int n = (int)c.u_mult[u];
   const bool io = c.u_io[u] != 0;
   const int bio = io ? n : 0, bot = io ? 0 : n;
   const int32_t* oi = c.io_vec(c.cur) + c.k0;
   const int32_t* oo = c.ot_vec(c.cur) + c.k0;
-  int32_t* ni = c.io_vec(c.cur ^ 1) + ASM_CAP;
-  int32_t* no = c.ot_vec(c.cur ^ 1) + ASM_CAP;
+  int32_t* ni = c.io_vec(c.cur ^ 1) + T::CAP;
+  int32_t* no = c.ot_vec(c.cur ^ 1) + T::CAP;
   const int span = end - start;
   const int mid = span < c.klen ? span : c.klen;
   const int tail = lr - end;
@@ -458,9 +502,9 @@ BK_DEV void set_superseq(RegionCtx& c, int u, const uint8_t* rd, int lr, int sta
     if (x >= start && x < start + mid) { a += oi[x - start]; b += oo[x - start]; }
     ni[x] = a; no[x] = b;
   }
-  c.cur ^= 1; c.k0 = ASM_CAP; c.klen = nl;
-  c.c0 = ASM_CAP; c.clen = lr;
-  for (int x = lane(); x < lr; x += WARP) { const uint8_t ch = rd[x]; c.cseq[ASM_CAP + x] = ch; c.s_contig[x] = ch; }
+  c.cur ^= 1; c.k0 = T::CAP; c.klen = nl;
+  c.c0 = T::CAP; c.clen = lr;
+  for (int x = lane(); x < lr; x += WARP) { const uint8_t ch = rd[x]; c.cseq[T::CAP + x] = ch; c.s_contig[x] = ch; }
   c.seq_ver += 1;
   syncwarp();
 }
@@ -488,20 +532,21 @@ int find_in_slice(const uint8_t* seq, int a, int b, int k, uint64_t code) {
 }
 
 // ---- contig.__init__ (:417-426) ---------------------------------------------------------
-BK_DEV void contig_init(RegionCtx& c, int seed_s, int u) {
+template <class T>
+BK_DEV void contig_init(RegionCtxT<T>& c, int seed_s, int u) {
   BK_PH_BEGIN
   c.serial += 1;
-  if (c.serial >= (1u << 20)) { c.status = ST_CAPACITY; return; }   // tag width of m_first
+  if (c.serial >= (1u << (32 - T::BITS))) { c.status = ST_CAPACITY; return; }   // tag width of m_first
   const int lr = stage_read(c, u);
-  c.c0 = ASM_CAP; c.clen = lr;
-  c.cur = 0; c.k0 = ASM_CAP; c.klen = lr;
+  c.c0 = T::CAP; c.clen = lr;
+  c.cur = 0; c.k0 = T::CAP; c.klen = lr;
   const int n = (int)c.u_mult[u];
   const bool io = c.u_io[u] != 0;
-  int32_t* vi = c.io_vec(0) + ASM_CAP;
-  int32_t* vo = c.ot_vec(0) + ASM_CAP;
+  int32_t* vi = c.io_vec(0) + T::CAP;
+  int32_t* vo = c.ot_vec(0) + T::CAP;
   for (int x = lane(); x < lr; x += WARP) {
     const uint8_t ch = c.s_read[x];
-    c.cseq[ASM_CAP + x] = ch; c.s_contig[x] = ch;
+    c.cseq[T::CAP + x] = ch; c.s_contig[x] = ch;
     vi[x] = io ? n : 0; vo[x] = io ? 0 : n;
   }
   c.nK = 0; c.nNK = 0;
@@ -549,9 +594,10 @@ void spec_dp(SpecShared* sp, const uint8_t* s_reads, int read_cap, const uint8_t
 
 // mer (local index) that stream slot `pos` belongs to, and where that mer sits in the
 // contig's gap buffer (a hint for the predictor; may be stale after a replacement)
-BK_DEV int slot_mer(const RegionCtx& c, int pos, int* anchor_buf) {
+template <class T>
+BK_DEV int slot_mer(const RegionCtxT<T>& c, int pos, int* anchor_buf) {
   if (c.round_seed >= 0) { *anchor_buf = c.seed_anchor; return c.round_seed; }
-  const int32_t* Ns = c.NK; const int32_t* Nend = c.NK + ASM_KCAP; const int32_t* Nb = c.NK + 3 * ASM_KCAP;
+  const int32_t* Ns = c.NK; const int32_t* Nend = c.NK + T::KCAP; const int32_t* Nb = c.NK + 3 * T::KCAP;
   int e = c.cur_e;
   while (pos >= Nend[e]) ++e;
   *anchor_buf = Nb[e];
@@ -561,7 +607,8 @@ BK_DEV int slot_mer(const RegionCtx& c, int pos, int* anchor_buf) {
 // Predicted contig after read slot w-1 is committed against contig buffer (src, la):
 // gapless overlap anchored at the shared k-mer.  Writes the prediction to dst (if it
 // differs) and returns its length; *same is set when the prediction is "unchanged".
-BK_DEV int predict_contig(const RegionCtx& c, const uint8_t* src, int la, const uint8_t* rd, int lr, int pos_r, int mer_s,
+template <class T>
+BK_DEV int predict_contig(const RegionCtxT<T>& c, const uint8_t* src, int la, const uint8_t* rd, int lr, int pos_r, int mer_s,
                           int xc_hint, uint8_t* dst, bool* same, int* shift) {
   *same = true;
   const int k = c.k;
@@ -597,12 +644,12 @@ BK_DEV int predict_contig(const RegionCtx& c, const uint8_t* src, int la, const 
     *shift = 0x40000000;                                        // coordinates of the old contig are void
   } else if (oL > 0) {                                          // prepend read[0:oL]
     nl = la + oL;
-    if (nl > NW_MAX_LEN) return la;
+    if (nl > T::MAX_LEN) return la;
     for (int x = lane(); x < nl; x += WARP) dst[x] = x < oL ? rd[x] : src[x - oL];
     *shift += oL;
   } else {                                                      // append read[lr-oR:]
     nl = la + oR;
-    if (nl > NW_MAX_LEN) return la;
+    if (nl > T::MAX_LEN) return la;
     for (int x = lane(); x < nl; x += WARP) dst[x] = x < la ? src[x] : rd[lr - oR + (x - la)];
   }
   *same = false;
@@ -610,8 +657,37 @@ BK_DEV int predict_contig(const RegionCtx& c, const uint8_t* src, int la, const 
   return nl;
 }
 
+#ifndef BK_SIM
+// The long kernel's pair (slot 0 of a width-1 round: staged read, current contig) through the anti-diagonal sweep of
+// nw_long.cuh, both directions, by every thread of the CTA.  v1 = nw(contig, read): columns = contig.
+__device__ __forceinline__ void long_pair_dp(SpecShared* sp, const uint8_t* rd, const uint8_t* ct, int32_t* diag) {
+  const int lr = sp->lr[0], lc = sp->la[0];
+  constexpr size_t stride = AsmCapLong::CAP + 1;
+  NwlEnd e = nwl_sweep(ct, lc, rd, lr, diag, stride, nullptr);
+  if (e.owner) sp->v1[0] = NwOut{lc, e.oj, e.i, e.oi, e.v};
+  e = nwl_sweep(rd, lr, ct, lc, diag, stride, nullptr);
+  if (e.owner) sp->v2[0] = NwOut{lr, e.oj, e.i, e.oi, e.v};
+}
+
+// DP of a long-kernel round: the warp DP of nw.cuh when both sequences are within its 4,095 bases (the staged read
+// and contig buffers hold at least NW_MAX_LEN + 1 bytes, as nw.cuh reads the row sequence that far), else the CTA
+// sweep; the other warps of the CTA wait for that command in assemble_long_kernel
+template <class T>
+BK_DEV void long_round_dp(RegionCtxT<T>& c) {
+  SpecShared* sp = c.sp;
+  if (sp->lr[0] <= NW_MAX_LEN && c.clen <= NW_MAX_LEN) {
+    spec_dp(sp, c.s_reads, c.P->read_cap, c.s_contig, nullptr, 0, c.edge_all, c.lastcol, c.tab);
+    return;
+  }
+  __syncthreads();                                   // command published (sp->n, lr[0], la[0])
+  long_pair_dp(sp, c.s_reads, c.s_contig, c.nwl_diag);
+  __syncthreads();                                   // results published
+}
+#endif
+
 // one speculation round over stream slots [pos, pos + cnt)
-BK_DEV void nw_round(RegionCtx& c, int pos, int cnt) {
+template <class T>
+BK_DEV void nw_round(RegionCtxT<T>& c, int pos, int cnt) {
   BK_PH_BEGIN
   SpecShared* sp = c.sp;
   syncwarp();
@@ -661,9 +737,13 @@ BK_DEV void nw_round(RegionCtx& c, int pos, int cnt) {
 #else
   {
     BK_PH_BEGIN
-    if (multi) __syncthreads();
-    spec_dp(sp, c.s_reads, c.P->read_cap, c.s_contig, c.s_pred, 0, c.edge_all, c.lastcol, c.tab);
-    if (multi) __syncthreads();
+    if constexpr (T::LONG) {
+      long_round_dp(c);
+    } else {
+      if (multi) __syncthreads();
+      spec_dp(sp, c.s_reads, c.P->read_cap, c.s_contig, c.s_pred, 0, c.edge_all, c.lastcol, c.tab);
+      if (multi) __syncthreads();
+    }
     BK_PH_END(c, PH_DP)
   }
 #endif
@@ -672,8 +752,10 @@ BK_DEV void nw_round(RegionCtx& c, int pos, int cnt) {
 }
 
 // ---- contig.check_align (:449-504), decision part: v1/v2 come from the round -------------------------------
-BK_DEV bool apply_align_impl(RegionCtx& c, int u, int seed_s, bool grow, const uint8_t* rd, int lr, const NwOut& v1, const NwOut& v2);
-BK_DEV bool apply_align(RegionCtx& c, int u, int seed_s, bool grow, const uint8_t* rd, int lr, const NwOut& v1, const NwOut& v2) {
+template <class T>
+BK_DEV bool apply_align_impl(RegionCtxT<T>& c, int u, int seed_s, bool grow, const uint8_t* rd, int lr, const NwOut& v1, const NwOut& v2);
+template <class T>
+BK_DEV bool apply_align(RegionCtxT<T>& c, int u, int seed_s, bool grow, const uint8_t* rd, int lr, const NwOut& v1, const NwOut& v2) {
   BK_PH_BEGIN
   const bool r = apply_align_impl(c, u, seed_s, grow, rd, lr, v1, v2);
   BK_PH_END(c, PH_APPLY)
@@ -682,7 +764,8 @@ BK_DEV bool apply_align(RegionCtx& c, int u, int seed_s, bool grow, const uint8_
 // contig.check_align (:449-504) with contig_overlap_read (:506-528) and read_overlap_contig (:530-546).  The decision
 // tree is evaluated first and yields one action; every action's body exists once (instruction footprint).
 enum { ACT_SUPERSEQ = 1, ACT_COUNTS, ACT_APPEND, ACT_PREPEND };
-BK_DEV bool apply_align_impl(RegionCtx& c, int u, int seed_s, bool grow, const uint8_t* rd, int lr, const NwOut& v1, const NwOut& v2) {
+template <class T>
+BK_DEV bool apply_align_impl(RegionCtxT<T>& c, int u, int seed_s, bool grow, const uint8_t* rd, int lr, const NwOut& v1, const NwOut& v2) {
   const int lc = c.clen;
   c.n_align += 1ull;
   c.n_cells += (unsigned long long)lc * (unsigned long long)lr;
@@ -735,7 +818,7 @@ BK_DEV bool apply_align_impl(RegionCtx& c, int u, int seed_s, bool grow, const u
     return true;
   } else if (act == ACT_APPEND) {
     const int plen = lr - v1.prei;                                    // post_seq = read[aln[4]:]
-    if (lc + plen > NW_MAX_LEN) { c.status = ST_CAPACITY; return true; }
+    if (lc + plen > T::MAX_LEN) { c.status = ST_CAPACITY; return true; }
     for (int x = lane(); x < plen; x += WARP) {
       const uint8_t ch = rd[v1.prei + x];
       c.cseq[c.c0 + lc + x] = ch; c.s_contig[lc + x] = ch;
@@ -748,7 +831,7 @@ BK_DEV bool apply_align_impl(RegionCtx& c, int u, int seed_s, bool grow, const u
     k_base = lc - (c.k - 1); k_len = (c.k - 1) + plen; k_order = ORDER_FOR;   // :521,525-527
   } else {
     const int plen = v2.j0;                                           // pre_seq = read[0:aln[3]]
-    if (lc + plen > NW_MAX_LEN) { c.status = ST_CAPACITY; return true; }
+    if (lc + plen > T::MAX_LEN) { c.status = ST_CAPACITY; return true; }
     for (int x = lane(); x < plen; x += WARP) c.cseq[c.c0 - plen + x] = rd[x];
     c.c0 -= plen; c.clen = lc + plen;
     c.seq_ver += 1;
@@ -768,7 +851,8 @@ BK_DEV bool apply_align_impl(RegionCtx& c, int u, int seed_s, bool grow, const u
 // ---- contig.check_read (:552-566, Q30) for stream slot `pos` -----------------------------------------------
 // Uses the slot's result from the last round if the contig it was aligned against
 // is byte-identical to the contig now; otherwise runs a new round starting here.
-BK_DEV bool round_slot_valid(const RegionCtx& c, int w) {
+template <class T>
+BK_DEV bool round_slot_valid(const RegionCtxT<T>& c, int w) {
   const SpecShared* sp = c.sp;
   const int b = sp->abuf[w];
   if (sp->la[w] != c.clen) return false;
@@ -779,7 +863,8 @@ BK_DEV bool round_slot_valid(const RegionCtx& c, int w) {
   return ballot(diff) == 0u;
 }
 
-BK_DEV bool check_read(RegionCtx& c, int seed_s, int pos, bool grow) {
+template <class T>
+BK_DEV bool check_read(RegionCtxT<T>& c, int seed_s, int pos, bool grow) {
   bool have = pos < c.rnd_base + c.rnd_cnt;
   if (have) {
     BK_PH_BEGIN
@@ -810,7 +895,8 @@ BK_DEV bool check_read(RegionCtx& c, int seed_s, int pos, bool grow) {
 }
 
 // ---- buffer.add_contig (:337-340) ----------------------------------------------------------------
-BK_DEV bool add_contig(RegionCtx& c, int u, int seed_s) {
+template <class T>
+BK_DEV bool add_contig(RegionCtxT<T>& c, int u, int seed_s) {
   const bool used = c.r_used[u];            // (a queued read is always used, so `id in contigs` is implied)
   syncwarp();                               // every lane has read the flag before lane 0 sets it
   if (used) return false;
@@ -824,7 +910,8 @@ BK_DEV bool add_contig(RegionCtx& c, int u, int seed_s) {
 }
 
 // ---- contig.check_alt_reads (:568-582, Q12, Q13) + finalize (:584-599) + rb.clean (:389-397, Q11) --
-BK_DEV void finalize(RegionCtx& c, bool setup) {
+template <class T>
+BK_DEV void finalize(RegionCtxT<T>& c, bool setup) {
   if (setup) set_kmers(c);
   BK_PH_BEGIN
   c.fin_serial += 1;
@@ -878,24 +965,28 @@ BK_DEV void finalize(RegionCtx& c, bool setup) {
 // all going to be checked by this contig, in this order, whatever the outcomes
 // (the k-mer snapshot loop of grow has no early exit), so adding them early is
 // unobservable.
-BK_DEV int find_reads(RegionCtx& c, int s, bool filter_buffer, bool rev, int at) {
+template <class T>
+BK_DEV int find_reads(RegionCtxT<T>& c, int s, bool filter_buffer, bool rev, int at) {
   BK_PH_BEGIN
   const int64_t a = c.P->post_off[c.gm0 + s], b = c.P->post_off[c.gm0 + s + 1];
   const int32_t* pr = c.P->post_read + a;
   const int32_t* pp = c.P->post_pos + a;
   const int n0 = (int)(b - a);
   const unsigned lt = lane_lt_mask();
+  using Key = typename T::Key;
+  constexpr unsigned KEY_MAX = T::BITS == 16 ? 0xFFFFFFFFu : (1u << (2 * T::BITS)) - 1u;
   int n = 0;
   if (n0 <= WARP) {
     // the whole posting list fits one warp pass: filter, rank and place from registers
     const int i = lane();
     bool keep = false;
-    int u = 0, key = 0, pos = 0;
+    int u = 0, pos = 0;
+    Key key = 0;
     if (i < n0) {
       u = pr[i]; pos = pp[i];
       keep = !c.r_deleted[u] && !(filter_buffer && c.r_buf[u] == c.serial);
-      // sort key: primary pos (or -pos), secondary -len; both < 4096
-      key = ((rev ? (ASM_CAP - 1 - pos) : pos) << 12) | (ASM_CAP - 1 - c.u_len[u]);
+      // sort key: primary pos (or -pos), secondary -len; both < CAP
+      key = ((Key)(rev ? (T::CAP - 1 - pos) : pos) << T::BITS) | (Key)(T::CAP - 1 - c.u_len[u]);
     }
     const unsigned mk = ballot(keep);
     n = popc(mk);
@@ -905,7 +996,7 @@ BK_DEV int find_reads(RegionCtx& c, int s, bool filter_buffer, bool rev, int at)
 #else
     for (unsigned rest = mk; rest; rest &= rest - 1) {
       const int j = __ffs((int)rest) - 1;
-      const int kj = __shfl_sync(0xffffffffu, key, j);
+      const Key kj = __shfl_sync(0xffffffffu, key, j);
       rank += (kj < key || (kj == key && j < i)) ? 1 : 0;          // stable: ties keep read order (Q9)
     }
 #endif
@@ -928,9 +1019,9 @@ BK_DEV int find_reads(RegionCtx& c, int s, bool filter_buffer, bool rev, int at)
       const unsigned mk = ballot(keep);
       if (keep) {
         const int dst = n + popc(mk & lt);
-        const unsigned key = (unsigned)(((rev ? (ASM_CAP - 1 - pos) : pos) << 12) | (ASM_CAP - 1 - c.u_len[u]));
+        const unsigned key = ((unsigned)(rev ? (T::CAP - 1 - pos) : pos) << T::BITS) | (unsigned)(T::CAP - 1 - c.u_len[u]);
         c.hit2_u[dst] = u;
-        c.sort_a[dst] = ((unsigned long long)(0xFFFFFFu - key) << 32) | (unsigned)(0x7FFFFFFF - dst);
+        c.sort_a[dst] = ((unsigned long long)(KEY_MAX - key) << 32) | (unsigned)(0x7FFFFFFF - dst);
         if (filter_buffer) c.r_buf[u] = c.serial;
       }
       n += popc(mk);
@@ -940,9 +1031,9 @@ BK_DEV int find_reads(RegionCtx& c, int s, bool filter_buffer, bool rev, int at)
     for (int r = lane(); r < n; r += WARP) {
       const uint64_t kk = sorted[r];
       const int i = 0x7FFFFFFF - (int)(kk & 0xFFFFFFFFu);
-      const int hi = (int)((0xFFFFFFu - (unsigned)(kk >> 32)) >> 12);
+      const int hi = (int)((KEY_MAX - (unsigned)(kk >> 32)) >> T::BITS);
       c.hit_u[at + r] = c.hit2_u[i];
-      c.hit_pos[at + r] = rev ? (ASM_CAP - 1 - hi) : hi;
+      c.hit_pos[at + r] = rev ? (T::CAP - 1 - hi) : hi;
     }
   }
   syncwarp();
@@ -953,7 +1044,8 @@ BK_DEV int find_reads(RegionCtx& c, int s, bool filter_buffer, bool rev, int at)
 
 // buffer.add_used_mer (:334-335): used_mers is a dict; the mers added since the last remove_kmers are also kept in a
 // list so that remove_kmers (:358-360) touches those instead of sweeping the whole table once per seed
-BK_DEV void add_used_mer(RegionCtx& c, int s) {
+template <class T>
+BK_DEV void add_used_mer(RegionCtxT<T>& c, int s) {
   if (!c.mused[s]) {                                                 // (warp-uniform: every lane reads the same byte)
     syncwarp();
     if (lane() == 0) { c.mused[s] = 1; c.l_mused[c.n_mused] = s; }
@@ -963,13 +1055,14 @@ BK_DEV void add_used_mer(RegionCtx& c, int s) {
 }
 
 // ---- set_kmer_locs (:434-438, Q25) + emit the accepted contig -------------------------------------------
-BK_DEV void emit_contig(RegionCtx& c) {
+template <class T>
+BK_DEV void emit_contig(RegionCtxT<T>& c) {
   BK_PH_BEGIN
   const AsmParams& P = *c.P;
   const int k = c.k, len = c.clen;
-  const int32_t* Ks = c.K; const int32_t* Kx = c.K + ASM_KCAP; const int32_t* Km = c.K + 2 * ASM_KCAP;
+  const int32_t* Ks = c.K; const int32_t* Kx = c.K + T::KCAP; const int32_t* Km = c.K + 2 * T::KCAP;
   // first window of every sample-only mer in the final contig (str.find), via a tagged
-  // per-mer table: [serial | 4095 - x] under atomicMax keeps the smallest x of this contig
+  // per-mer table: [serial | CAP - 1 - x] under atomicMax keeps the smallest x of this contig
   const int nwin = len - k + 1;
   for (int x = lane(); x <= len; x += WARP) c.diff[x] = 0;
   {
@@ -977,14 +1070,14 @@ BK_DEV void emit_contig(RegionCtx& c) {
     lookup_windows(c, c.s_contig, nwin, win);
     for (int x = lane(); x < nwin; x += WARP) {
       const int s = win[x];
-      if (s >= 0) atomic_max(&c.first[s], (c.serial << 12) | (unsigned)(4095 - x));
+      if (s >= 0) atomic_max(&c.first[s], (c.serial << T::BITS) | (unsigned)(T::CAP - 1 - x));
     }
   }
   syncwarp();
   for (int e = lane(); e < c.nK; e += WARP) {
     const unsigned v = c.first[Ks[e]];
-    if ((v >> 12) == c.serial) {                                     // find() == -1 touches nothing (Q25)
-      const int p = 4095 - (int)(v & 4095u);
+    if ((v >> T::BITS) == c.serial) {                                // find() == -1 touches nothing (Q25)
+      const int p = T::CAP - 1 - (int)(v & (unsigned)(T::CAP - 1));
       atomic_add(&c.diff[p], 1);
       atomic_add(&c.diff[(p + k) < len ? (p + k) : len], -1);
     }
@@ -1063,12 +1156,14 @@ BK_DEV void emit_contig(RegionCtx& c) {
 //                    finalize still run against it, then it is dropped
 //   GROW_ONLY        a contig popped from the FIFO
 enum { GROW_ONLY = 0, GROW_SETUP = 1, GROW_SETUP_ONLY = 2 };
-BK_DEV void grow(RegionCtx& c, int mode, int seed_s) {
+template <class T>
+BK_DEV void grow(RegionCtxT<T>& c, int mode, int seed_s) {
   bool setup = mode != GROW_ONLY;
   if (!setup && !c.ct_setup) set_kmers(c);
   const unsigned lt = lane_lt_mask();
-  int32_t* Ks = c.K; int32_t* Km = c.K + 2 * ASM_KCAP; int32_t* Kb = c.K + 3 * ASM_KCAP;
-  int32_t* Ns = c.NK; int32_t* Nend = c.NK + ASM_KCAP; int32_t* Nm = c.NK + 2 * ASM_KCAP; int32_t* Nb = c.NK + 3 * ASM_KCAP;
+  constexpr int KCAP = T::KCAP;
+  int32_t* Ks = c.K; int32_t* Km = c.K + 2 * KCAP; int32_t* Kb = c.K + 3 * KCAP;
+  int32_t* Ns = c.NK; int32_t* Nend = c.NK + KCAP; int32_t* Nm = c.NK + 2 * KCAP; int32_t* Nb = c.NK + 3 * KCAP;
   while (c.status == ST_OK) {
     int nn = 1;
     if (!setup) {
@@ -1114,7 +1209,7 @@ BK_DEV void grow(RegionCtx& c, int mode, int seed_s) {
       add_used_mer(c, seed_s);                                         // buff.add_used_mer (:15)
       if (st == 0) { c.setup_queued = false; return; }                 // no read holds the seed: nothing to set up
       c.round_seed = seed_s;
-      c.seed_anchor = ASM_CAP + c.hit_pos[0];                          // contig_init puts the first read at ASM_CAP
+      c.seed_anchor = T::CAP + c.hit_pos[0];                           // contig_init puts the first read at CAP
       c.rnd_cnt = 1;                                                   // slot 0 is the contig's own read: nothing to align
       const int u0 = c.hit_u[0];
       contig_init(c, seed_s, u0);
@@ -1159,7 +1254,8 @@ BK_DEV void grow(RegionCtx& c, int mode, int seed_s) {
   }
 }
 
-BK_DEV int total_reads(const RegionCtx& c) {                         // :178-179
+template <class T>
+BK_DEV int total_reads(const RegionCtxT<T>& c) {                         // :178-179
   const int32_t* vi = c.io_vec(c.cur) + c.k0;
   const int32_t* vo = c.ot_vec(c.cur) + c.k0;
   int a = -0x7fffffff, b = -0x7fffffff;
@@ -1168,7 +1264,8 @@ BK_DEV int total_reads(const RegionCtx& c) {                         // :178-179
 }
 
 // after grow: accept or drop (:53-59, Q21)
-BK_DEV void finish_contig(RegionCtx& c, int rc_thresh, int read_len) {
+template <class T>
+BK_DEV void finish_contig(RegionCtxT<T>& c, int rc_thresh, int read_len) {
   if (c.status != ST_OK) return;
   if (total_reads(c) < rc_thresh || c.clen <= read_len) return;
   emit_contig(c);
@@ -1178,7 +1275,8 @@ BK_DEV void finish_contig(RegionCtx& c, int rc_thresh, int read_len) {
 // The reference keeps the mers in an OrderedDict sorted by (count, mer) descending and takes the first remaining one:
 // the first live entry of the region's seed order.  Mers only ever leave akmers, so a cursor over the order suffices;
 // 32 entries are tested per step.  Returns -1 when no live mer with count > 1 is left.
-BK_DEV int next_seed(RegionCtx& c) {
+template <class T>
+BK_DEV int next_seed(RegionCtxT<T>& c) {
   while (c.seed_cursor < c.S) {
     const int i = c.seed_cursor + lane();
     bool live = false;
@@ -1197,7 +1295,8 @@ BK_DEV int next_seed(RegionCtx& c) {
 }
 
 // ---- init_assembly (:30-63) for one region ------------------------------------------------------------------
-BK_DEV void assemble_region(RegionCtx& c) {
+template <class T>
+BK_DEV void assemble_region(RegionCtxT<T>& c) {
   const AsmParams& P = *c.P;
   const int read_len = P.read_len[c.region];
   c.serial = 0; c.fin_serial = 0; c.status = ST_OK; c.n_out = 0; c.n_align = 0; c.n_cells = 0;
@@ -1248,14 +1347,16 @@ BK_DEV void assemble_region(RegionCtx& c) {
 // ---- kmers.get_all_kmer_values (:280-285, Q7): the region's mers by (count, mer) descending -----------------------
 // Keys [count | local index] are unique, mers ascend with the index: one warp_sort_desc per region instead of a scan
 // per seed.
-BK_DEV void build_seed_order(RegionCtx& c, uint64_t* a, uint64_t* b) {
+template <class T>
+BK_DEV void build_seed_order(RegionCtxT<T>& c, uint64_t* a, uint64_t* b) {
   for (int i = lane(); i < c.S; i += WARP) a[i] = ((unsigned long long)c.cnt[i] << 32) | (unsigned)i;
   syncwarp();
   c.seed_keys = warp_sort_desc(a, b, c.S);
   c.seed_cursor = 0;
 }
 
-BK_DEV void bind_region(RegionCtx& c, const AsmParams& P, int region, int64_t slot, uint8_t* s_reads, uint8_t* s_contig,
+template <class T>
+BK_DEV void bind_region(RegionCtxT<T>& c, const AsmParams& P, int region, int64_t slot, uint8_t* s_reads, uint8_t* s_contig,
                         uint8_t* s_pred, int32_t* s_hash, SpecShared* sp, int spec_w) {
   c.s_hash = s_hash;
   c.spec_w = spec_w; c.s_pred = s_pred; c.round_seed = -1; c.cur_e = 0; c.rnd_ver = 0;
@@ -1273,12 +1374,12 @@ BK_DEV void bind_region(RegionCtx& c, const AsmParams& P, int region, int64_t sl
   c.hit_u = P.hit_u + c.gu0; c.hit_pos = P.hit_pos + c.gu0; c.hit2_u = P.hit2_u + c.gu0; c.hit2_pos = P.hit2_pos + c.gu0;
   c.sort_a = P.sort_a + c.gu0; c.sort_b = P.sort_b + c.gu0;
   c.l_mused = P.l_mused + c.gm0; c.n_mused = 0;
-  c.cseq = P.w_cseq + slot * ASM_BUF;
-  c.cnt_buf = P.w_cnt + slot * 4 * ASM_BUF;
-  c.K = P.w_K + slot * 4 * ASM_KCAP;
-  c.NK = P.w_NK + slot * 4 * ASM_KCAP;
-  c.wcode = P.w_wcode + slot * ASM_CAP;
-  c.diff = P.w_diff + slot * (ASM_CAP + 1);
+  c.cseq = P.w_cseq + slot * T::BUF;
+  c.cnt_buf = P.w_cnt + slot * 4 * T::BUF;
+  c.K = P.w_K + slot * 4 * T::KCAP;
+  c.NK = P.w_NK + slot * 4 * T::KCAP;
+  c.wcode = P.w_wcode + slot * T::CAP;
+  c.diff = P.w_diff + slot * (T::CAP + 1);
   c.edge_all = P.w_edge ? P.w_edge + slot * spec_w * 2 * ASM_CAP : nullptr;
   c.lastcol = P.w_lastcol ? P.w_lastcol + (size_t)slot * spec_w * ASM_LASTCOL : nullptr;
   c.tab = P.w_tab ? P.w_tab + (size_t)slot * spec_w * NW_TAB_BYTES : nullptr;
@@ -1384,6 +1485,15 @@ __global__ void __launch_bounds__(32 * W, (CTAS > 0 ? CTAS : (W >= 8 ? 1 : (W ==
     __syncthreads();
   }
 }
+
+// ---- assemble_long_kernel: the same state machine with AsmCapLong (reads and contigs up to 65,535 bases) ----------
+// Per-CTA scratch in global memory (the contig and the staged read do not fit shared memory at this capacity)
+struct AsmLongScratch {
+  uint8_t* reads;                  // read_cap bytes per CTA (>= longest read + 2 and > NW_MAX_LEN)
+  uint8_t* contig;                 // AsmCapLong::CAP bytes per CTA
+  int32_t* diag;                   // 9 * (AsmCapLong::CAP + 1) ints per CTA: the sweep's rolling diagonals
+};
+
 #endif
 
 }  // namespace bk

@@ -10,11 +10,9 @@
 // need no pointer table; only when the alignment STRINGS are asked for (direction A of bk_nw_batch with want_aln) is
 // the (n+1)(m+1)-byte pointer table written and walked back by one thread as olc.py does.
 #pragma once
-#include "common.cuh"
+#include "nw_sweep.cuh"
 
 namespace bk {
-
-constexpr int NWL_THREADS = 256;
 
 struct NwLongParams {
   const uint8_t* seqs;
@@ -36,8 +34,6 @@ struct NwLongParams {
 
 // grid = 2 * n_long: CTA 2q = nw(seq1, seq2) of long pair q (fields 0-4 of its output row), CTA 2q+1 = nw(seq2, seq1)
 __global__ void __launch_bounds__(NWL_THREADS) nw_long_kernel(NwLongParams p) {
-  __shared__ int red_v[NWL_THREADS];
-  __shared__ int red_i[NWL_THREADS];
   const int tid = threadIdx.x;
   const int64_t q = blockIdx.x >> 1;
   const int dir = blockIdx.x & 1;
@@ -49,67 +45,16 @@ __global__ void __launch_bounds__(NWL_THREADS) nw_long_kernel(NwLongParams p) {
   const int m = (int)(p.seq_off[ia + 1] - p.seq_off[ia]);
   const int n = (int)(p.seq_off[ib + 1] - p.seq_off[ib]);
   int32_t* base = p.diag + (size_t)blockIdx.x * 9 * p.diag_stride;
-  const size_t stride = (size_t)p.diag_stride;                      // buffer b, field f (score, stop row, stop column) at (3b + f) * stride
   const bool want_ptr = p.want_aln && dir == 0;
   uint8_t* pm = want_ptr ? p.ptr_scratch + p.ptr_off[q] : nullptr;
   const size_t width = (size_t)m + 1;
-
-  // end cell of olc.py:79-83 over the last column (row 0 scores 0); per thread in ascending rows with >=
-  int best_v = tid == 0 ? 0 : -2147483647 - 1, best_i = 0, best_oi = 0, best_oj = 0;
-  int cur = 0;                                                       // buffer of diagonal d; (cur+2)%3 = d-1, (cur+1)%3 = d-2
-  for (int d = 2; d <= m + n; ++d) {
-    const int32_t* s_1 = base + (size_t)(3 * ((cur + 2) % 3)) * stride;     // diagonal d-1
-    const int32_t* i_1 = s_1 + stride;
-    const int32_t* j_1 = i_1 + stride;
-    const int32_t* s_2 = base + (size_t)(3 * ((cur + 1) % 3)) * stride;     // diagonal d-2
-    const int32_t* i_2 = s_2 + stride;
-    const int32_t* j_2 = i_2 + stride;
-    int32_t* s_0 = base + (size_t)(3 * cur) * stride;                       // diagonal d
-    int32_t* i_0 = s_0 + stride;
-    int32_t* j_0 = i_0 + stride;
-    const int ilo = d - m > 1 ? d - m : 1;
-    const int ihi = d - 1 < n ? d - 1 : n;
-    for (int i = ilo + tid; i <= ihi; i += NWL_THREADS) {
-      const int j = d - i;
-      const bool top = i == 1, lft = j == 1;                         // the neighbours in row 0 / column 0 score 0
-      const int dg = ((top || lft) ? 0 : s_2[i - 1]) + (s1[j - 1] == s2[i - 1] ? 1 : -2);   // olc.py:18-20, 63
-      const int up = (lft ? 0 : s_1[i]) - 2;                         // score[i][j-1]: consumes seq1 (olc.py:64)
-      const int lf = (top ? 0 : s_1[i - 1]) - 2;                     // score[i-1][j]: consumes seq2 (olc.py:65)
-      int best = lf > up ? lf : up;
-      best = dg > best ? dg : best;
-      int si, sj;
-      uint8_t t;
-      if (best == dg)      { t = 3; if (top || lft) { si = i - 1; sj = j - 1; } else { si = i_2[i - 1]; sj = j_2[i - 1]; } }
-      else if (best == up) { t = 2; if (lft)        { si = i;     sj = 0;     } else { si = i_1[i];     sj = j_1[i];     } }
-      else                 { t = 1; if (top)        { si = 0;     sj = j;     } else { si = i_1[i - 1]; sj = j_1[i - 1]; } }
-      s_0[i] = best;
-      i_0[i] = si;
-      j_0[i] = sj;
-      if (want_ptr) pm[(size_t)i * width + j] = t;
-      if (j == m && best >= best_v) { best_v = best; best_i = i; best_oi = si; best_oj = sj; }
-    }
-    __syncthreads();
-    cur = (cur + 1) % 3;
-  }
-  // the largest row among the maxima wins (>= scan in ascending rows)
-  red_v[tid] = best_v;
-  red_i[tid] = best_i;
-  __syncthreads();
-  for (int s = NWL_THREADS / 2; s > 0; s >>= 1) {
-    if (tid < s) {
-      const int v = red_v[tid + s], i2 = red_i[tid + s];
-      if (v > red_v[tid] || (v == red_v[tid] && i2 > red_i[tid])) { red_v[tid] = v; red_i[tid] = i2; }
-    }
-    __syncthreads();
-  }
-  const int end_v = red_v[0], end_i = red_i[0];
-  if (best_v == end_v && best_i == end_i && (end_i > 0 || tid == 0)) {         // exactly one thread owns the end cell
+  const NwlEnd e = nwl_sweep(s1, m, s2, n, base, (size_t)p.diag_stride, pm);
+  if (e.owner) {
     int32_t* o = p.out + pi * 10 + dir * 5;
-    if (end_i == 0) { best_oi = 0; best_oj = m - 1; }               // pointer[0][m] = 2 (olc.py:58-59): one step along row 0
-    o[0] = m; o[1] = best_oj; o[2] = end_i; o[3] = best_oi; o[4] = end_v;
+    o[0] = m; o[1] = e.oj; o[2] = e.i; o[3] = e.oi; o[4] = e.v;
   }
   if (want_ptr && tid == 0) {                                        // olc.py:86-105; stored end-first, the host flips
-    int i = end_i, j = m, len = 0;
+    int i = e.i, j = m, len = 0;
     uint8_t* a1 = p.aln1 + p.aln_off[pi];
     uint8_t* a2 = p.aln2 + p.aln_off[pi];
     for (;;) {

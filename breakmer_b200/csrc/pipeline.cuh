@@ -67,6 +67,8 @@ struct PendingBatch {
   Pipeline local;                          // non-resident submits own their Pipeline
   AsmParams A;
   int spec_w = 4, ctas_per_sm = 3, grid = 1, dyn_smem = 0;
+  bool long_path = false;                  // bk_compare_kmers_long: assemble_long_kernel with its scratch L
+  AsmLongScratch L{};
   uint8_t* zero_lo = nullptr;
   size_t zero_bytes = 0;
   unsigned long long cap_seq = 0;

@@ -1,5 +1,5 @@
 // Host orchestration of the batched whole-path pipeline (bk_batch_submit / bk_batch_wait, and the one-call forms
-// bk_compare_kmers_batch, bk_batch_upload + bk_compare_kmers_resident).  Included into api.cu.
+// bk_compare_kmers_batch, bk_batch_upload + bk_compare_kmers_resident, bk_compare_kmers_long).  Included into api.cu.
 //
 // Stage order on the handle's stream (every stage is a kernel in this directory):
 //   1. group identical reads            prep.cuh   read_hash -> radix sort -> leaders -> scan -> scatter
@@ -70,14 +70,15 @@ void upload_record_set(bk_handle_t h, Arena<false>& A, const char* bases, const 
   h2d += n_bases + (n_rec + 1) * 8;
 }
 
-void pipeline_upload_into(bk_handle_t h, Arena<false>& A, const bk_batch_input* in, Pipeline& p) {
+// max_len: the longest read the assembler of this call takes (NW_MAX_LEN, or ASM_LONG_MAX_LEN for bk_compare_kmers_long)
+void pipeline_upload_into(bk_handle_t h, Arena<false>& A, const bk_batch_input* in, Pipeline& p, int max_len = NW_MAX_LEN) {
   p = Pipeline();
   if (in->n_regions < 0 || in->n_regions > 65535) fail(BK_ERR_ARG, "batch: n_regions must be in 0..65535 per call");
   if (in->k < 2 || in->k > 31) fail(BK_ERR_ARG, "batch: k must be in 2..31");
   const int R = in->n_regions;
   p.n_regions = R; p.k = in->k; p.rc_thresh = in->rc_thresh; p.have_mers = in->have_mers;
   if (!in->read_off || !in->read_reg_off) fail(BK_ERR_ARG, "batch: read arrays missing");
-  // per-region read statistics; a region holding a read the DP cannot take is left out of the device pass (its
+  // per-region read statistics; a region holding a read the assembler cannot take is left out of the device pass (its
   // region_status becomes BK_ERR_CAPACITY) instead of failing the call: the other regions are unaffected
   std::vector<int32_t> rl(R ? R : 1, 0);
   int mx = 0;
@@ -88,7 +89,7 @@ void pipeline_upload_into(bk_handle_t h, Arena<false>& A, const bk_batch_input* 
     for (int64_t i = in->read_reg_off[r]; i < in->read_reg_off[r + 1]; ++i)
       m = std::max<int>(m, (int)std::min<int64_t>(in->read_off[i + 1] - in->read_off[i], int64_t(1) << 30));
     rl[r] = in->read_len ? in->read_len[r] : m;                    // utils.py:236
-    if (m > NW_MAX_LEN) {
+    if (m > max_len) {
       if (p.region_skipped.empty()) p.region_skipped.assign(R, 0);
       p.region_skipped[r] = 1;
       ++n_skipped;
@@ -260,6 +261,28 @@ void ref_cache_build(bk_handle_t h, const char* ref_bases, const int64_t* ref_of
   h->ref_cache_mers = mers; h->ref_cache_koff = koff; h->ref_cache_regions = R; h->ref_cache_k = k;
 }
 
+// assemble_long_kernel's grid and per-CTA scratch: one CTA per region up to one per SM, contig-sized arrays for
+// AsmCapLong (a few MB per CTA), the staged read for the longest read of the call
+void long_assembly_scratch(bk_handle_t h, PendingBatch& B, const Pipeline& p, int R) {
+  AsmParams& A = B.A;
+  using C = AsmCapLong;
+  const int grid = (int)std::max<int64_t>(1, std::min<int64_t>(R, h->sm_count));
+  B.long_path = true; B.spec_w = 1; B.grid = grid; B.dyn_smem = 0;
+  A.read_cap = (int)((std::max<int64_t>(NW_MAX_LEN + 1, p.max_read_len + 2) + 15) / 16 * 16);
+  A.w_cseq = h->dev.get<uint8_t>((size_t)grid * C::BUF);
+  A.w_cnt = h->dev.get<int32_t>((size_t)grid * 4 * C::BUF);
+  A.w_K = h->dev.get<int32_t>((size_t)grid * 4 * C::KCAP);
+  A.w_NK = h->dev.get<int32_t>((size_t)grid * 4 * C::KCAP);
+  A.w_wcode = h->dev.get<uint64_t>((size_t)grid * C::CAP);
+  A.w_diff = h->dev.get<int32_t>((size_t)grid * (C::CAP + 1));
+  A.w_edge = h->dev.get<int2>((size_t)grid * 2 * ASM_CAP);         // the warp DP's scratch (pairs within NW_MAX_LEN)
+  A.w_lastcol = h->dev.get<uint2>((size_t)grid * ASM_LASTCOL);
+  A.w_tab = h->dev.get<uint8_t>((size_t)grid * NW_TAB_BYTES);
+  B.L.reads = h->dev.get<uint8_t>((size_t)grid * A.read_cap);
+  B.L.contig = h->dev.get<uint8_t>((size_t)grid * C::CAP);
+  B.L.diag = h->dev.get<int32_t>((size_t)grid * 9 * (C::CAP + 1));
+}
+
 // (re)launch the assembler of a submitted batch: zero the mutable state, allocate the output arena for the current
 // capacity, launch, and queue the copies of the counters wait() looks at first
 void launch_assembly(bk_handle_t h, PendingBatch& B) {
@@ -275,7 +298,10 @@ void launch_assembly(bk_handle_t h, PendingBatch& B) {
   A.o_kmer_meta = h->dev.get<int32_t>(A.cap_kmers);
   A.o_desc = h->dev.get<int64_t>(A.cap_ctg * 10);
   BK_CUDA(cudaMemsetAsync(B.zero_lo, 0, B.zero_bytes, st));
-  if (R > 0) {
+  if (R > 0 && B.long_path) {
+    TimedLaunch t(h->timers, st, KF_ASSEMBLE);
+    BK_CUDA(launch_assemble_long(A, B.L, B.grid, st));
+  } else if (R > 0) {
     TimedLaunch t(h->timers, st, KF_ASSEMBLE);
     // shared-memory carve-out: just enough for the resident CTAs, the rest of the 256 KB stays L1
     int carve = (int)((100 * (size_t)B.ctas_per_sm * ((size_t)B.dyn_smem + 1024) + 228 * 1024 - 1) / (228 * 1024));
@@ -295,8 +321,9 @@ void launch_assembly(bk_handle_t h, PendingBatch& B) {
   B.h_cells = to_host(h, A.region_cells, (size_t)(R ? R : 1));
 }
 
-// Enqueue the whole device pass of one batch.  in == nullptr: the batch uploaded with bk_batch_upload.
-void pipeline_submit(bk_handle_t h, const bk_batch_input* in) {
+// Enqueue the whole device pass of one batch.  in == nullptr: the batch uploaded with bk_batch_upload.  long_path: the
+// assembler is assemble_long_kernel, and regions with reads up to ASM_LONG_MAX_LEN bases take part (bk_compare_kmers_long).
+void pipeline_submit(bk_handle_t h, const bk_batch_input* in, bool long_path = false) {
   cudaStream_t st = h->st;
   if (h->pending.active) fail(BK_ERR_ARG, "a batch is already in flight on this handle (call bk_batch_wait first)");
   h->dev.reset();
@@ -308,7 +335,7 @@ void pipeline_submit(bk_handle_t h, const bk_batch_input* in) {
     if (!h->pipe) fail(BK_ERR_ARG, "bk_compare_kmers_resident: no batch uploaded");
     B.p = h->pipe.get();
   } else {
-    pipeline_upload_into(h, h->dev, in, B.local);
+    pipeline_upload_into(h, h->dev, in, B.local, long_path ? ASM_LONG_MAX_LEN : NW_MAX_LEN);
     B.p = &B.local;
   }
   const Pipeline& p = *B.p;
@@ -443,12 +470,15 @@ void pipeline_submit(bk_handle_t h, const bk_batch_input* in) {
     {
       TimedLaunch t(h->timers, st, KF_INDEX);
       const int ws_stride = ((p.max_read_len + 31) / 32) * 32 + 32;
-      const size_t idx_smem = (size_t)IDX_WARPS * ws_stride * sizeof(int32_t);
+      // window table of a warp's read: shared memory up to NW_MAX_LEN bases; longer reads (bk_compare_kmers_long) use a
+      // global table, one window per read base at the read's own offset
+      int32_t* ws_global = p.max_read_len > NW_MAX_LEN ? h->dev.get<int32_t>((size_t)cap) : nullptr;
+      const size_t idx_smem = ws_global ? 0 : (size_t)IDX_WARPS * ws_stride * sizeof(int32_t);
       std::lock_guard<std::mutex> hold(launch_attr_mutex());
       if (idx_smem > 48 * 1024) BK_CUDA(cudaFuncSetAttribute(index_emit_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)idx_smem));
       index_emit_kernel<<<nblk(NUB, IDX_WARPS), 32 * IDX_WARPS, idx_smem, st>>>(p.reads.bases, p.reads.off, u_off, u_rec, R, d_NU, so_off,
                                                                                 so_mer, k, ik, iv, ik2, iv2, u_bits, s_bits, ws_stride,
-                                                                                d_npost, (uint32_t)std::min<int64_t>(cap, 0xFFFFFFFFll));
+                                                                                ws_global, d_npost, (uint32_t)std::min<int64_t>(cap, 0xFFFFFFFFll));
     }
     const int64_t tiles = rs_num_tiles(cap);
     RadixSortScratch sc;
@@ -489,30 +519,34 @@ void pipeline_submit(bk_handle_t h, const bk_batch_input* in) {
   A.so_off = so_off; A.so_mer = so_mer; A.so_cnt = so_cnt;
   A.post_off = post_off; A.post_read = post_read; A.post_pos = post_pos;
   A.work_order = order;
-  // speculation width and residency of the assembler (see assemble_kernel).  Auto = 4: one aligning warp per SM
-  // sub-partition; 8 warps share the four ALU pipes of the SM and finish a round no sooner (measured on C4).
-  int spec_w = h->spec_width;
-  if (const char* e = getenv("BK_SPEC_W")) spec_w = atoi(e);
-  if (spec_w <= 0) spec_w = 4;
-  spec_w = spec_w >= 8 ? 8 : (spec_w >= 4 ? 4 : (spec_w >= 2 ? 2 : 1));
-  int ctas_per_sm = spec_w == 8 ? 1 : (spec_w == 4 ? 3 : (spec_w == 2 ? 6 : 8));
-  if (const char* e = getenv("BK_ASM_CTAS_PER_SM")) ctas_per_sm = std::max(1, atoi(e));
-  int grid = (int)std::min<int64_t>(R, (int64_t)h->sm_count * ctas_per_sm);
-  if (grid < 1) grid = 1;
-  // dynamic shared memory: exactly what the kernel needs (padding it to bound residency starves L1: 15 % slower)
-  A.read_cap = (int)std::min<int64_t>(ASM_CAP, std::max<int64_t>(64, (p.max_read_len + 2 + 15) / 16 * 16));
-  B.spec_w = spec_w; B.ctas_per_sm = ctas_per_sm; B.grid = grid;
-  B.dyn_smem = (int)assemble_smem_bytes(spec_w, A.read_cap);
-  if (getenv("BK_ASM_PAD")) B.dyn_smem = std::max(B.dyn_smem, (int)((227 * 1024) / ctas_per_sm) - 1024);
-  A.w_cseq = h->dev.get<uint8_t>((size_t)grid * ASM_BUF);
-  A.w_cnt = h->dev.get<int32_t>((size_t)grid * 4 * ASM_BUF);
-  A.w_K = h->dev.get<int32_t>((size_t)grid * 4 * ASM_KCAP);
-  A.w_NK = h->dev.get<int32_t>((size_t)grid * 4 * ASM_KCAP);
-  A.w_wcode = h->dev.get<uint64_t>((size_t)grid * ASM_CAP);
-  A.w_diff = h->dev.get<int32_t>((size_t)grid * (ASM_CAP + 1));
-  A.w_edge = p.max_read_len > 256 ? h->dev.get<int2>((size_t)grid * spec_w * 2 * ASM_CAP) : nullptr;
-  A.w_lastcol = h->dev.get<uint2>((size_t)grid * spec_w * ASM_LASTCOL);
-  A.w_tab = getenv("BK_NW_PACKED") ? nullptr : h->dev.get<uint8_t>((size_t)grid * spec_w * NW_TAB_BYTES);   // (env: the packed-cell DP everywhere, for A/B runs)
+  if (long_path) {
+    long_assembly_scratch(h, B, p, R);
+  } else {
+    // speculation width and residency of the assembler (see assemble_kernel).  Auto = 4: one aligning warp per SM
+    // sub-partition; 8 warps share the four ALU pipes of the SM and finish a round no sooner (measured on C4).
+    int spec_w = h->spec_width;
+    if (const char* e = getenv("BK_SPEC_W")) spec_w = atoi(e);
+    if (spec_w <= 0) spec_w = 4;
+    spec_w = spec_w >= 8 ? 8 : (spec_w >= 4 ? 4 : (spec_w >= 2 ? 2 : 1));
+    int ctas_per_sm = spec_w == 8 ? 1 : (spec_w == 4 ? 3 : (spec_w == 2 ? 6 : 8));
+    if (const char* e = getenv("BK_ASM_CTAS_PER_SM")) ctas_per_sm = std::max(1, atoi(e));
+    int grid = (int)std::min<int64_t>(R, (int64_t)h->sm_count * ctas_per_sm);
+    if (grid < 1) grid = 1;
+    // dynamic shared memory: exactly what the kernel needs (padding it to bound residency starves L1: 15 % slower)
+    A.read_cap = (int)std::min<int64_t>(ASM_CAP, std::max<int64_t>(64, (p.max_read_len + 2 + 15) / 16 * 16));
+    B.spec_w = spec_w; B.ctas_per_sm = ctas_per_sm; B.grid = grid;
+    B.dyn_smem = (int)assemble_smem_bytes(spec_w, A.read_cap);
+    if (getenv("BK_ASM_PAD")) B.dyn_smem = std::max(B.dyn_smem, (int)((227 * 1024) / ctas_per_sm) - 1024);
+    A.w_cseq = h->dev.get<uint8_t>((size_t)grid * ASM_BUF);
+    A.w_cnt = h->dev.get<int32_t>((size_t)grid * 4 * ASM_BUF);
+    A.w_K = h->dev.get<int32_t>((size_t)grid * 4 * ASM_KCAP);
+    A.w_NK = h->dev.get<int32_t>((size_t)grid * 4 * ASM_KCAP);
+    A.w_wcode = h->dev.get<uint64_t>((size_t)grid * ASM_CAP);
+    A.w_diff = h->dev.get<int32_t>((size_t)grid * (ASM_CAP + 1));
+    A.w_edge = p.max_read_len > 256 ? h->dev.get<int2>((size_t)grid * spec_w * 2 * ASM_CAP) : nullptr;
+    A.w_lastcol = h->dev.get<uint2>((size_t)grid * spec_w * ASM_LASTCOL);
+    A.w_tab = getenv("BK_NW_PACKED") ? nullptr : h->dev.get<uint8_t>((size_t)grid * spec_w * NW_TAB_BYTES);   // (env: the packed-cell DP everywhere, for A/B runs)
+  }
   A.region_status = h->dev.get<int32_t>(R ? R : 1);
   A.region_ncontigs = h->dev.get<int32_t>(R ? R : 1);
   A.region_cells = h->dev.get<unsigned long long>(R ? R : 1);

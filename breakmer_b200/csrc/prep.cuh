@@ -171,7 +171,7 @@ __global__ void __launch_bounds__(32 * IDX_WARPS) index_emit_kernel(
     const int32_t* __restrict__ u_rec, int n_regions, const uint32_t* __restrict__ n_uniq_dev, const int64_t* __restrict__ so_off,
     const uint64_t* __restrict__ so_mer, int k, uint64_t* __restrict__ keys, uint32_t* __restrict__ vals,
     uint64_t* __restrict__ keys2, uint32_t* __restrict__ vals2, int u_bits, int s_bits, int ws_stride,
-    uint32_t* __restrict__ n_out, uint32_t cap) {
+    int32_t* __restrict__ ws_global, uint32_t* __restrict__ n_out, uint32_t cap) {
   extern __shared__ int32_t ws_all[];          // IDX_WARPS x ws_stride : local mer index of every window of the warp's read
   const int w = threadIdx.x >> 5, l = threadIdx.x & 31;
   int32_t* ws = ws_all + (size_t)w * ws_stride;
@@ -189,6 +189,7 @@ __global__ void __launch_bounds__(32 * IDX_WARPS) index_emit_kernel(
   const int rec = u_rec[u];
   const uint8_t* seq = rbases + roff[rec];
   const int len = (int)(roff[rec + 1] - roff[rec]);
+  if (ws_global) ws = ws_global + roff[rec];         // reads above the shared table's reach: one slot per base of the read
   const int nwin = len - k + 1;                        // find_reads sees the last window too (Q8)
   const uint64_t ulocal = (uint64_t)(u - u_off[region]);
   if (S == 0) return;

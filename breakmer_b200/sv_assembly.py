@@ -224,21 +224,14 @@ def _clean_mers(mers, kmer_len):
     return mers
 
 
-def init_assembly_batch(calls, device=0, on_capacity="raise"):
-    """calls: [(mers, fq_recs, kmer_len, rc_thresh, read_len), ...] with one common
-    kmer_len and rc_thresh -> list (per call) of contig lists.  One GPU pass.
-
-    A call whose region exceeds a device limit (a read longer than 4095 bases) does not disturb the others:
-    with on_capacity="raise" (default) a RuntimeError naming those calls is raised after every other call was completed
-    and stored in the exception's `.results`; with on_capacity="none" their entry in the returned list is None."""
+def _assemble_calls(calls, device, long):
+    """One device pass over `calls` -> (contig list or None per call, indices of the calls reported BK_ERR_CAPACITY)."""
     import numpy as np
-    if not calls:
-        return []
     inputs = [_AssemblyInput("r%d" % i, c[1], c[2], c[3]) for i, c in enumerate(calls)]
     pk = batch.PackedBatch(inputs, rc_thresh=int(calls[0][3]))
     pk.set_mers([_clean_mers(c[0], int(c[2])) for c in calls])
     pk.read_len = np.array([int(c[4]) for c in calls] + [0], dtype=np.int32)
-    out = batch.run(get_handle(device), pk)
+    out = batch.run(get_handle(device), pk, long=long)
     objs = [o for inp in inputs for o in inp.objs]
     result = []
     bad = []
@@ -248,9 +241,34 @@ def init_assembly_batch(calls, device=0, on_capacity="raise"):
             result.append(None)
             continue
         result.append([contig(out, cidx, objs, int(c[2])) for cidx in range(int(out.ctg_reg_off[i]), int(out.ctg_reg_off[i + 1]))])
-    if bad and on_capacity == "raise":
-        err = RuntimeError("init_assembly: device capacity exceeded in call(s) %s (a read or contig longer than 4095 bases); "
-                           "the other calls completed (see .results)" % bad)
+    return result, bad
+
+
+def init_assembly_batch(calls, device=0, on_capacity="raise"):
+    """calls: [(mers, fq_recs, kmer_len, rc_thresh, read_len), ...] with one common
+    kmer_len and rc_thresh -> list (per call) of contig lists.  One GPU pass.
+
+    A call whose region exceeds a limit of the batched assembler (a read or contig longer than 4095 bases) does not
+    disturb the others.  on_capacity says what happens to it:
+      "raise" (default)  a RuntimeError naming those calls is raised after every other call was completed, the results
+                         stored in the exception's `.results`;
+      "none"             their entry in the returned list is None;
+      "assemble"         they are run again through the long assembler (bk_compare_kmers_long, reads and contigs up to
+                         65,535 bases) and their contigs filled in; a RuntimeError as with "raise" names the calls that
+                         exceed that limit too."""
+    if not calls:
+        return []
+    result, bad = _assemble_calls(calls, device, False)
+    limit = 4095
+    if bad and on_capacity == "assemble":
+        again, still = _assemble_calls([calls[i] for i in bad], device, True)
+        for i, r in zip(bad, again):
+            result[i] = r
+        bad = [bad[j] for j in still]
+        limit = 65535
+    if bad and on_capacity in ("raise", "assemble"):
+        err = RuntimeError("init_assembly: device capacity exceeded in call(s) %s (a read or contig longer than %d bases); "
+                           "the other calls completed (see .results)" % (bad, limit))
         err.results = result
         raise err
     return result

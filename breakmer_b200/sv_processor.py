@@ -34,6 +34,8 @@ caller's; of these the rest of the reference only reads .id/.seq/.qual, SURVEY.m
 `write_contigs=True` additionally writes, for every contig of every target, the files
 contig.setup writes before blat (sv_processor.py:749-782) under target.paths['contigs'], on the
 library's host threads (bk_write_contigs, SURVEY.md section 8.7 f.3).
+`on_capacity="assemble"` runs the targets the batched assembler cannot take (a read or contig above
+4,095 bases) again through the long assembler (bk_compare_kmers_long, up to 65,535 bases).
 """
 import os
 
@@ -105,9 +107,10 @@ class _K:
 
 
 class CapacityError(RuntimeError):
-    """Some targets exceeded a device limit (a read or contig longer than 4095 bases).  Every other target of the
-    batch was completed; `.targets` lists the ones that were not (their state is untouched, so the reference's own
-    compare_kmers() can still be run on them)."""
+    """Some targets exceeded a device limit: a read or contig longer than 4095 bases (compare_kmers_batch's default
+    on_capacity="raise"), or longer than 65,535 bases (on_capacity="assemble", the long assembler's limit).  Every other
+    target of the batch was completed; `.targets` lists the ones that were not (their state is untouched, so the
+    reference's own compare_kmers() can still be run on them)."""
 
     def __init__(self, names):
         RuntimeError.__init__(self, "compare_kmers: device capacity exceeded for target(s) %s; all other targets completed"
@@ -181,7 +184,7 @@ def _pack_targets(targets, ingest, slot=0):
 
 
 def compare_kmers_batch(targets, device=0, ingest="python", write_contigs=False, devices=None, max_targets=125, inflight=4,
-                        apply_thread=False):
+                        apply_thread=False, on_capacity="raise"):
     """target.compare_kmers() for many targets (the region loop of sv_processor.py:185-201 as one call).
 
     The targets are cut into chunks of at most max_targets, most expensive first (static cost, breakmer_b200.shard), and
@@ -196,8 +199,13 @@ def compare_kmers_batch(targets, device=0, ingest="python", write_contigs=False,
     after it was submitted, whatever its size, and applying them is GIL-bound Python; the option pays when parsing is
     the larger share, i.e. big inputs per target.)
 
-    Targets that exceed a device limit do not disturb the others: everything else completes, then CapacityError lists
-    them (their state is untouched)."""
+    Targets that exceed a limit of the batched assembler (a read or contig above 4,095 bases) do not disturb the others.
+    With on_capacity="raise" (default) everything else completes, then CapacityError lists them (their state is
+    untouched).  With on_capacity="assemble" they are packed again (same ingest) and run through the long assembler
+    (bk_compare_kmers_long: reads and contigs up to 65,535 bases) on the first device, and their results applied like
+    every other target's (files included); CapacityError then lists only the targets beyond that limit."""
+    if on_capacity not in ("raise", "assemble"):
+        raise ValueError("on_capacity must be 'raise' or 'assemble'")
     if not targets:
         return
     if write_contigs and ingest != "native":
@@ -212,6 +220,13 @@ def compare_kmers_batch(targets, device=0, ingest="python", write_contigs=False,
         _apply_chunk(targets, pk, res, ks, objs, ingest, write_contigs, failed)
     else:
         _sharded(targets, devices, ingest, write_contigs, max_targets, inflight, failed, apply_thread)
+    if failed and on_capacity == "assemble":
+        names = set(failed)
+        redo = [t for t in targets if t.name in names]
+        failed = []
+        pk, ks, objs = _pack_targets(redo, ingest)
+        res = batch.run(get_handle(devices[0]), pk, decode=False, long=True)
+        _apply_chunk(redo, pk, res, ks, objs, ingest, write_contigs, failed)
     if failed:
         raise CapacityError(sorted(failed))
 

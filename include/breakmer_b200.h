@@ -36,7 +36,8 @@ extern "C" {
 #define BK_ERR_ARG (-2)
 #define BK_ERR_NOMEM (-3)
 #define BK_ERR_CAPACITY (-4)  /* a device-side hard limit is exceeded (a read or contig above 4095 bases inside the
-                                  batched assembler; bk_nw_batch itself has no length limit) */
+                                  batched assembler of bk_compare_kmers_batch, above 65535 bases in that of
+                                  bk_compare_kmers_long; bk_nw_batch itself has no length limit) */
 #define BK_ERR_EMPTY_SEQ (-5) /* olc.nw raises NameError on an empty sequence (olc.py:86-87) */
 #define BK_ERR_FORMAT (-6)    /* malformed FASTQ record (FastqFile raises, utils.py:704-719) */
 #define BK_ERR_IO (-7)        /* an input file cannot be read */
@@ -172,6 +173,14 @@ typedef struct bk_batch_result {
 } bk_batch_result;
 
 int bk_compare_kmers_batch(bk_handle_t h, const bk_batch_input* in, bk_batch_result* out);
+
+/* The same call for regions beyond the limits of bk_compare_kmers_batch's assembler: reads and contigs up to 65535
+ * bases (a region with a longer read, or whose contig would grow longer, or that starts more than 65535 contigs, is
+ * reported through region_status as BK_ERR_CAPACITY; the other regions are unaffected).  Same inputs, outputs and
+ * k-mer stage; the assembler runs one 256-thread CTA per region, without speculation, and aligns pairs above 4095
+ * bases with the anti-diagonal sweep of bk_nw_batch's long pairs.  Synchronous; meant for the few regions the batched
+ * call reports as BK_ERR_CAPACITY, not as a replacement for it. */
+int bk_compare_kmers_long(bk_handle_t h, const bk_batch_input* in, bk_batch_result* out);
 
 /* The same call in two halves, for callers that keep several batches in flight from ONE host thread (the region loop
  * of sv_processor.py:185-201 turned into a pipeline; one handle per batch in flight, several handles per GPU):
