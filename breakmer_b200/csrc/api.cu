@@ -26,6 +26,7 @@ struct bk_handle_s {
   cudaStream_t st = nullptr;
   int sm_count = 148;
   int spec_width = 0;      // assembler speculation width (bk_set_option); 0 = choose per batch
+  int long_regions = 0;    // bk_set_option "long_regions": the batched entries also assemble regions up to 65,535 bases
   cudaEvent_t sync_ev = nullptr;   // blocking-sync event (BK_BLOCKING_SYNC=1)
   bool spin_sync = true;
   Arena<false> dev;        // per-call device scratch
@@ -618,6 +619,9 @@ int bk_set_option(bk_handle_t h, const char* name, int64_t value) {
       h->spec_width = (int)value;
     } else if (strcmp(name, "blocking_sync") == 0) {
       h->spin_sync = value == 0;
+    } else if (strcmp(name, "long_regions") == 0) {
+      if (value != 0 && value != 1) fail(BK_ERR_ARG, "long_regions must be 0 or 1");
+      h->long_regions = (int)value;
     } else {
       fail(BK_ERR_ARG, "bk_set_option: unknown option %s", name);
     }

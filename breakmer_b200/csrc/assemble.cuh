@@ -1492,6 +1492,7 @@ struct AsmLongScratch {
   uint8_t* reads;                  // read_cap bytes per CTA (>= longest read + 2 and > NW_MAX_LEN)
   uint8_t* contig;                 // AsmCapLong::CAP bytes per CTA
   int32_t* diag;                   // 9 * (AsmCapLong::CAP + 1) ints per CTA: the sweep's rolling diagonals
+  const int* n_queue;              // device: length of P.work_order, written by route_long_kernel (null: P.n_regions)
 };
 
 #endif

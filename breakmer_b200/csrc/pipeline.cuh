@@ -58,6 +58,12 @@ struct Pipeline {
   std::vector<char> filt_bases;           // the filtered host copies (alive until the upload copies are done)
   std::vector<int64_t> filt_off, filt_reg_off;
   std::vector<uint8_t> filt_flags;
+  // the "long_regions" mode (bk_set_option), fixed at upload: regions with reads up to ASM_LONG_MAX_LEN bases are kept,
+  // and those with a read above NW_MAX_LEN go to assemble_long_kernel only
+  bool long_regions = false;
+  int n_routed = 0;                       // regions with a read above NW_MAX_LEN
+  const uint8_t* d_routed = nullptr;      // device, per region (null when n_routed == 0)
+  int max_short_read_len = 0;             // longest read of the other regions (sizes assemble_kernel's read buffers)
 };
 
 // everything submit() leaves behind for wait()
@@ -69,6 +75,18 @@ struct PendingBatch {
   int spec_w = 4, ctas_per_sm = 3, grid = 1, dyn_smem = 0;
   bool long_path = false;                  // bk_compare_kmers_long: assemble_long_kernel with its scratch L
   AsmLongScratch L{};
+  // the "long_regions" mode: assemble_kernel on the first n_short regions of the work order, route_long_kernel, then
+  // assemble_long_kernel (grid long_grid) on the device queue with A_long = A plus the long scratch
+  bool route = false;
+  int n_short = 0, long_grid = 0;
+  AsmParams A_long;                        // only its scratch fields (read_cap, w_*) are kept; the rest comes from A
+  int32_t* queue = nullptr;
+  int* n_queue = nullptr;
+  int* long_counter = nullptr;
+  unsigned long long* ctg_snapshot = nullptr;
+  const int32_t* h_queue = nullptr;        // pinned copies
+  const int* h_n_queue = nullptr;
+  const unsigned long long* h_snapshot = nullptr;
   uint8_t* zero_lo = nullptr;
   size_t zero_bytes = 0;
   unsigned long long cap_seq = 0;

@@ -70,9 +70,13 @@ void upload_record_set(bk_handle_t h, Arena<false>& A, const char* bases, const 
   h2d += n_bases + (n_rec + 1) * 8;
 }
 
-// max_len: the longest read the assembler of this call takes (NW_MAX_LEN, or ASM_LONG_MAX_LEN for bk_compare_kmers_long)
-void pipeline_upload_into(bk_handle_t h, Arena<false>& A, const bk_batch_input* in, Pipeline& p, int max_len = NW_MAX_LEN) {
+// max_len: the longest read the assembler of this call takes (NW_MAX_LEN, or ASM_LONG_MAX_LEN for bk_compare_kmers_long
+// and the "long_regions" mode).  long_regions: that mode (regions with a read above NW_MAX_LEN are marked for
+// assemble_long_kernel).
+void pipeline_upload_into(bk_handle_t h, Arena<false>& A, const bk_batch_input* in, Pipeline& p, int max_len = NW_MAX_LEN,
+                          bool long_regions = false) {
   p = Pipeline();
+  p.long_regions = long_regions;
   if (in->n_regions < 0 || in->n_regions > 65535) fail(BK_ERR_ARG, "batch: n_regions must be in 0..65535 per call");
   if (in->k < 2 || in->k > 31) fail(BK_ERR_ARG, "batch: k must be in 2..31");
   const int R = in->n_regions;
@@ -81,7 +85,8 @@ void pipeline_upload_into(bk_handle_t h, Arena<false>& A, const bk_batch_input* 
   // per-region read statistics; a region holding a read the assembler cannot take is left out of the device pass (its
   // region_status becomes BK_ERR_CAPACITY) instead of failing the call: the other regions are unaffected
   std::vector<int32_t> rl(R ? R : 1, 0);
-  int mx = 0;
+  std::vector<uint8_t> routed;
+  int mx = 0, mx_short = 0;
   int64_t n_skipped = 0;
   for (int r = 0; r < R; ++r) {
     if (in->read_reg_off[r + 1] < in->read_reg_off[r]) fail(BK_ERR_ARG, "batch: read region offsets not monotone");
@@ -95,10 +100,19 @@ void pipeline_upload_into(bk_handle_t h, Arena<false>& A, const bk_batch_input* 
       ++n_skipped;
     } else {
       mx = std::max(mx, m);
+      if (m <= NW_MAX_LEN) {
+        mx_short = std::max(mx_short, m);
+      } else if (long_regions) {
+        if (routed.empty()) routed.assign(R, 0);
+        routed[r] = 1;
+        ++p.n_routed;
+      }
       p.max_reg_records = std::max(p.max_reg_records, in->read_reg_off[r + 1] - in->read_reg_off[r]);
     }
   }
   p.max_read_len = mx;
+  p.max_short_read_len = mx_short;
+  if (p.n_routed) p.d_routed = to_device(h, A, routed.data(), (size_t)R);
   const char* read_bases = in->read_bases;
   const int64_t* read_off = in->read_off;
   const int64_t* read_reg_off = in->read_reg_off;
@@ -176,7 +190,8 @@ void pipeline_upload_into(bk_handle_t h, Arena<false>& A, const bk_batch_input* 
 void pipeline_upload(bk_handle_t h, const bk_batch_input* in) {
   h->resident.reset();
   h->pipe.reset(new Pipeline());
-  pipeline_upload_into(h, h->resident, in, *h->pipe);
+  const bool lr = h->long_regions != 0;
+  pipeline_upload_into(h, h->resident, in, *h->pipe, lr ? ASM_LONG_MAX_LEN : NW_MAX_LEN, lr);
   BK_CUDA(stream_wait(h));
 }
 
@@ -261,13 +276,10 @@ void ref_cache_build(bk_handle_t h, const char* ref_bases, const int64_t* ref_of
   h->ref_cache_mers = mers; h->ref_cache_koff = koff; h->ref_cache_regions = R; h->ref_cache_k = k;
 }
 
-// assemble_long_kernel's grid and per-CTA scratch: one CTA per region up to one per SM, contig-sized arrays for
-// AsmCapLong (a few MB per CTA), the staged read for the longest read of the call
-void long_assembly_scratch(bk_handle_t h, PendingBatch& B, const Pipeline& p, int R) {
-  AsmParams& A = B.A;
+// assemble_long_kernel's per-CTA scratch for `grid` CTAs: contig-sized arrays for AsmCapLong (about 11 MB per CTA), the
+// staged read for the longest read of the call
+void long_assembly_scratch(bk_handle_t h, AsmParams& A, AsmLongScratch& L, const Pipeline& p, int grid) {
   using C = AsmCapLong;
-  const int grid = (int)std::max<int64_t>(1, std::min<int64_t>(R, h->sm_count));
-  B.long_path = true; B.spec_w = 1; B.grid = grid; B.dyn_smem = 0;
   A.read_cap = (int)((std::max<int64_t>(NW_MAX_LEN + 1, p.max_read_len + 2) + 15) / 16 * 16);
   A.w_cseq = h->dev.get<uint8_t>((size_t)grid * C::BUF);
   A.w_cnt = h->dev.get<int32_t>((size_t)grid * 4 * C::BUF);
@@ -278,9 +290,28 @@ void long_assembly_scratch(bk_handle_t h, PendingBatch& B, const Pipeline& p, in
   A.w_edge = h->dev.get<int2>((size_t)grid * 2 * ASM_CAP);         // the warp DP's scratch (pairs within NW_MAX_LEN)
   A.w_lastcol = h->dev.get<uint2>((size_t)grid * ASM_LASTCOL);
   A.w_tab = h->dev.get<uint8_t>((size_t)grid * NW_TAB_BYTES);
-  B.L.reads = h->dev.get<uint8_t>((size_t)grid * A.read_cap);
-  B.L.contig = h->dev.get<uint8_t>((size_t)grid * C::CAP);
-  B.L.diag = h->dev.get<int32_t>((size_t)grid * 9 * (C::CAP + 1));
+  L.reads = h->dev.get<uint8_t>((size_t)grid * A.read_cap);
+  L.contig = h->dev.get<uint8_t>((size_t)grid * C::CAP);
+  L.diag = h->dev.get<int32_t>((size_t)grid * 9 * (C::CAP + 1));
+}
+
+// CTAs of assemble_long_kernel in the "long_regions" mode.  How many regions will overgrow in assemble_kernel is known
+// only on the device, so the grid is the regions routed at upload plus this allowance, within the SM count and R; the
+// CTAs are persistent, so a small grid is only slower.
+constexpr int LONG_ROUTE_SPARE_CTAS = 4;
+
+// assemble_kernel<W> at the width, residency and shared memory chosen at submit
+cudaError_t launch_assembly_batched(const PendingBatch& B, const AsmParams& A, cudaStream_t st) {
+  // shared-memory carve-out: just enough for the resident CTAs, the rest of the 256 KB stays L1
+  int carve = (int)((100 * (size_t)B.ctas_per_sm * ((size_t)B.dyn_smem + 1024) + 228 * 1024 - 1) / (228 * 1024));
+  if (const char* e = getenv("BK_ASM_CARVEOUT")) carve = atoi(e);
+  carve = std::min(100, std::max(0, carve));
+  if (B.spec_w == 8) return launch_assemble_w8(A, B.grid, B.dyn_smem, carve, st);
+  if (B.spec_w == 4 && B.ctas_per_sm >= 5) return launch_assemble_w4c5(A, B.grid, B.dyn_smem, carve, st);
+  if (B.spec_w == 4 && B.ctas_per_sm == 4) return launch_assemble_w4c4(A, B.grid, B.dyn_smem, carve, st);
+  if (B.spec_w == 4) return launch_assemble_w4(A, B.grid, B.dyn_smem, carve, st);
+  if (B.spec_w == 2) return launch_assemble_w2(A, B.grid, B.dyn_smem, carve, st);
+  return launch_assemble_w1(A, B.grid, B.dyn_smem, carve, st);
 }
 
 // (re)launch the assembler of a submitted batch: zero the mutable state, allocate the output arena for the current
@@ -301,20 +332,36 @@ void launch_assembly(bk_handle_t h, PendingBatch& B) {
   if (R > 0 && B.long_path) {
     TimedLaunch t(h->timers, st, KF_ASSEMBLE);
     BK_CUDA(launch_assemble_long(A, B.L, B.grid, st));
+  } else if (R > 0 && B.route) {
+    AsmParams S = A;                                       // assemble_kernel takes only the first n_short of the work order
+    S.n_regions = B.n_short;
+    if (B.n_short > 0) {
+      TimedLaunch t(h->timers, st, KF_ASSEMBLE);
+      BK_CUDA(launch_assembly_batched(B, S, st));
+    }
+    {
+      TimedLaunch t(h->timers, st, KF_PREP);
+      route_long_kernel<<<1, ROUTE_THREADS, 0, st>>>(A.work_order, B.n_short, R, A.region_status, A.out_cursor, B.queue, B.n_queue,
+                                                     B.ctg_snapshot);
+    }
+    AsmParams Lp = A;
+    Lp.read_cap = B.A_long.read_cap;
+    Lp.w_cseq = B.A_long.w_cseq; Lp.w_cnt = B.A_long.w_cnt; Lp.w_K = B.A_long.w_K; Lp.w_NK = B.A_long.w_NK;
+    Lp.w_wcode = B.A_long.w_wcode; Lp.w_diff = B.A_long.w_diff; Lp.w_edge = B.A_long.w_edge; Lp.w_lastcol = B.A_long.w_lastcol;
+    Lp.w_tab = B.A_long.w_tab;
+    Lp.work_counter = B.long_counter; Lp.work_order = B.queue;
+    TimedLaunch t(h->timers, st, KF_ASSEMBLE);
+    BK_CUDA(launch_assemble_long(Lp, B.L, B.long_grid, st));
   } else if (R > 0) {
     TimedLaunch t(h->timers, st, KF_ASSEMBLE);
-    // shared-memory carve-out: just enough for the resident CTAs, the rest of the 256 KB stays L1
-    int carve = (int)((100 * (size_t)B.ctas_per_sm * ((size_t)B.dyn_smem + 1024) + 228 * 1024 - 1) / (228 * 1024));
-    if (const char* e = getenv("BK_ASM_CARVEOUT")) carve = atoi(e);
-    carve = std::min(100, std::max(0, carve));
-    if (B.spec_w == 8) BK_CUDA(launch_assemble_w8(A, B.grid, B.dyn_smem, carve, st));
-    else if (B.spec_w == 4 && B.ctas_per_sm >= 5) BK_CUDA(launch_assemble_w4c5(A, B.grid, B.dyn_smem, carve, st));
-    else if (B.spec_w == 4 && B.ctas_per_sm == 4) BK_CUDA(launch_assemble_w4c4(A, B.grid, B.dyn_smem, carve, st));
-    else if (B.spec_w == 4) BK_CUDA(launch_assemble_w4(A, B.grid, B.dyn_smem, carve, st));
-    else if (B.spec_w == 2) BK_CUDA(launch_assemble_w2(A, B.grid, B.dyn_smem, carve, st));
-    else BK_CUDA(launch_assemble_w1(A, B.grid, B.dyn_smem, carve, st));
+    BK_CUDA(launch_assembly_batched(B, A, st));
   }
   BK_CUDA(cudaGetLastError());
+  if (B.route) {
+    B.h_queue = to_host(h, B.queue, (size_t)R);
+    B.h_n_queue = to_host(h, B.n_queue, 1);
+    B.h_snapshot = to_host(h, B.ctg_snapshot, 1);
+  }
   B.h_cursor = to_host(h, A.out_cursor, 5);
   B.h_stats = to_host(h, A.stats, 32);
   B.h_status = to_host(h, A.region_status, (size_t)(R ? R : 1));
@@ -323,6 +370,8 @@ void launch_assembly(bk_handle_t h, PendingBatch& B) {
 
 // Enqueue the whole device pass of one batch.  in == nullptr: the batch uploaded with bk_batch_upload.  long_path: the
 // assembler is assemble_long_kernel, and regions with reads up to ASM_LONG_MAX_LEN bases take part (bk_compare_kmers_long).
+// Otherwise the batch's "long_regions" mode (the handle's option when the inputs were uploaded) decides whether
+// assemble_long_kernel follows assemble_kernel in the same pass.
 void pipeline_submit(bk_handle_t h, const bk_batch_input* in, bool long_path = false) {
   cudaStream_t st = h->st;
   if (h->pending.active) fail(BK_ERR_ARG, "a batch is already in flight on this handle (call bk_batch_wait first)");
@@ -335,7 +384,8 @@ void pipeline_submit(bk_handle_t h, const bk_batch_input* in, bool long_path = f
     if (!h->pipe) fail(BK_ERR_ARG, "bk_compare_kmers_resident: no batch uploaded");
     B.p = h->pipe.get();
   } else {
-    pipeline_upload_into(h, h->dev, in, B.local, long_path ? ASM_LONG_MAX_LEN : NW_MAX_LEN);
+    const bool lr = !long_path && h->long_regions != 0;
+    pipeline_upload_into(h, h->dev, in, B.local, long_path || lr ? ASM_LONG_MAX_LEN : NW_MAX_LEN, lr);
     B.p = &B.local;
   }
   const Pipeline& p = *B.p;
@@ -506,7 +556,7 @@ void pipeline_submit(bk_handle_t h, const bk_batch_input* in, bool long_path = f
   int32_t* order = h->dev.get<int32_t>(R ? R : 1);
   if (R > 0) {
     TimedLaunch t(h->timers, st, KF_PREP);
-    work_order_kernel<<<1, 1024, 0, st>>>(so_off, u_off, R, order);
+    work_order_kernel<<<1, 1024, 0, st>>>(so_off, u_off, R, p.d_routed, order);
   }
 
   // ---- 5. assembly ----------------------------------------------------------------------------------------
@@ -520,8 +570,12 @@ void pipeline_submit(bk_handle_t h, const bk_batch_input* in, bool long_path = f
   A.post_off = post_off; A.post_read = post_read; A.post_pos = post_pos;
   A.work_order = order;
   if (long_path) {
-    long_assembly_scratch(h, B, p, R);
+    const int grid = (int)std::max<int64_t>(1, std::min<int64_t>(R, h->sm_count));     // one CTA per region up to one per SM
+    B.long_path = true; B.spec_w = 1; B.grid = grid; B.dyn_smem = 0;
+    long_assembly_scratch(h, B.A, B.L, p, grid);
   } else {
+    B.route = p.long_regions;
+    B.n_short = R - p.n_routed;
     // speculation width and residency of the assembler (see assemble_kernel).  Auto = 4: one aligning warp per SM
     // sub-partition; 8 warps share the four ALU pipes of the SM and finish a round no sooner (measured on C4).
     int spec_w = h->spec_width;
@@ -530,10 +584,10 @@ void pipeline_submit(bk_handle_t h, const bk_batch_input* in, bool long_path = f
     spec_w = spec_w >= 8 ? 8 : (spec_w >= 4 ? 4 : (spec_w >= 2 ? 2 : 1));
     int ctas_per_sm = spec_w == 8 ? 1 : (spec_w == 4 ? 3 : (spec_w == 2 ? 6 : 8));
     if (const char* e = getenv("BK_ASM_CTAS_PER_SM")) ctas_per_sm = std::max(1, atoi(e));
-    int grid = (int)std::min<int64_t>(R, (int64_t)h->sm_count * ctas_per_sm);
+    int grid = (int)std::min<int64_t>(B.n_short, (int64_t)h->sm_count * ctas_per_sm);
     if (grid < 1) grid = 1;
     // dynamic shared memory: exactly what the kernel needs (padding it to bound residency starves L1: 15 % slower)
-    A.read_cap = (int)std::min<int64_t>(ASM_CAP, std::max<int64_t>(64, (p.max_read_len + 2 + 15) / 16 * 16));
+    A.read_cap = (int)std::min<int64_t>(ASM_CAP, std::max<int64_t>(64, (p.max_short_read_len + 2 + 15) / 16 * 16));
     B.spec_w = spec_w; B.ctas_per_sm = ctas_per_sm; B.grid = grid;
     B.dyn_smem = (int)assemble_smem_bytes(spec_w, A.read_cap);
     if (getenv("BK_ASM_PAD")) B.dyn_smem = std::max(B.dyn_smem, (int)((227 * 1024) / ctas_per_sm) - 1024);
@@ -543,9 +597,14 @@ void pipeline_submit(bk_handle_t h, const bk_batch_input* in, bool long_path = f
     A.w_NK = h->dev.get<int32_t>((size_t)grid * 4 * ASM_KCAP);
     A.w_wcode = h->dev.get<uint64_t>((size_t)grid * ASM_CAP);
     A.w_diff = h->dev.get<int32_t>((size_t)grid * (ASM_CAP + 1));
-    A.w_edge = p.max_read_len > 256 ? h->dev.get<int2>((size_t)grid * spec_w * 2 * ASM_CAP) : nullptr;
+    A.w_edge = p.max_short_read_len > 256 ? h->dev.get<int2>((size_t)grid * spec_w * 2 * ASM_CAP) : nullptr;
     A.w_lastcol = h->dev.get<uint2>((size_t)grid * spec_w * ASM_LASTCOL);
     A.w_tab = getenv("BK_NW_PACKED") ? nullptr : h->dev.get<uint8_t>((size_t)grid * spec_w * NW_TAB_BYTES);   // (env: the packed-cell DP everywhere, for A/B runs)
+    if (B.route) {
+      B.long_grid = (int)std::max<int64_t>(1, std::min<int64_t>({(int64_t)p.n_routed + LONG_ROUTE_SPARE_CTAS, (int64_t)h->sm_count, (int64_t)R}));
+      long_assembly_scratch(h, B.A_long, B.L, p, B.long_grid);
+      B.queue = h->dev.get<int32_t>(R ? R : 1);
+    }
   }
   A.region_status = h->dev.get<int32_t>(R ? R : 1);
   A.region_ncontigs = h->dev.get<int32_t>(R ? R : 1);
@@ -560,7 +619,14 @@ void pipeline_submit(bk_handle_t h, const bk_batch_input* in, bool long_path = f
   const size_t o_mused = zalloc(SB), o_checked = zalloc(SB * 4), o_taken = zalloc(SB * 4), o_first = zalloc(SB * 4);
   const size_t o_rused = zalloc(NUB), o_rdel = zalloc(NUB), o_rq = zalloc(NUB), o_rbuf = zalloc(NUB * 4), o_rin = zalloc(NUB * 4);
   const size_t o_work = zalloc(sizeof(int)), o_cursor = zalloc(5 * sizeof(unsigned long long)), o_stats = zalloc(32 * sizeof(unsigned long long));
+  const size_t o_route = B.route ? zalloc(2 * sizeof(int) + sizeof(unsigned long long)) : 0;   // long counter, queue length, snapshot
   uint8_t* zero_lo = h->dev.get<uint8_t>(zero_bytes);
+  if (B.route) {
+    B.long_counter = (int*)(zero_lo + o_route);
+    B.n_queue = B.long_counter + 1;
+    B.ctg_snapshot = (unsigned long long*)(B.long_counter + 2);
+    B.L.n_queue = B.n_queue;
+  }
   B.zero_lo = zero_lo; B.zero_bytes = zero_bytes;
   A.m_used = zero_lo + o_mused; A.m_checked = (uint32_t*)(zero_lo + o_checked); A.m_taken = (uint32_t*)(zero_lo + o_taken); A.m_first = (uint32_t*)(zero_lo + o_first);
   A.r_used = zero_lo + o_rused; A.r_deleted = zero_lo + o_rdel; A.r_queued = zero_lo + o_rq;
@@ -617,8 +683,7 @@ void pipeline_wait(bk_handle_t h, bk_batch_result* out) {
   }
   const int64_t NU = B.h_counts[0], S_total = B.h_counts[1];
   const unsigned long long* h_cursor = B.h_cursor;
-  const int64_t n_ctg = (int64_t)h_cursor[4];
-  out->n_contigs = n_ctg;
+  const int64_t n_desc = (int64_t)h_cursor[4];
   out->n_check_align = (int64_t)B.h_stats[0];
   out->n_dp_cells = (int64_t)B.h_stats[1];
   if (getenv("BK_PHASE_PRINT")) phase_print(h, B);
@@ -631,7 +696,7 @@ void pipeline_wait(bk_handle_t h, bk_batch_result* out) {
   out->uniq_mult = to_host(h, B.u_mult, (size_t)NU);
   out->region_status = B.h_status;
   out->region_dp_cells = (const int64_t*)B.h_cells;
-  const int64_t* h_desc = to_host(h, A.o_desc, (size_t)n_ctg * 10);
+  const int64_t* h_desc = to_host(h, A.o_desc, (size_t)n_desc * 10);
   out->ctg_seq = (const char*)to_host(h, A.o_seq, (size_t)h_cursor[0]);
   out->ctg_kmer_locs = to_host(h, A.o_locs, (size_t)h_cursor[0]);
   out->ctg_indel_only = to_host(h, A.o_io, (size_t)h_cursor[1]);
@@ -649,8 +714,21 @@ void pipeline_wait(bk_handle_t h, bk_batch_result* out) {
 
   // contigs left the device in completion order; the table below puts them in
   // (region, acceptance order) -- payload arrays stay where they are
-  std::vector<int64_t> idx(n_ctg);
+  std::vector<int64_t> idx(n_desc);
   std::iota(idx.begin(), idx.end(), 0);
+  if (B.route) {
+    // a region assemble_long_kernel took over keeps only that kernel's contigs (descriptors from the snapshot on), and
+    // none if it failed there too; the payloads of the dropped descriptors stay unreferenced in the arrays
+    std::vector<uint8_t> rerouted(R ? R : 1, 0);
+    for (int i = 0; i < *B.h_n_queue; ++i) rerouted[B.h_queue[i]] = 1;
+    const int64_t snap = (int64_t)*B.h_snapshot;
+    idx.erase(std::remove_if(idx.begin(), idx.end(), [&](int64_t c) {
+                const int64_t r = h_desc[c * 10];
+                return rerouted[r] && (c < snap || B.h_status[r] != ST_OK);
+              }), idx.end());
+  }
+  const int64_t n_ctg = (int64_t)idx.size();
+  out->n_contigs = n_ctg;
   std::sort(idx.begin(), idx.end(), [&](int64_t a, int64_t b) {
     const int64_t* da = h_desc + a * 10; const int64_t* db = h_desc + b * 10;
     return da[0] != db[0] ? da[0] < db[0] : da[1] < db[1];

@@ -122,24 +122,28 @@ __global__ void __launch_bounds__(256) widen_scan_kernel(const uint32_t* __restr
 // Work order of the assembler: regions by descending cost class.  cost = unique reads x sample-only mers (the DP work of a
 // region grows with both); class = floor(8 * log2(cost + 1)) quantises it to 1/8 octave, which is all the longest-first
 // heuristic needs.  One block: histogram, scan, scatter (order inside a class is arbitrary; results never depend on it).
+// routed (or null): regions with a read above 4,095 bases in the "long_regions" mode; they come after all others (a
+// second set of classes), so that assemble_kernel, bounded to the others, never binds one.
 constexpr int WO_CLASSES = 512;
 __global__ void __launch_bounds__(1024) work_order_kernel(const int64_t* __restrict__ so_off, const int64_t* __restrict__ u_off,
-                                                          int n_regions, int32_t* __restrict__ order) {
-  __shared__ unsigned hist[WO_CLASSES];
-  __shared__ unsigned start[WO_CLASSES];
-  for (int c = threadIdx.x; c < WO_CLASSES; c += blockDim.x) hist[c] = 0;
+                                                          int n_regions, const uint8_t* __restrict__ routed,
+                                                          int32_t* __restrict__ order) {
+  __shared__ unsigned hist[2 * WO_CLASSES];
+  __shared__ unsigned start[2 * WO_CLASSES];
+  const int n_cls = routed ? 2 * WO_CLASSES : WO_CLASSES;
+  for (int c = threadIdx.x; c < n_cls; c += blockDim.x) hist[c] = 0;
   __syncthreads();
   auto cls = [&](int r) {
     const float cost = (float)(so_off[r + 1] - so_off[r]) * (float)(u_off[r + 1] - u_off[r]) + 1.0f;
     int c = (int)(8.0f * __log2f(cost));
     c = c < 0 ? 0 : (c > WO_CLASSES - 1 ? WO_CLASSES - 1 : c);
-    return WO_CLASSES - 1 - c;                       // ascending class = descending cost
+    return WO_CLASSES - 1 - c + (routed && routed[r] ? WO_CLASSES : 0);   // ascending class = descending cost
   };
   for (int r = threadIdx.x; r < n_regions; r += blockDim.x) atomicAdd(&hist[cls(r)], 1u);
   __syncthreads();
   if (threadIdx.x == 0) {
     unsigned run = 0;
-    for (int c = 0; c < WO_CLASSES; ++c) { start[c] = run; run += hist[c]; }
+    for (int c = 0; c < n_cls; ++c) { start[c] = run; run += hist[c]; }
   }
   __syncthreads();
   for (int r = threadIdx.x; r < n_regions; r += blockDim.x) order[atomicAdd(&start[cls(r)], 1u)] = r;

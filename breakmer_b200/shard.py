@@ -151,9 +151,10 @@ def digest_of_digests(by_name):
 
 class DevicePipeline:
     """`inflight` handles of one device driven by ONE host thread: submit keeps up to `inflight` batches queued on the
-    device (bk_batch_submit), results come back in submission order (bk_batch_wait)."""
+    device (bk_batch_submit), results come back in submission order (bk_batch_wait).  long_regions=True sets the
+    handles' "long_regions" option: regions with reads or contigs up to 65,535 bases are assembled in the same pass."""
 
-    def __init__(self, device, inflight=3, spec_width=0):
+    def __init__(self, device, inflight=3, spec_width=0, long_regions=False):
         from . import _lib
         self.device = device
         self.handles = [_lib.Handle(device) for _ in range(max(1, inflight))]
@@ -161,6 +162,8 @@ class DevicePipeline:
             h.set_option("blocking_sync", 1)           # a waiting host thread sleeps; it never competes with other GPUs' threads
             if spec_width:
                 h.set_option("spec_width", spec_width)
+            if long_regions:
+                h.set_option("long_regions", 1)
         self._queue = []                               # (handle index, packed, tag) in submission order
         self._next = 0
 
@@ -191,13 +194,14 @@ class DevicePipeline:
         self.handles = []
 
 
-def run_sharded(regions, devices=(0,), max_regions=2048, inflight=3, costs=None, pack=None, on_result=None):
+def run_sharded(regions, devices=(0,), max_regions=2048, inflight=3, costs=None, pack=None, on_result=None, long_regions=False):
     """The region loop of sv_processor.py:185-201 over several GPUs of one box, single process.
 
     regions     region-like objects (see batch.PackedBatch)
     devices     CUDA device ordinals; one host thread and `inflight` handles per device
     pack        callable(list of regions) -> PackedBatch (default batch.PackedBatch)
     on_result   callable(indices, BatchOutput, PackedBatch) called from the worker threads, once per chunk
+    long_regions  assemble regions with reads or contigs up to 65,535 bases in the same pass (DevicePipeline)
 
     Chunks of at most max_regions regions are handed out dynamically, most expensive first (static `region_cost`),
     so a device that drew cheap chunks simply takes more of them.  Returns {region name: (BatchOutput, index in it)}
@@ -226,7 +230,7 @@ def run_sharded(regions, devices=(0,), max_regions=2048, inflight=3, costs=None,
     def worker(dev):
         pipe = None
         try:
-            pipe = DevicePipeline(dev, inflight=inflight)
+            pipe = DevicePipeline(dev, inflight=inflight, long_regions=long_regions)
 
             def drain_one():
                 out, pk, idx = pipe.pop()

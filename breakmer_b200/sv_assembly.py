@@ -224,14 +224,23 @@ def _clean_mers(mers, kmer_len):
     return mers
 
 
-def _assemble_calls(calls, device, long):
-    """One device pass over `calls` -> (contig list or None per call, indices of the calls reported BK_ERR_CAPACITY)."""
+def _assemble_calls(calls, device, long_regions):
+    """One device pass over `calls` -> (contig list or None per call, indices of the calls reported BK_ERR_CAPACITY).
+    long_regions: the pass also assembles calls with reads or contigs up to 65,535 bases (the handle's option of that
+    name, set for this call only)."""
     import numpy as np
     inputs = [_AssemblyInput("r%d" % i, c[1], c[2], c[3]) for i, c in enumerate(calls)]
     pk = batch.PackedBatch(inputs, rc_thresh=int(calls[0][3]))
     pk.set_mers([_clean_mers(c[0], int(c[2])) for c in calls])
     pk.read_len = np.array([int(c[4]) for c in calls] + [0], dtype=np.int32)
-    out = batch.run(get_handle(device), pk, long=long)
+    h = get_handle(device)
+    if long_regions:
+        h.set_option("long_regions", 1)
+    try:
+        out = batch.run(h, pk)
+    finally:
+        if long_regions:
+            h.set_option("long_regions", 0)
     objs = [o for inp in inputs for o in inp.objs]
     result = []
     bad = []
@@ -253,19 +262,12 @@ def init_assembly_batch(calls, device=0, on_capacity="raise"):
       "raise" (default)  a RuntimeError naming those calls is raised after every other call was completed, the results
                          stored in the exception's `.results`;
       "none"             their entry in the returned list is None;
-      "assemble"         they are run again through the long assembler (bk_compare_kmers_long, reads and contigs up to
-                         65,535 bases) and their contigs filled in; a RuntimeError as with "raise" names the calls that
-                         exceed that limit too."""
+      "assemble"         the same pass assembles them too (the handle's "long_regions" option: reads and contigs up
+                         to 65,535 bases); a RuntimeError as with "raise" names the calls that exceed that limit."""
     if not calls:
         return []
-    result, bad = _assemble_calls(calls, device, False)
-    limit = 4095
-    if bad and on_capacity == "assemble":
-        again, still = _assemble_calls([calls[i] for i in bad], device, True)
-        for i, r in zip(bad, again):
-            result[i] = r
-        bad = [bad[j] for j in still]
-        limit = 65535
+    result, bad = _assemble_calls(calls, device, on_capacity == "assemble")
+    limit = 65535 if on_capacity == "assemble" else 4095
     if bad and on_capacity in ("raise", "assemble"):
         err = RuntimeError("init_assembly: device capacity exceeded in call(s) %s (a read or contig longer than %d bases); "
                            "the other calls completed (see .results)" % (bad, limit))

@@ -34,8 +34,8 @@ caller's; of these the rest of the reference only reads .id/.seq/.qual, SURVEY.m
 `write_contigs=True` additionally writes, for every contig of every target, the files
 contig.setup writes before blat (sv_processor.py:749-782) under target.paths['contigs'], on the
 library's host threads (bk_write_contigs, SURVEY.md section 8.7 f.3).
-`on_capacity="assemble"` runs the targets the batched assembler cannot take (a read or contig above
-4,095 bases) again through the long assembler (bk_compare_kmers_long, up to 65,535 bases).
+`on_capacity="assemble"` assembles targets with reads or contigs above 4,095 bases (up to 65,535) in the
+same device pass as all others (the handles' "long_regions" option).
 """
 import os
 
@@ -108,8 +108,8 @@ class _K:
 
 class CapacityError(RuntimeError):
     """Some targets exceeded a device limit: a read or contig longer than 4095 bases (compare_kmers_batch's default
-    on_capacity="raise"), or longer than 65,535 bases (on_capacity="assemble", the long assembler's limit).  Every other
-    target of the batch was completed; `.targets` lists the ones that were not (their state is untouched, so the
+    on_capacity="raise"), or longer than 65,535 bases (on_capacity="assemble", where the same pass assembles everything
+    up to that length).  Every other target of the batch was completed; `.targets` lists the ones that were not (their state is untouched, so the
     reference's own compare_kmers() can still be run on them)."""
 
     def __init__(self, names):
@@ -183,6 +183,14 @@ def _pack_targets(targets, ingest, slot=0):
     raise ValueError("ingest must be 'python' or 'native'")
 
 
+def _set_long_regions(handles, value):
+    """The "long_regions" option of handles this thread shares with later calls: set for one call, then 0 (the default)
+    again, so that a later default call on the same handles still reports the long targets.  Closed handles are skipped."""
+    for h in handles:
+        if h.h:
+            h.set_option("long_regions", value)
+
+
 def compare_kmers_batch(targets, device=0, ingest="python", write_contigs=False, devices=None, max_targets=125, inflight=4,
                         apply_thread=False, on_capacity="raise"):
     """target.compare_kmers() for many targets (the region loop of sv_processor.py:185-201 as one call).
@@ -201,9 +209,10 @@ def compare_kmers_batch(targets, device=0, ingest="python", write_contigs=False,
 
     Targets that exceed a limit of the batched assembler (a read or contig above 4,095 bases) do not disturb the others.
     With on_capacity="raise" (default) everything else completes, then CapacityError lists them (their state is
-    untouched).  With on_capacity="assemble" they are packed again (same ingest) and run through the long assembler
-    (bk_compare_kmers_long: reads and contigs up to 65,535 bases) on the first device, and their results applied like
-    every other target's (files included); CapacityError then lists only the targets beyond that limit."""
+    untouched).  With on_capacity="assemble" every call runs with the handles' "long_regions" option: such targets are
+    assembled in the same device pass as the others (reads and contigs up to 65,535 bases), on the device that ran their
+    chunk, and their results applied like every other target's (files included); CapacityError then lists only the
+    targets beyond that limit."""
     if on_capacity not in ("raise", "assemble"):
         raise ValueError("on_capacity must be 'raise' or 'assemble'")
     if not targets:
@@ -214,19 +223,20 @@ def compare_kmers_batch(targets, device=0, ingest="python", write_contigs=False,
         raise ValueError("ingest must be 'python' or 'native'")
     failed = []
     devices = list(devices) if devices else [device]
+    long_regions = on_capacity == "assemble"
     if len(targets) <= max_targets and len(devices) == 1:
         pk, ks, objs = _pack_targets(targets, ingest)
-        res = batch.run(get_handle(devices[0]), pk, decode=False)
+        h = get_handle(devices[0])
+        if long_regions:
+            _set_long_regions([h], 1)
+        try:
+            res = batch.run(h, pk, decode=False)
+        finally:
+            if long_regions:
+                _set_long_regions([h], 0)
         _apply_chunk(targets, pk, res, ks, objs, ingest, write_contigs, failed)
     else:
-        _sharded(targets, devices, ingest, write_contigs, max_targets, inflight, failed, apply_thread)
-    if failed and on_capacity == "assemble":
-        names = set(failed)
-        redo = [t for t in targets if t.name in names]
-        failed = []
-        pk, ks, objs = _pack_targets(redo, ingest)
-        res = batch.run(get_handle(devices[0]), pk, decode=False, long=True)
-        _apply_chunk(redo, pk, res, ks, objs, ingest, write_contigs, failed)
+        _sharded(targets, devices, ingest, write_contigs, max_targets, inflight, failed, apply_thread, long_regions)
     if failed:
         raise CapacityError(sorted(failed))
 
@@ -244,7 +254,7 @@ def _get_pipe(dev, inflight):
     return _pipes[key]
 
 
-def _sharded(targets, devices, ingest, write_contigs, max_targets, inflight, failed, apply_thread=False):
+def _sharded(targets, devices, ingest, write_contigs, max_targets, inflight, failed, apply_thread=False, long_regions=False):
     """Chunked, pipelined (and with several devices region-sharded) pass: sv_processor.py:185-201 over `devices`."""
     import threading
     costs = [_target_cost(t) for t in targets]
@@ -271,7 +281,12 @@ def _sharded(targets, devices, ingest, write_contigs, max_targets, inflight, fai
         n_sub = 0
         pipe = None
         try:
-            pipe = shard.DevicePipeline(dev, inflight=inflight) if own_pipe else _get_pipe(dev, inflight)
+            if own_pipe:
+                pipe = shard.DevicePipeline(dev, inflight=inflight, long_regions=long_regions)
+            else:
+                pipe = _get_pipe(dev, inflight)
+                if long_regions:
+                    _set_long_regions(pipe.handles, 1)
 
             # (the writer the applying thread uses: made here so that it is cached under the calling thread's key)
             apply_ing = _get_ingest("apply") if (apply_thread and ingest == "native") else None
@@ -355,6 +370,8 @@ def _sharded(targets, devices, ingest, write_contigs, max_targets, inflight, fai
         finally:
             if pipe is not None and own_pipe:
                 pipe.close()
+            elif pipe is not None and long_regions:
+                _set_long_regions(pipe.handles, 0)
 
     if len(devices) == 1:
         worker(devices[0], False)                        # one device: the calling thread drives it (handles are kept)

@@ -163,11 +163,14 @@ typedef struct bk_batch_result {
   const int32_t* region_status;      /* 0 or BK_ERR_CAPACITY per region */
   /* work counters of this call (for roofline arithmetic) */
   int64_t n_check_align;             /* contig.check_align calls (each = two olc.nw) */
-  int64_t n_dp_cells;                /* sum over those of len(contig)*len(read) (one sweep each) */
+  int64_t n_dp_cells;                /* sum over those of len(contig)*len(read) (one sweep each).  With the
+                                        "long_regions" option both count all device work of the call, including the
+                                        abandoned first attempt of a region the long assembler took over */
   int64_t n_kmer_occurrences;        /* k-mer windows of all inputs (reference forward + reverse, reads, soft clips, normal) */
   double  gpu_ms;                    /* device time of the call, CUDA events */
   int64_t n_sorted_keys;             /* windows that went through the sort (the sample's; the rest are streamed past) */
-  const int64_t* region_dp_cells;    /* per region: its share of n_dp_cells (cost models for sharding, shard.py) */
+  const int64_t* region_dp_cells;    /* per region: its share of n_dp_cells (cost models for sharding, shard.py); with
+                                        "long_regions", that of the pass that produced the region's result */
   double host_wait_ms;               /* bk_batch_wait: time blocked on the device ... */
   double host_post_ms;               /* ... and time spent building the result tables on the host */
 } bk_batch_result;
@@ -189,7 +192,8 @@ int bk_compare_kmers_long(bk_handle_t h, const bk_batch_input* in, bk_batch_resu
  * that pass is done and fills `out`.  in == NULL submits the batch uploaded with bk_batch_upload.  The input arrays
  * must stay valid and unchanged until bk_batch_submit returns (page-locked inputs, e.g. from bk_ingest_*: until
  * bk_batch_wait returns).  One batch in flight per handle.  A region holding a read longer than 4095 bases is left
- * out of the device pass and reported through region_status (BK_ERR_CAPACITY); the other regions are unaffected. */
+ * out of the device pass and reported through region_status (BK_ERR_CAPACITY); the other regions are unaffected
+ * (the handle's "long_regions" option, bk_set_option, assembles such regions in the same pass). */
 int bk_batch_submit(bk_handle_t h, const bk_batch_input* in);
 int bk_batch_wait(bk_handle_t h, bk_batch_result* out);
 
@@ -209,11 +213,21 @@ int bk_batch_upload(bk_handle_t h, const bk_batch_input* in);
 int bk_ref_cache_build(bk_handle_t h, const char* ref_bases, const int64_t* ref_off, int32_t n_regions, int32_t k);
 int bk_ref_cache_clear(bk_handle_t h);
 
-/* Tuning knobs.  "spec_width" = 0 | 1 | 2 | 4 | 8: warps per region in the assembler (how many
+/* Options of a handle.  "spec_width" = 0 | 1 | 2 | 4 | 8: warps per region in the assembler (how many
  * reads are aligned speculatively at once).  0 (default) = 4, one aligning warp per SM
  * sub-partition.  "blocking_sync" = 0 | 1: host threads waiting for the handle's stream spin (default, lowest
  * latency) or sleep on a blocking event (for hosts with fewer cores than handles in flight).  Results never
- * depend on either. */
+ * depend on either.
+ * "long_regions" = 0 | 1 changes which regions get results.  0 (default): the batched entries report a region with a
+ * read or contig above 4095 bases as BK_ERR_CAPACITY, as described above.  1: bk_compare_kmers_batch,
+ * bk_batch_submit / bk_batch_wait and bk_batch_upload + bk_compare_kmers_resident assemble such regions in the same
+ * device pass, up to 65535 bases, with the results bk_compare_kmers_long gives them: a region with a longer read is
+ * left out and reported as BK_ERR_CAPACITY, and so is a region the long assembler cannot finish either (its contig
+ * would grow past 65535 bases); such a region has no contigs in the result.  Contigs of a region's abandoned first
+ * attempt never appear.  The option is read when the inputs are uploaded (bk_batch_submit with inputs,
+ * bk_compare_kmers_batch, bk_batch_upload): a batch in flight or already uploaded keeps the mode it was uploaded
+ * with.  It costs device memory per call (scratch of the long assembler, about 11 MB per CTA for at least 4 CTAs)
+ * and two small launches; with 0 nothing extra is allocated or launched. */
 int bk_set_option(bk_handle_t h, const char* name, int64_t value);
 int bk_compare_kmers_resident(bk_handle_t h, bk_batch_result* out);
 int bk_kernel_times(bk_handle_t h, const char** names, const double** ms, const int64_t** launches, int32_t* n);
