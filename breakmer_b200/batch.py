@@ -7,6 +7,7 @@ the concatenated host arrays the ABI takes; `run` calls the library; `BatchOutpu
 gives per-region views of the result in the reference's own shapes
 ({mer: count} dicts, contig records).
 """
+import contextlib
 import ctypes
 
 import numpy as np
@@ -214,6 +215,21 @@ def run(handle, packed, resident=False, decode=True, long=False):
     if not decode:
         return res
     return BatchOutput(res, packed)
+
+
+@contextlib.contextmanager
+def long_regions(handles, on=True):
+    """The handles' "long_regions" option for the duration of a call (on=False: untouched), then 0 (the default) again,
+    so that later calls on handles the caller shares still report long regions.  Closed handles are skipped."""
+    def set_all(value):
+        for h in handles if on else ():
+            if h.h:
+                h.set_option("long_regions", value)
+    set_all(1)
+    try:
+        yield
+    finally:
+        set_all(0)
 
 
 def submit(handle, packed=None):

@@ -543,12 +543,12 @@ int bk_sample_only(bk_handle_t h, int k, const uint64_t* case_mers, const uint32
 }
 
 // On a failed submit the stream may hold work that uses the arenas: drain it so that the handle is reusable.
-static int submit_guarded(bk_handle_t h, const bk_batch_input* in, bool long_path = false) {
+static int submit_guarded(bk_handle_t h, const bk_batch_input* in, LongMode mode) {
   if (h && h->pending.active) {                     // refused without touching the batch that is in flight
     h->err = "a batch is already in flight on this handle (call bk_batch_wait first)";
     return BK_ERR_ARG;
   }
-  const int rc = guarded(h, [&] { pipeline_submit(h, in, long_path); });
+  const int rc = guarded(h, [&] { pipeline_submit(h, in, mode); });
   if (rc != BK_OK && h) { cudaStreamSynchronize(h->st); cudaGetLastError(); h->pending.active = false; }
   return rc;
 }
@@ -561,7 +561,7 @@ static int wait_guarded(bk_handle_t h, bk_batch_result* out) {
 
 int bk_batch_submit(bk_handle_t h, const bk_batch_input* in) {
   if (h && !in && !h->pipe) { h->err = "bk_batch_submit: null input and no batch uploaded"; return BK_ERR_ARG; }
-  return submit_guarded(h, in);
+  return submit_guarded(h, in, option_mode(h));
 }
 
 int bk_batch_wait(bk_handle_t h, bk_batch_result* out) {
@@ -571,13 +571,13 @@ int bk_batch_wait(bk_handle_t h, bk_batch_result* out) {
 
 int bk_compare_kmers_batch(bk_handle_t h, const bk_batch_input* in, bk_batch_result* out) {
   if (h && (!in || !out)) { h->err = "bk_compare_kmers_batch: null argument"; return BK_ERR_ARG; }
-  const int rc = submit_guarded(h, in);
+  const int rc = submit_guarded(h, in, option_mode(h));
   return rc != BK_OK ? rc : wait_guarded(h, out);
 }
 
 int bk_compare_kmers_long(bk_handle_t h, const bk_batch_input* in, bk_batch_result* out) {
   if (h && (!in || !out)) { h->err = "bk_compare_kmers_long: null argument"; return BK_ERR_ARG; }
-  const int rc = submit_guarded(h, in, true);
+  const int rc = submit_guarded(h, in, LONG_ALL);
   return rc != BK_OK ? rc : wait_guarded(h, out);
 }
 
@@ -591,7 +591,7 @@ int bk_batch_upload(bk_handle_t h, const bk_batch_input* in) {
 int bk_compare_kmers_resident(bk_handle_t h, bk_batch_result* out) {
   if (h && !out) { h->err = "bk_compare_kmers_resident: null argument"; return BK_ERR_ARG; }
   if (h && !h->pipe) { h->err = "bk_compare_kmers_resident: no batch uploaded"; return BK_ERR_ARG; }
-  const int rc = submit_guarded(h, nullptr);
+  const int rc = submit_guarded(h, nullptr, option_mode(h));
   return rc != BK_OK ? rc : wait_guarded(h, out);
 }
 

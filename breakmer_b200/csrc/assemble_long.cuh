@@ -18,9 +18,9 @@ BK_DEV void clear_region_state(const AsmParams& P, int region) {
   syncwarp();
 }
 
-// One CTA of NWL_THREADS threads per region slot, regions from the same queue as assemble_kernel.  Warp 0 runs the state
-// machine without speculation (width 1); all warps join the anti-diagonal sweep of a pair beyond the warp DP's 4,095
-// bases (long_round_dp).
+// One CTA of NWL_THREADS threads per region slot, regions from the queue route_long_kernel built (P.work_order, *L.n_queue
+// long).  Warp 0 runs the state machine without speculation (width 1); all warps join the anti-diagonal sweep of a pair
+// beyond the warp DP's 4,095 bases (long_round_dp).
 __global__ void __launch_bounds__(NWL_THREADS, 1) assemble_long_kernel(AsmParams P, AsmLongScratch L) {
   __shared__ int32_t s_hash[MER_HASH_SIZE];
   __shared__ SpecShared sp;
@@ -37,7 +37,7 @@ __global__ void __launch_bounds__(NWL_THREADS, 1) assemble_long_kernel(AsmParams
     }
   }
   RegionCtxT<AsmCapLong> c;
-  const int n_work = L.n_queue ? *L.n_queue : P.n_regions;
+  const int n_work = *L.n_queue;
   for (;;) {
     int w = 0;
     if (lane() == 0) w = atomicAdd(P.work_counter, 1);
@@ -60,11 +60,11 @@ __global__ void __launch_bounds__(NWL_THREADS, 1) assemble_long_kernel(AsmParams
   __syncthreads();
 }
 
-// The "long_regions" mode of the batched entries: after assemble_kernel, build assemble_long_kernel's queue on the
-// device.  order[n_short, n_regions) are the regions routed at upload (a read above 4,095 bases; assemble_kernel never
-// saw them), most expensive first; then, in work order, every region of order[0, n_short) that assemble_kernel finished
-// with ST_CAPACITY.  *ctg_snapshot = the contig cursor at this point: the descriptors below it are assemble_kernel's,
-// and those of a rerouted region are dropped from the result.  One block.
+// The long modes: after assemble_kernel, build assemble_long_kernel's queue on the device.  order[n_short, n_regions) are
+// the regions routed at upload (a read above 4,095 bases, or every region with n_short = 0 for bk_compare_kmers_long;
+// assemble_kernel never saw them), most expensive first; then, in work order, every region of order[0, n_short) that
+// assemble_kernel finished with ST_CAPACITY.  *ctg_snapshot = the contig cursor at this point: the descriptors below it
+// are assemble_kernel's, and those of a rerouted region are dropped from the result.  One block.
 constexpr int ROUTE_THREADS = 256;
 __global__ void __launch_bounds__(ROUTE_THREADS) route_long_kernel(const int32_t* __restrict__ order, int n_short, int n_regions,
                                                                    const int32_t* __restrict__ region_status,

@@ -28,6 +28,13 @@ struct RecordSet {          // one of: reads, soft clips, normal reads (device c
   int64_t max_reg_bases = 0;          // largest region (bases)
 };
 
+// Which regions the assembly of a call takes, and with which kernel
+enum LongMode {
+  LONG_OFF,     // reads up to NW_MAX_LEN bases, assemble_kernel only (the default)
+  LONG_ROUTE,   // reads up to ASM_LONG_MAX_LEN bases: assemble_kernel, then assemble_long_kernel (the "long_regions" option)
+  LONG_ALL,     // reads up to ASM_LONG_MAX_LEN bases, every region to assemble_long_kernel (bk_compare_kmers_long)
+};
+
 struct Pipeline {
   int n_regions = 0, k = 0, rc_thresh = 0, have_mers = 0;
   bool use_ref_cache = false;
@@ -58,12 +65,23 @@ struct Pipeline {
   std::vector<char> filt_bases;           // the filtered host copies (alive until the upload copies are done)
   std::vector<int64_t> filt_off, filt_reg_off;
   std::vector<uint8_t> filt_flags;
-  // the "long_regions" mode (bk_set_option), fixed at upload: regions with reads up to ASM_LONG_MAX_LEN bases are kept,
-  // and those with a read above NW_MAX_LEN go to assemble_long_kernel only
-  bool long_regions = false;
-  int n_routed = 0;                       // regions with a read above NW_MAX_LEN
-  const uint8_t* d_routed = nullptr;      // device, per region (null when n_routed == 0)
+  // the long assembler's mode, fixed at upload.  assemble_kernel takes the first n_short regions of the work order; in
+  // the long modes, assemble_long_kernel takes the others and those assemble_kernel stopped with ST_CAPACITY
+  LongMode long_mode = LONG_OFF;
+  int n_short = 0;                        // LONG_OFF: all; LONG_ROUTE: those without a read above NW_MAX_LEN; LONG_ALL: 0
+  const uint8_t* d_routed = nullptr;      // device, per region: a read above NW_MAX_LEN (LONG_ROUTE; null when none)
   int max_short_read_len = 0;             // longest read of the other regions (sizes assemble_kernel's read buffers)
+};
+
+// assemble_long_kernel's grid, scratch, queue and work counter in the long modes (long_assembly_scratch, long_params)
+struct LongAssembly {
+  int grid = 0, read_cap = 0;
+  uint8_t* w_cseq = nullptr; int32_t* w_cnt = nullptr; int32_t* w_K = nullptr; int32_t* w_NK = nullptr;
+  uint64_t* w_wcode = nullptr; int32_t* w_diff = nullptr; int2* w_edge = nullptr; uint2* w_lastcol = nullptr;
+  uint8_t* w_tab = nullptr;
+  int32_t* queue = nullptr;
+  int* counter = nullptr;
+  AsmLongScratch L{};
 };
 
 // everything submit() leaves behind for wait()
@@ -71,18 +89,12 @@ struct PendingBatch {
   bool active = false;
   const Pipeline* p = nullptr;
   Pipeline local;                          // non-resident submits own their Pipeline
-  AsmParams A;
+  AsmParams A;                             // assemble_kernel's; assemble_long_kernel's is long_params(A, LA)
   int spec_w = 4, ctas_per_sm = 3, grid = 1, dyn_smem = 0;
-  bool long_path = false;                  // bk_compare_kmers_long: assemble_long_kernel with its scratch L
-  AsmLongScratch L{};
-  // the "long_regions" mode: assemble_kernel on the first n_short regions of the work order, route_long_kernel, then
-  // assemble_long_kernel (grid long_grid) on the device queue with A_long = A plus the long scratch
+  // the long modes: after assemble_kernel (if n_short > 0), route_long_kernel, then assemble_long_kernel on the queue
   bool route = false;
-  int n_short = 0, long_grid = 0;
-  AsmParams A_long;                        // only its scratch fields (read_cap, w_*) are kept; the rest comes from A
-  int32_t* queue = nullptr;
+  LongAssembly LA;
   int* n_queue = nullptr;
-  int* long_counter = nullptr;
   unsigned long long* ctg_snapshot = nullptr;
   const int32_t* h_queue = nullptr;        // pinned copies
   const int* h_n_queue = nullptr;

@@ -7,7 +7,8 @@
 //                                                  -> candidate table -> probe (reference fwd + rc, normal) -> survivors
 //   3. k-mer -> read inverted index     prep.cuh   index_emit -> two radix sorts -> post_off / post_split
 //   4. work order                       prep.cuh   regions by descending cost class (one block)
-//   5. assembly                         assemble.cuh  one CTA per region slot, dynamic region queue
+//   5. assembly                         assemble.cuh  one CTA per region slot, dynamic region queue; in the long modes
+//                                                     (LongMode) then route_long_kernel and assemble_long_kernel
 //   6. results to pinned host memory
 //
 // The host never waits for the device between stages: every intermediate count (unique reads, candidates, sample-only
@@ -70,17 +71,17 @@ void upload_record_set(bk_handle_t h, Arena<false>& A, const char* bases, const 
   h2d += n_bases + (n_rec + 1) * 8;
 }
 
-// max_len: the longest read the assembler of this call takes (NW_MAX_LEN, or ASM_LONG_MAX_LEN for bk_compare_kmers_long
-// and the "long_regions" mode).  long_regions: that mode (regions with a read above NW_MAX_LEN are marked for
-// assemble_long_kernel).
-void pipeline_upload_into(bk_handle_t h, Arena<false>& A, const bk_batch_input* in, Pipeline& p, int max_len = NW_MAX_LEN,
-                          bool long_regions = false) {
+// Regions with a read above NW_MAX_LEN (ASM_LONG_MAX_LEN in the long modes) are left out; LONG_ROUTE marks those with a
+// read above NW_MAX_LEN for assemble_long_kernel.
+void pipeline_upload_into(bk_handle_t h, Arena<false>& A, const bk_batch_input* in, Pipeline& p, LongMode mode) {
   p = Pipeline();
-  p.long_regions = long_regions;
+  p.long_mode = mode;
+  const int max_len = mode == LONG_OFF ? NW_MAX_LEN : ASM_LONG_MAX_LEN;
   if (in->n_regions < 0 || in->n_regions > 65535) fail(BK_ERR_ARG, "batch: n_regions must be in 0..65535 per call");
   if (in->k < 2 || in->k > 31) fail(BK_ERR_ARG, "batch: k must be in 2..31");
   const int R = in->n_regions;
   p.n_regions = R; p.k = in->k; p.rc_thresh = in->rc_thresh; p.have_mers = in->have_mers;
+  p.n_short = mode == LONG_ALL ? 0 : R;
   if (!in->read_off || !in->read_reg_off) fail(BK_ERR_ARG, "batch: read arrays missing");
   // per-region read statistics; a region holding a read the assembler cannot take is left out of the device pass (its
   // region_status becomes BK_ERR_CAPACITY) instead of failing the call: the other regions are unaffected
@@ -102,17 +103,17 @@ void pipeline_upload_into(bk_handle_t h, Arena<false>& A, const bk_batch_input* 
       mx = std::max(mx, m);
       if (m <= NW_MAX_LEN) {
         mx_short = std::max(mx_short, m);
-      } else if (long_regions) {
+      } else if (mode == LONG_ROUTE) {
         if (routed.empty()) routed.assign(R, 0);
         routed[r] = 1;
-        ++p.n_routed;
+        --p.n_short;
       }
       p.max_reg_records = std::max(p.max_reg_records, in->read_reg_off[r + 1] - in->read_reg_off[r]);
     }
   }
   p.max_read_len = mx;
   p.max_short_read_len = mx_short;
-  if (p.n_routed) p.d_routed = to_device(h, A, routed.data(), (size_t)R);
+  if (!routed.empty()) p.d_routed = to_device(h, A, routed.data(), (size_t)R);
   const char* read_bases = in->read_bases;
   const int64_t* read_off = in->read_off;
   const int64_t* read_reg_off = in->read_reg_off;
@@ -187,11 +188,13 @@ void pipeline_upload_into(bk_handle_t h, Arena<false>& A, const bk_batch_input* 
   }
 }
 
+// the mode of the batched entries: the handle's "long_regions" option, read when their inputs are uploaded
+LongMode option_mode(bk_handle_t h) { return h && h->long_regions ? LONG_ROUTE : LONG_OFF; }
+
 void pipeline_upload(bk_handle_t h, const bk_batch_input* in) {
   h->resident.reset();
   h->pipe.reset(new Pipeline());
-  const bool lr = h->long_regions != 0;
-  pipeline_upload_into(h, h->resident, in, *h->pipe, lr ? ASM_LONG_MAX_LEN : NW_MAX_LEN, lr);
+  pipeline_upload_into(h, h->resident, in, *h->pipe, option_mode(h));
   BK_CUDA(stream_wait(h));
 }
 
@@ -276,29 +279,43 @@ void ref_cache_build(bk_handle_t h, const char* ref_bases, const int64_t* ref_of
   h->ref_cache_mers = mers; h->ref_cache_koff = koff; h->ref_cache_regions = R; h->ref_cache_k = k;
 }
 
-// assemble_long_kernel's per-CTA scratch for `grid` CTAs: contig-sized arrays for AsmCapLong (about 11 MB per CTA), the
-// staged read for the longest read of the call
-void long_assembly_scratch(bk_handle_t h, AsmParams& A, AsmLongScratch& L, const Pipeline& p, int grid) {
+// CTAs of assemble_long_kernel.  How many regions will overgrow in assemble_kernel is known only on the device, so the
+// grid is the regions routed at upload plus this allowance, within the SM count and R (with LONG_ALL: min(R, SM count));
+// the CTAs are persistent, so a small grid is only slower.
+constexpr int LONG_ROUTE_SPARE_CTAS = 4;
+
+// assemble_long_kernel's grid, queue and per-CTA scratch: contig-sized arrays for AsmCapLong (about 11 MB per CTA), the
+// staged read for the longest read of the call.  The work counter lives in the zeroed block (pipeline_submit).
+void long_assembly_scratch(bk_handle_t h, LongAssembly& S, const Pipeline& p) {
   using C = AsmCapLong;
-  A.read_cap = (int)((std::max<int64_t>(NW_MAX_LEN + 1, p.max_read_len + 2) + 15) / 16 * 16);
-  A.w_cseq = h->dev.get<uint8_t>((size_t)grid * C::BUF);
-  A.w_cnt = h->dev.get<int32_t>((size_t)grid * 4 * C::BUF);
-  A.w_K = h->dev.get<int32_t>((size_t)grid * 4 * C::KCAP);
-  A.w_NK = h->dev.get<int32_t>((size_t)grid * 4 * C::KCAP);
-  A.w_wcode = h->dev.get<uint64_t>((size_t)grid * C::CAP);
-  A.w_diff = h->dev.get<int32_t>((size_t)grid * (C::CAP + 1));
-  A.w_edge = h->dev.get<int2>((size_t)grid * 2 * ASM_CAP);         // the warp DP's scratch (pairs within NW_MAX_LEN)
-  A.w_lastcol = h->dev.get<uint2>((size_t)grid * ASM_LASTCOL);
-  A.w_tab = h->dev.get<uint8_t>((size_t)grid * NW_TAB_BYTES);
-  L.reads = h->dev.get<uint8_t>((size_t)grid * A.read_cap);
-  L.contig = h->dev.get<uint8_t>((size_t)grid * C::CAP);
-  L.diag = h->dev.get<int32_t>((size_t)grid * 9 * (C::CAP + 1));
+  const int R = p.n_regions;
+  const int grid = (int)std::max<int64_t>(1, std::min<int64_t>({(int64_t)(R - p.n_short) + LONG_ROUTE_SPARE_CTAS, (int64_t)h->sm_count, (int64_t)R}));
+  S.grid = grid;
+  S.read_cap = (int)((std::max<int64_t>(NW_MAX_LEN + 1, p.max_read_len + 2) + 15) / 16 * 16);
+  S.w_cseq = h->dev.get<uint8_t>((size_t)grid * C::BUF);
+  S.w_cnt = h->dev.get<int32_t>((size_t)grid * 4 * C::BUF);
+  S.w_K = h->dev.get<int32_t>((size_t)grid * 4 * C::KCAP);
+  S.w_NK = h->dev.get<int32_t>((size_t)grid * 4 * C::KCAP);
+  S.w_wcode = h->dev.get<uint64_t>((size_t)grid * C::CAP);
+  S.w_diff = h->dev.get<int32_t>((size_t)grid * (C::CAP + 1));
+  S.w_edge = h->dev.get<int2>((size_t)grid * 2 * ASM_CAP);         // the warp DP's scratch (pairs within NW_MAX_LEN)
+  S.w_lastcol = h->dev.get<uint2>((size_t)grid * ASM_LASTCOL);
+  S.w_tab = h->dev.get<uint8_t>((size_t)grid * NW_TAB_BYTES);
+  S.L.reads = h->dev.get<uint8_t>((size_t)grid * S.read_cap);
+  S.L.contig = h->dev.get<uint8_t>((size_t)grid * C::CAP);
+  S.L.diag = h->dev.get<int32_t>((size_t)grid * 9 * (C::CAP + 1));
+  S.queue = h->dev.get<int32_t>(R ? R : 1);
 }
 
-// CTAs of assemble_long_kernel in the "long_regions" mode.  How many regions will overgrow in assemble_kernel is known
-// only on the device, so the grid is the regions routed at upload plus this allowance, within the SM count and R; the
-// CTAs are persistent, so a small grid is only slower.
-constexpr int LONG_ROUTE_SPARE_CTAS = 4;
+// assemble_long_kernel's AsmParams: A with the long kernel's scratch, its queue as the work order and its own work
+// counter; the inputs, the per-region state and the output arena are A's
+AsmParams long_params(AsmParams A, const LongAssembly& S) {
+  A.read_cap = S.read_cap;
+  A.w_cseq = S.w_cseq; A.w_cnt = S.w_cnt; A.w_K = S.w_K; A.w_NK = S.w_NK; A.w_wcode = S.w_wcode; A.w_diff = S.w_diff;
+  A.w_edge = S.w_edge; A.w_lastcol = S.w_lastcol; A.w_tab = S.w_tab;
+  A.work_order = S.queue; A.work_counter = S.counter;
+  return A;
+}
 
 // assemble_kernel<W> at the width, residency and shared memory chosen at submit
 cudaError_t launch_assembly_batched(const PendingBatch& B, const AsmParams& A, cudaStream_t st) {
@@ -329,36 +346,25 @@ void launch_assembly(bk_handle_t h, PendingBatch& B) {
   A.o_kmer_meta = h->dev.get<int32_t>(A.cap_kmers);
   A.o_desc = h->dev.get<int64_t>(A.cap_ctg * 10);
   BK_CUDA(cudaMemsetAsync(B.zero_lo, 0, B.zero_bytes, st));
-  if (R > 0 && B.long_path) {
-    TimedLaunch t(h->timers, st, KF_ASSEMBLE);
-    BK_CUDA(launch_assemble_long(A, B.L, B.grid, st));
-  } else if (R > 0 && B.route) {
+  const int n_short = B.p->n_short;
+  if (n_short > 0) {
     AsmParams S = A;                                       // assemble_kernel takes only the first n_short of the work order
-    S.n_regions = B.n_short;
-    if (B.n_short > 0) {
-      TimedLaunch t(h->timers, st, KF_ASSEMBLE);
-      BK_CUDA(launch_assembly_batched(B, S, st));
-    }
+    S.n_regions = n_short;
+    TimedLaunch t(h->timers, st, KF_ASSEMBLE);
+    BK_CUDA(launch_assembly_batched(B, S, st));
+  }
+  if (R > 0 && B.route) {
     {
       TimedLaunch t(h->timers, st, KF_PREP);
-      route_long_kernel<<<1, ROUTE_THREADS, 0, st>>>(A.work_order, B.n_short, R, A.region_status, A.out_cursor, B.queue, B.n_queue,
+      route_long_kernel<<<1, ROUTE_THREADS, 0, st>>>(A.work_order, n_short, R, A.region_status, A.out_cursor, B.LA.queue, B.n_queue,
                                                      B.ctg_snapshot);
     }
-    AsmParams Lp = A;
-    Lp.read_cap = B.A_long.read_cap;
-    Lp.w_cseq = B.A_long.w_cseq; Lp.w_cnt = B.A_long.w_cnt; Lp.w_K = B.A_long.w_K; Lp.w_NK = B.A_long.w_NK;
-    Lp.w_wcode = B.A_long.w_wcode; Lp.w_diff = B.A_long.w_diff; Lp.w_edge = B.A_long.w_edge; Lp.w_lastcol = B.A_long.w_lastcol;
-    Lp.w_tab = B.A_long.w_tab;
-    Lp.work_counter = B.long_counter; Lp.work_order = B.queue;
     TimedLaunch t(h->timers, st, KF_ASSEMBLE);
-    BK_CUDA(launch_assemble_long(Lp, B.L, B.long_grid, st));
-  } else if (R > 0) {
-    TimedLaunch t(h->timers, st, KF_ASSEMBLE);
-    BK_CUDA(launch_assembly_batched(B, A, st));
+    BK_CUDA(launch_assemble_long(long_params(A, B.LA), B.LA.L, B.LA.grid, st));
   }
   BK_CUDA(cudaGetLastError());
   if (B.route) {
-    B.h_queue = to_host(h, B.queue, (size_t)R);
+    B.h_queue = to_host(h, B.LA.queue, (size_t)R);
     B.h_n_queue = to_host(h, B.n_queue, 1);
     B.h_snapshot = to_host(h, B.ctg_snapshot, 1);
   }
@@ -368,11 +374,10 @@ void launch_assembly(bk_handle_t h, PendingBatch& B) {
   B.h_cells = to_host(h, A.region_cells, (size_t)(R ? R : 1));
 }
 
-// Enqueue the whole device pass of one batch.  in == nullptr: the batch uploaded with bk_batch_upload.  long_path: the
-// assembler is assemble_long_kernel, and regions with reads up to ASM_LONG_MAX_LEN bases take part (bk_compare_kmers_long).
-// Otherwise the batch's "long_regions" mode (the handle's option when the inputs were uploaded) decides whether
-// assemble_long_kernel follows assemble_kernel in the same pass.
-void pipeline_submit(bk_handle_t h, const bk_batch_input* in, bool long_path = false) {
+// Enqueue the whole device pass of one batch.  in == nullptr: the batch uploaded with bk_batch_upload, in the mode it was
+// uploaded with.  Otherwise mode: LONG_ALL for bk_compare_kmers_long (assemble_kernel gets no regions and is not
+// launched), option_mode(h) for the batched entries.
+void pipeline_submit(bk_handle_t h, const bk_batch_input* in, LongMode mode) {
   cudaStream_t st = h->st;
   if (h->pending.active) fail(BK_ERR_ARG, "a batch is already in flight on this handle (call bk_batch_wait first)");
   h->dev.reset();
@@ -384,8 +389,7 @@ void pipeline_submit(bk_handle_t h, const bk_batch_input* in, bool long_path = f
     if (!h->pipe) fail(BK_ERR_ARG, "bk_compare_kmers_resident: no batch uploaded");
     B.p = h->pipe.get();
   } else {
-    const bool lr = !long_path && h->long_regions != 0;
-    pipeline_upload_into(h, h->dev, in, B.local, long_path || lr ? ASM_LONG_MAX_LEN : NW_MAX_LEN, lr);
+    pipeline_upload_into(h, h->dev, in, B.local, mode);
     B.p = &B.local;
   }
   const Pipeline& p = *B.p;
@@ -569,13 +573,7 @@ void pipeline_submit(bk_handle_t h, const bk_batch_input* in, bool long_path = f
   A.so_off = so_off; A.so_mer = so_mer; A.so_cnt = so_cnt;
   A.post_off = post_off; A.post_read = post_read; A.post_pos = post_pos;
   A.work_order = order;
-  if (long_path) {
-    const int grid = (int)std::max<int64_t>(1, std::min<int64_t>(R, h->sm_count));     // one CTA per region up to one per SM
-    B.long_path = true; B.spec_w = 1; B.grid = grid; B.dyn_smem = 0;
-    long_assembly_scratch(h, B.A, B.L, p, grid);
-  } else {
-    B.route = p.long_regions;
-    B.n_short = R - p.n_routed;
+  if (p.n_short > 0) {
     // speculation width and residency of the assembler (see assemble_kernel).  Auto = 4: one aligning warp per SM
     // sub-partition; 8 warps share the four ALU pipes of the SM and finish a round no sooner (measured on C4).
     int spec_w = h->spec_width;
@@ -584,8 +582,7 @@ void pipeline_submit(bk_handle_t h, const bk_batch_input* in, bool long_path = f
     spec_w = spec_w >= 8 ? 8 : (spec_w >= 4 ? 4 : (spec_w >= 2 ? 2 : 1));
     int ctas_per_sm = spec_w == 8 ? 1 : (spec_w == 4 ? 3 : (spec_w == 2 ? 6 : 8));
     if (const char* e = getenv("BK_ASM_CTAS_PER_SM")) ctas_per_sm = std::max(1, atoi(e));
-    int grid = (int)std::min<int64_t>(B.n_short, (int64_t)h->sm_count * ctas_per_sm);
-    if (grid < 1) grid = 1;
+    const int grid = (int)std::min<int64_t>(p.n_short, (int64_t)h->sm_count * ctas_per_sm);
     // dynamic shared memory: exactly what the kernel needs (padding it to bound residency starves L1: 15 % slower)
     A.read_cap = (int)std::min<int64_t>(ASM_CAP, std::max<int64_t>(64, (p.max_short_read_len + 2 + 15) / 16 * 16));
     B.spec_w = spec_w; B.ctas_per_sm = ctas_per_sm; B.grid = grid;
@@ -600,12 +597,9 @@ void pipeline_submit(bk_handle_t h, const bk_batch_input* in, bool long_path = f
     A.w_edge = p.max_short_read_len > 256 ? h->dev.get<int2>((size_t)grid * spec_w * 2 * ASM_CAP) : nullptr;
     A.w_lastcol = h->dev.get<uint2>((size_t)grid * spec_w * ASM_LASTCOL);
     A.w_tab = getenv("BK_NW_PACKED") ? nullptr : h->dev.get<uint8_t>((size_t)grid * spec_w * NW_TAB_BYTES);   // (env: the packed-cell DP everywhere, for A/B runs)
-    if (B.route) {
-      B.long_grid = (int)std::max<int64_t>(1, std::min<int64_t>({(int64_t)p.n_routed + LONG_ROUTE_SPARE_CTAS, (int64_t)h->sm_count, (int64_t)R}));
-      long_assembly_scratch(h, B.A_long, B.L, p, B.long_grid);
-      B.queue = h->dev.get<int32_t>(R ? R : 1);
-    }
   }
+  B.route = p.long_mode != LONG_OFF;
+  if (B.route) long_assembly_scratch(h, B.LA, p);
   A.region_status = h->dev.get<int32_t>(R ? R : 1);
   A.region_ncontigs = h->dev.get<int32_t>(R ? R : 1);
   A.region_cells = h->dev.get<unsigned long long>(R ? R : 1);
@@ -622,10 +616,10 @@ void pipeline_submit(bk_handle_t h, const bk_batch_input* in, bool long_path = f
   const size_t o_route = B.route ? zalloc(2 * sizeof(int) + sizeof(unsigned long long)) : 0;   // long counter, queue length, snapshot
   uint8_t* zero_lo = h->dev.get<uint8_t>(zero_bytes);
   if (B.route) {
-    B.long_counter = (int*)(zero_lo + o_route);
-    B.n_queue = B.long_counter + 1;
-    B.ctg_snapshot = (unsigned long long*)(B.long_counter + 2);
-    B.L.n_queue = B.n_queue;
+    B.LA.counter = (int*)(zero_lo + o_route);
+    B.n_queue = B.LA.counter + 1;
+    B.ctg_snapshot = (unsigned long long*)(B.LA.counter + 2);
+    B.LA.L.n_queue = B.n_queue;
   }
   B.zero_lo = zero_lo; B.zero_bytes = zero_bytes;
   A.m_used = zero_lo + o_mused; A.m_checked = (uint32_t*)(zero_lo + o_checked); A.m_taken = (uint32_t*)(zero_lo + o_taken); A.m_first = (uint32_t*)(zero_lo + o_first);
@@ -718,7 +712,7 @@ void pipeline_wait(bk_handle_t h, bk_batch_result* out) {
   std::iota(idx.begin(), idx.end(), 0);
   if (B.route) {
     // a region assemble_long_kernel took over keeps only that kernel's contigs (descriptors from the snapshot on), and
-    // none if it failed there too; the payloads of the dropped descriptors stay unreferenced in the arrays
+    // none if it failed there too (LONG_ALL: the snapshot is 0); the dropped descriptors' payloads stay unreferenced
     std::vector<uint8_t> rerouted(R ? R : 1, 0);
     for (int i = 0; i < *B.h_n_queue; ++i) rerouted[B.h_queue[i]] = 1;
     const int64_t snap = (int64_t)*B.h_snapshot;

@@ -234,13 +234,8 @@ def _assemble_calls(calls, device, long_regions):
     pk.set_mers([_clean_mers(c[0], int(c[2])) for c in calls])
     pk.read_len = np.array([int(c[4]) for c in calls] + [0], dtype=np.int32)
     h = get_handle(device)
-    if long_regions:
-        h.set_option("long_regions", 1)
-    try:
+    with batch.long_regions([h], long_regions):
         out = batch.run(h, pk)
-    finally:
-        if long_regions:
-            h.set_option("long_regions", 0)
     objs = [o for inp in inputs for o in inp.objs]
     result = []
     bad = []

@@ -183,14 +183,6 @@ def _pack_targets(targets, ingest, slot=0):
     raise ValueError("ingest must be 'python' or 'native'")
 
 
-def _set_long_regions(handles, value):
-    """The "long_regions" option of handles this thread shares with later calls: set for one call, then 0 (the default)
-    again, so that a later default call on the same handles still reports the long targets.  Closed handles are skipped."""
-    for h in handles:
-        if h.h:
-            h.set_option("long_regions", value)
-
-
 def compare_kmers_batch(targets, device=0, ingest="python", write_contigs=False, devices=None, max_targets=125, inflight=4,
                         apply_thread=False, on_capacity="raise"):
     """target.compare_kmers() for many targets (the region loop of sv_processor.py:185-201 as one call).
@@ -227,13 +219,8 @@ def compare_kmers_batch(targets, device=0, ingest="python", write_contigs=False,
     if len(targets) <= max_targets and len(devices) == 1:
         pk, ks, objs = _pack_targets(targets, ingest)
         h = get_handle(devices[0])
-        if long_regions:
-            _set_long_regions([h], 1)
-        try:
+        with batch.long_regions([h], long_regions):
             res = batch.run(h, pk, decode=False)
-        finally:
-            if long_regions:
-                _set_long_regions([h], 0)
         _apply_chunk(targets, pk, res, ks, objs, ingest, write_contigs, failed)
     else:
         _sharded(targets, devices, ingest, write_contigs, max_targets, inflight, failed, apply_thread, long_regions)
@@ -281,87 +268,82 @@ def _sharded(targets, devices, ingest, write_contigs, max_targets, inflight, fai
         n_sub = 0
         pipe = None
         try:
-            if own_pipe:
-                pipe = shard.DevicePipeline(dev, inflight=inflight, long_regions=long_regions)
-            else:
-                pipe = _get_pipe(dev, inflight)
-                if long_regions:
-                    _set_long_regions(pipe.handles, 1)
+            pipe = shard.DevicePipeline(dev, inflight=inflight) if own_pipe else _get_pipe(dev, inflight)
+            with batch.long_regions(pipe.handles, long_regions):
+                # (the writer the applying thread uses: made here so that it is cached under the calling thread's key)
+                apply_ing = _get_ingest("apply") if (apply_thread and ingest == "native") else None
 
-            # (the writer the applying thread uses: made here so that it is cached under the calling thread's key)
-            apply_ing = _get_ingest("apply") if (apply_thread and ingest == "native") else None
+                def drain_one():
+                    res, pk, tag = pipe.pop(decode=False)
+                    chunk, ks, objs = tag
+                    mine = []
+                    _apply_chunk(chunk, pk, res, ks, objs, ingest, write_contigs, mine, apply_ing)
+                    with lock:
+                        failed.extend(mine)
 
-            def drain_one():
-                res, pk, tag = pipe.pop(decode=False)
-                chunk, ks, objs = tag
-                mine = []
-                _apply_chunk(chunk, pk, res, ks, objs, ingest, write_contigs, mine, apply_ing)
-                with lock:
-                    failed.extend(mine)
+                if apply_thread:
+                    # this thread parses and submits; a second one takes the results in submission order and applies them.
+                    # A handle is free again only when its chunk has been applied (the result arrays live in its arena).
+                    free = threading.Semaphore(inflight)
+                    submitted = []                           # grows by append only; the applier follows it by index
+                    more = threading.Condition()
+                    state = {"done": False}
 
-            if apply_thread:
-                # this thread parses and submits; a second one takes the results in submission order and applies them.
-                # A handle is free again only when its chunk has been applied (the result arrays live in its arena).
-                free = threading.Semaphore(inflight)
-                submitted = []                           # grows by append only; the applier follows it by index
-                more = threading.Condition()
-                state = {"done": False}
-
-                def applier():
-                    at = 0
-                    try:
-                        while True:
-                            with more:
-                                while at >= len(submitted) and not state["done"]:
-                                    more.wait()
-                                if at >= len(submitted):
-                                    return
-                            at += 1
-                            drain_one()
+                    def applier():
+                        at = 0
+                        try:
+                            while True:
+                                with more:
+                                    while at >= len(submitted) and not state["done"]:
+                                        more.wait()
+                                    if at >= len(submitted):
+                                        return
+                                at += 1
+                                drain_one()
+                                free.release()
+                        except Exception as e:               # noqa: BLE001 -- re-raised on the calling thread
+                            errors.append(e)
+                            state["failed"] = True
                             free.release()
-                    except Exception as e:               # noqa: BLE001 -- re-raised on the calling thread
-                        errors.append(e)
-                        state["failed"] = True
-                        free.release()
 
-                helper = threading.Thread(target=applier)
-                helper.start()
-                try:
-                    while not state.get("failed"):
-                        idx = take()
-                        if idx is None:
-                            break
-                        chunk = [targets[i] for i in idx]
-                        pk, ks, objs = _pack_targets(chunk, ingest, slot=n_sub % (inflight + 1))
-                        free.acquire()
-                        if state.get("failed"):
-                            break
-                        n_sub += 1
-                        pipe.submit(pk, (chunk, ks, objs))
+                    helper = threading.Thread(target=applier)
+                    helper.start()
+                    try:
+                        while not state.get("failed"):
+                            idx = take()
+                            if idx is None:
+                                break
+                            chunk = [targets[i] for i in idx]
+                            pk, ks, objs = _pack_targets(chunk, ingest, slot=n_sub % (inflight + 1))
+                            free.acquire()
+                            if state.get("failed"):
+                                break
+                            n_sub += 1
+                            pipe.submit(pk, (chunk, ks, objs))
+                            with more:
+                                submitted.append(n_sub)
+                                more.notify()
+                    finally:
                         with more:
-                            submitted.append(n_sub)
+                            state["done"] = True
                             more.notify()
-                finally:
-                    with more:
-                        state["done"] = True
-                        more.notify()
-                    helper.join()
-                if state.get("failed"):
-                    raise errors.pop()
-                return
-            while True:
-                idx = take()
-                if idx is None:
-                    break
-                chunk = [targets[i] for i in idx]
-                if pipe.full():
+                        helper.join()
+                    if state.get("failed"):
+                        raise errors.pop()
+                    return
+                while True:
+                    idx = take()
+                    if idx is None:
+                        break
+                    chunk = [targets[i] for i in idx]
+                    if pipe.full():
+                        drain_one()
+                    # (a native ingest buffer is reused call to call: `inflight` of them rotate under the batches in flight)
+                    pk, ks, objs = _pack_targets(chunk, ingest, slot=n_sub % inflight)
+                    n_sub += 1
+                    pipe.submit(pk, (chunk, ks, objs))
+                while pipe.pending():
                     drain_one()
-                # (a native ingest buffer is reused call to call: `inflight` of them rotate under the batches in flight)
-                pk, ks, objs = _pack_targets(chunk, ingest, slot=n_sub % inflight)
-                n_sub += 1
-                pipe.submit(pk, (chunk, ks, objs))
-            while pipe.pending():
-                drain_one()
         except Exception as e:                           # noqa: BLE001 -- re-raised on the calling thread
             errors.append(e)
             if pipe is not None and not own_pipe:        # a cached pipeline with batches in flight is not reusable
@@ -370,8 +352,6 @@ def _sharded(targets, devices, ingest, write_contigs, max_targets, inflight, fai
         finally:
             if pipe is not None and own_pipe:
                 pipe.close()
-            elif pipe is not None and long_regions:
-                _set_long_regions(pipe.handles, 0)
 
     if len(devices) == 1:
         worker(devices[0], False)                        # one device: the calling thread drives it (handles are kept)

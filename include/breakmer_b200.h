@@ -179,10 +179,11 @@ int bk_compare_kmers_batch(bk_handle_t h, const bk_batch_input* in, bk_batch_res
 
 /* The same call for regions beyond the limits of bk_compare_kmers_batch's assembler: reads and contigs up to 65535
  * bases (a region with a longer read, or whose contig would grow longer, or that starts more than 65535 contigs, is
- * reported through region_status as BK_ERR_CAPACITY; the other regions are unaffected).  Same inputs, outputs and
- * k-mer stage; the assembler runs one 256-thread CTA per region, without speculation, and aligns pairs above 4095
- * bases with the anti-diagonal sweep of bk_nw_batch's long pairs.  Synchronous; meant for the few regions the batched
- * call reports as BK_ERR_CAPACITY, not as a replacement for it. */
+ * reported through region_status as BK_ERR_CAPACITY, with no contigs in the result; the other regions are unaffected).
+ * Same inputs, outputs and k-mer stage; it is the "long_regions" pass (bk_set_option) with every region given to the
+ * long assembler, which runs one 256-thread CTA per region, without speculation, and aligns pairs above 4095 bases
+ * with the anti-diagonal sweep of bk_nw_batch's long pairs.  Synchronous; meant for the few regions the batched call
+ * reports as BK_ERR_CAPACITY, not as a replacement for it. */
 int bk_compare_kmers_long(bk_handle_t h, const bk_batch_input* in, bk_batch_result* out);
 
 /* The same call in two halves, for callers that keep several batches in flight from ONE host thread (the region loop

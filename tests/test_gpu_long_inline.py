@@ -114,11 +114,8 @@ def test_nothing_changes_for_normal_calls(handle):
     for regions in groups:
         pk = batch.PackedBatch(regions)
         a = batch.run(handle, pk)
-        handle.set_option("long_regions", 1)
-        try:
+        with batch.long_regions([handle]):
             b = batch.run(handle, pk)
-        finally:
-            handle.set_option("long_regions", 0)
         for f in ("n_regions", "n_contigs", "n_check_align", "n_dp_cells", "n_kmer_occurrences"):
             assert getattr(a, f) == getattr(b, f), f
         for f in ("so_off", "so_mers", "so_counts", "uniq_reg_off", "uniq_rec", "uniq_mult", "ctg_reg_off", "region_status",
@@ -136,11 +133,8 @@ def test_abandoned_contigs_are_dropped(handle):
     off = batch.run(handle, pk)
     assert list(off.region_status) == [_lib.BK_ERR_CAPACITY]
     assert off.ctg_reg_off[1] > 0                      # contigs of the abandoned attempt are in the default result
-    handle.set_option("long_regions", 1)
-    try:
+    with batch.long_regions([handle]):
         on = batch.run(handle, pk)
-    finally:
-        handle.set_option("long_regions", 0)
     only, ctg = _oracle("mix", 15)
     assert list(on.region_status) == [0]
     assert on.sample_only(0) == only
