@@ -115,6 +115,7 @@ def load():
     lib.bk_set_option.argtypes = [H, c_char_p, c_int64]
     lib.bk_ref_cache_build.argtypes = [H, c_void_p, c_void_p, c_int32, c_int32]
     lib.bk_ref_cache_clear.argtypes = [H]
+    lib.bk_region_report.argtypes = [H, POINTER(POINTER(c_int32)), POINTER(c_int32)]
     lib.bk_ingest_create.argtypes = [c_int, c_int, POINTER(H)]
     lib.bk_ingest_destroy.argtypes = [H]
     lib.bk_ingest_last_error.argtypes = [H]
@@ -132,7 +133,7 @@ def load():
     for name in ("bk_create", "bk_destroy", "bk_nw_batch", "bk_dedup_reads", "bk_count_kmers", "bk_sample_only",
                  "bk_compare_kmers_batch", "bk_compare_kmers_long", "bk_batch_submit", "bk_batch_wait", "bk_batch_upload",
                  "bk_compare_kmers_resident", "bk_kernel_times", "bk_kernel_times_reset", "bk_set_option", "bk_ref_cache_build",
-                 "bk_ref_cache_clear"):
+                 "bk_ref_cache_clear", "bk_region_report"):
         getattr(lib, name).restype = c_int
     _lib = lib
     return lib
@@ -141,7 +142,7 @@ def load():
 EXPORTED_SYMBOLS = (
     "bk_version", "bk_device_count", "bk_create", "bk_destroy", "bk_last_error", "bk_nw_batch", "bk_dedup_reads",
     "bk_count_kmers", "bk_sample_only", "bk_compare_kmers_batch", "bk_compare_kmers_long", "bk_batch_submit", "bk_batch_wait", "bk_batch_upload", "bk_compare_kmers_resident", "bk_kernel_times",
-    "bk_kernel_times_reset", "bk_set_option", "bk_ref_cache_build", "bk_ref_cache_clear",
+    "bk_kernel_times_reset", "bk_set_option", "bk_ref_cache_build", "bk_ref_cache_clear", "bk_region_report",
     "bk_ingest_create", "bk_ingest_destroy", "bk_ingest_last_error", "bk_ingest_buffers", "bk_ingest_files",
     "bk_write_contigs", "bk_write_sample_kmers")
 
@@ -181,6 +182,7 @@ class Handle:
             raise BreakmerError(rc, "bk_create(device=%d) failed: no usable CUDA device (there is no CPU fallback)"
                                 % device)
         self.device = device
+        self.result_regions = None         # n_regions of the handle's last result (batch.run / batch.wait set it)
 
     def close(self):
         if self.h:
@@ -273,6 +275,18 @@ class Handle:
 
     def set_option(self, name, value):
         self._check(self.lib.bk_set_option(self.h, name.encode(), int(value)))
+
+    def region_report(self):
+        """bk_region_report: the per-region report of the handle's last result (batch.run / batch.wait), as an
+        (n_regions, BK_RR_FIELDS) int32 copy.  Read it before the handle's next call."""
+        table, nf = POINTER(c_int32)(), c_int32()
+        self._check(self.lib.bk_region_report(self.h, byref(table), byref(nf)))
+        n = self.result_regions
+        if n is None:                      # a result the library holds but this object did not see (no row count)
+            raise BreakmerError(BK_ERR_ARG, "region_report: no result of batch.run / batch.wait on this handle")
+        if n == 0:
+            return np.zeros((0, nf.value), np.int32)
+        return np.ctypeslib.as_array(table, shape=(int(n), nf.value)).copy()
 
     # ---- timers -------------------------------------------------------------------------
     def kernel_times_reset(self, enable=True):

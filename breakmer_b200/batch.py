@@ -212,6 +212,7 @@ def run(handle, packed, resident=False, decode=True, long=False):
     else:
         s = packed.struct()
         handle._check(handle.lib.bk_compare_kmers_batch(handle.h, ctypes.byref(s), ctypes.byref(res)))
+    handle.result_regions = res.n_regions
     if not decode:
         return res
     return BatchOutput(res, packed)
@@ -232,6 +233,36 @@ def long_regions(handles, on=True):
         set_all(0)
 
 
+# bk_region_report (include/breakmer_b200.h): the BK_RR_* fields in column order, and the names of the reason codes
+REPORT_FIELDS = ("reason", "pass", "first_reason", "seeds", "find_reads", "check_align", "grown", "rejected_support",
+                 "rejected_length")
+REASONS = ("ok", "read_too_long", "contig_too_long", "kmer_list_full", "too_many_contigs", "output_arena")
+PASSES = ("none", "batched", "long")
+
+
+def region_report(handle):
+    """Why each region of the handle's last result (run / wait) stopped and what the assembler did (bk_region_report):
+    one dict per region with the REPORT_FIELDS as keys; "reason" and "first_reason" are names from REASONS, "pass" one of
+    PASSES, the counters are ints.  Read it before the handle's next call."""
+    rows = handle.region_report()
+    out = []
+    for row in rows.tolist():
+        d = dict(zip(REPORT_FIELDS, row))
+        d["reason"] = REASONS[d["reason"]]
+        d["first_reason"] = REASONS[d["first_reason"]]
+        d["pass"] = PASSES[d["pass"]]
+        out.append(d)
+    return out
+
+
+def any_failed(res):
+    """True if some region of a result (BatchOutput, or the BatchResult of decode=False) has a nonzero status."""
+    if isinstance(res, BatchOutput):
+        return bool(res.region_status.any())
+    n = res.n_regions
+    return n > 0 and bool(np.ctypeslib.as_array(res.region_status, shape=(n,)).any())
+
+
 def submit(handle, packed=None):
     """bk_batch_submit: enqueue the device pass of `packed` (None: the batch uploaded with `upload`) and return.
     `packed` must stay alive until `wait` has returned."""
@@ -246,6 +277,7 @@ def wait(handle, packed=None, decode=True):
     """bk_batch_wait: block until the submitted batch is done; BatchResult, or BatchOutput if decode."""
     res = _lib.BatchResult()
     handle._check(handle.lib.bk_batch_wait(handle.h, ctypes.byref(res)))
+    handle.result_regions = res.n_regions
     if not decode:
         return res
     return BatchOutput(res, packed)

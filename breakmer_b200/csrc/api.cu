@@ -628,6 +628,25 @@ int bk_set_option(bk_handle_t h, const char* name, int64_t value) {
   });
 }
 
+static_assert(RR_FIELDS == BK_RR_FIELDS && RR_REASON == BK_RR_REASON && RR_PASS == BK_RR_PASS &&
+                  RR_FIRST_REASON == BK_RR_FIRST_REASON && RR_SEEDS == BK_RR_SEEDS && RR_FIND_READS == BK_RR_FIND_READS &&
+                  RR_CHECK_ALIGN == BK_RR_CHECK_ALIGN && RR_GROWN == BK_RR_GROWN && RR_REJ_SUPPORT == BK_RR_REJ_SUPPORT &&
+                  RR_REJ_LENGTH == BK_RR_REJ_LENGTH,
+              "report fields of common.cuh and include/breakmer_b200.h differ");
+static_assert(RR_OK == BK_RR_OK && RR_READ_TOO_LONG == BK_RR_READ_TOO_LONG && RR_CONTIG_TOO_LONG == BK_RR_CONTIG_TOO_LONG &&
+                  RR_KMER_LIST_FULL == BK_RR_KMER_LIST_FULL && RR_TOO_MANY_CONTIGS == BK_RR_TOO_MANY_CONTIGS &&
+                  RR_OUTPUT_ARENA == BK_RR_OUTPUT_ARENA && RR_PASS_NONE == BK_RR_PASS_NONE &&
+                  RR_PASS_BATCHED == BK_RR_PASS_BATCHED && RR_PASS_LONG == BK_RR_PASS_LONG,
+              "report codes of common.cuh and include/breakmer_b200.h differ");
+
+int bk_region_report(bk_handle_t h, const int32_t** table, int32_t* n_fields) {
+  return guarded(h, [&] {
+    if (!table || !n_fields) fail(BK_ERR_ARG, "bk_region_report: null argument");
+    *table = region_report(h);
+    *n_fields = RR_FIELDS;
+  });
+}
+
 int bk_kernel_times(bk_handle_t h, const char** names, const double** ms, const int64_t** launches, int32_t* n) {
   return guarded(h, [&] {
     h->timers.collect();

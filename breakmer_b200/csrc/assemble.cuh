@@ -169,9 +169,10 @@ struct AsmParams {
   uint64_t* o_kmer_mer; int32_t* o_kmer_pos; int32_t* o_kmer_meta;
   int64_t* o_desc;                 // per contig 10 x int64: region, ordinal, seq_off, seq_len, cnt_off, cnt_len,
                                    //                        reads_off, n_reads, kmers_off, n_kmers
-  int32_t* region_status;
+  int32_t* region_status;          // per region: its status (ST_OK or the RR_* reason it stopped for)
   int32_t* region_ncontigs;
   unsigned long long* region_cells;  // per region: sum over its check_align calls of len(contig) * len(read)
+  int32_t* region_report;          // per region: RR_FIELDS ints (common.cuh, bk_region_report), or null: no report
   unsigned long long* stats;       // [0] check_align calls, [1] DP cells, [2] find_reads, [3] seeds, [8..] phase cycles
   unsigned long long* prof_regions; // BK_PHASE_PROF: n_regions x 8 phase cycles (or null)
 };
@@ -298,7 +299,7 @@ struct RegionCtxT {
   bool ct_setup, ct_finalized;
   bool setup_queued;              // setup_contigs: the new contig went into buffer.contigs
   int ct_init_read;
-  int status;
+  int status;                     // ST_OK, or the reason (RR_*) the region stopped for
   int n_out;
   unsigned long long n_align, n_cells;   // work counters of the region (flushed once at its end)
 #if defined(BK_PHASE_PROF) && !defined(BK_SIM)
@@ -313,6 +314,36 @@ struct RegionCtxT {
   BK_DEV const uint8_t* read_ptr(int u) const { return P->rbases + P->roff[u_rec[u]]; }
 };
 using RegionCtx = RegionCtxT<AsmCap>;
+
+// ---- per-region report (bk_region_report) ------------------------------------------------------------------------------
+// A region that stops keeps the reason in c.status (ST_OK while it runs), which becomes its region_status.  Its counters
+// are kept in s_report, a shared-memory row of the CTA at a fixed address, while it runs (lane 0 of the warp that runs the
+// state machine writes it: one CTA owns a region), and copied to P.region_report when it ends, with its check_align
+// calls.  Neither the counters nor the table's address live in registers, and the copy-in and copy-out are out of line:
+// assemble_kernel<W> compiles to the same registers, stack and spills as without the report.  RR_REASON and RR_PASS are
+// filled in on the host from region_status and the long kernel's queue; RR_FIRST_REASON is route_long_kernel's.
+#if defined(BK_SIM)
+static int s_report[RR_FIELDS];
+#define BK_DEV_OUTLINE inline
+#elif defined(BK_SIMT)
+__shared__ int s_report[RR_FIELDS];
+#define BK_DEV_OUTLINE inline
+#else
+__shared__ int s_report[RR_FIELDS];
+#define BK_DEV_OUTLINE static __device__ __noinline__
+#endif
+BK_DEV void report_add(int field, int v) {
+  if (lane() == 0) s_report[field] += v;
+}
+BK_DEV_OUTLINE void report_begin() {                                    // (bind_region syncs the warp after it)
+  for (int f = lane(); f < RR_FIELDS; f += WARP) s_report[f] = 0;
+}
+// table is null in the single-region harnesses of tests/sim
+BK_DEV_OUTLINE void report_end(int32_t* table, int region, unsigned long long n_align) {
+  syncwarp();                                                            // lane 0's counters are visible to the warp
+  for (int f = lane(); f < RR_FIELDS; f += WARP)
+    if (table && f >= RR_SEEDS) table[(size_t)region * RR_FIELDS + f] = f == RR_CHECK_ALIGN ? (int32_t)n_align : s_report[f];
+}
 
 // lookup of a code in the region's ascending mer table; -1 if absent.  Regions with up
 // to MER_HASH_MAX mers use an open-addressed table in shared memory (entry =
@@ -452,7 +483,7 @@ BK_DEV void append_kmers(RegionCtxT<T>& c, const uint8_t* seq, int base, int nle
       c.nK += popc(mk);
     }
   }
-  if (c.nK > KCAP) { c.nK = KCAP; c.status = ST_CAPACITY; }
+  if (c.nK > KCAP) { c.nK = KCAP; c.status = RR_KMER_LIST_FULL; }
   syncwarp();
   BK_PH_END(c, PH_KMERS)
 }
@@ -536,7 +567,7 @@ template <class T>
 BK_DEV void contig_init(RegionCtxT<T>& c, int seed_s, int u) {
   BK_PH_BEGIN
   c.serial += 1;
-  if (c.serial >= (1u << (32 - T::BITS))) { c.status = ST_CAPACITY; return; }   // tag width of m_first
+  if (c.serial >= (1u << (32 - T::BITS))) { c.status = RR_TOO_MANY_CONTIGS; return; }   // tag width of m_first
   const int lr = stage_read(c, u);
   c.c0 = T::CAP; c.clen = lr;
   c.cur = 0; c.k0 = T::CAP; c.klen = lr;
@@ -818,7 +849,7 @@ BK_DEV bool apply_align_impl(RegionCtxT<T>& c, int u, int seed_s, bool grow, con
     return true;
   } else if (act == ACT_APPEND) {
     const int plen = lr - v1.prei;                                    // post_seq = read[aln[4]:]
-    if (lc + plen > T::MAX_LEN) { c.status = ST_CAPACITY; return true; }
+    if (lc + plen > T::MAX_LEN) { c.status = RR_CONTIG_TOO_LONG; return true; }
     for (int x = lane(); x < plen; x += WARP) {
       const uint8_t ch = rd[v1.prei + x];
       c.cseq[c.c0 + lc + x] = ch; c.s_contig[lc + x] = ch;
@@ -831,7 +862,7 @@ BK_DEV bool apply_align_impl(RegionCtxT<T>& c, int u, int seed_s, bool grow, con
     k_base = lc - (c.k - 1); k_len = (c.k - 1) + plen; k_order = ORDER_FOR;   // :521,525-527
   } else {
     const int plen = v2.j0;                                           // pre_seq = read[0:aln[3]]
-    if (lc + plen > T::MAX_LEN) { c.status = ST_CAPACITY; return true; }
+    if (lc + plen > T::MAX_LEN) { c.status = RR_CONTIG_TOO_LONG; return true; }
     for (int x = lane(); x < plen; x += WARP) c.cseq[c.c0 - plen + x] = rd[x];
     c.c0 -= plen; c.clen = lc + plen;
     c.seq_ver += 1;
@@ -1038,6 +1069,7 @@ BK_DEV int find_reads(RegionCtxT<T>& c, int s, bool filter_buffer, bool rev, int
   }
   syncwarp();
   if (lane() == 0) atomic_add(&c.P->stats[2], 1ull);
+  report_add(RR_FIND_READS, 1);
   BK_PH_END(c, PH_FIND)
   return n;
 }
@@ -1106,7 +1138,7 @@ BK_DEV void emit_contig(RegionCtxT<T>& c) {
   o_seq = shfl(o_seq, 0); o_cnt = shfl(o_cnt, 0); o_rd = shfl(o_rd, 0); o_km = shfl(o_km, 0); o_ct = shfl(o_ct, 0);
   if (o_seq + len > P.cap_seq || o_cnt + c.klen > P.cap_cnt || o_rd + n_reads > P.cap_reads || o_km + c.nK > P.cap_kmers ||
       o_ct + 1 > P.cap_ctg) {
-    c.status = ST_CAPACITY;
+    c.status = RR_OUTPUT_ARENA;
     return;
   }
   // kmer_locs = prefix sum of diff (sequential over chunks of a warp)
@@ -1267,7 +1299,9 @@ BK_DEV int total_reads(const RegionCtxT<T>& c) {                         // :178
 template <class T>
 BK_DEV void finish_contig(RegionCtxT<T>& c, int rc_thresh, int read_len) {
   if (c.status != ST_OK) return;
-  if (total_reads(c) < rc_thresh || c.clen <= read_len) return;
+  report_add(RR_GROWN, 1);
+  if (total_reads(c) < rc_thresh) { report_add(RR_REJ_SUPPORT, 1); return; }
+  if (c.clen <= read_len) { report_add(RR_REJ_LENGTH, 1); return; }
   emit_contig(c);
 }
 
@@ -1311,6 +1345,7 @@ BK_DEV void assemble_region(RegionCtxT<T>& c) {
     }
     if (seed < 0) break;
     if (lane() == 0) atomic_add(&P.stats[3], 1ull);
+    report_add(RR_SEEDS, 1);
     // setup_contigs (:11-26) for the seed, then `while len(buff.contigs) > 0` (:50): the set-up contig first if it was
     // queued (the queue was empty, so it is the FIFO head), then whatever check_alt_reads queued
     int mode = GROW_SETUP;
@@ -1385,6 +1420,7 @@ BK_DEV void bind_region(RegionCtxT<T>& c, const AsmParams& P, int region, int64_
   c.tab = P.w_tab ? P.w_tab + (size_t)slot * spec_w * NW_TAB_BYTES : nullptr;
   c.edge = c.edge_all;
   c.s_reads = s_reads; c.s_read = s_reads; c.s_contig = s_contig; c.sp = sp;
+  report_begin();
   c.st_n = 0; c.rnd_base = 0; c.rnd_cnt = 0; c.seq_ver = 0;
   // kmers.add_kmer (:272-278, Q5): a homopolymer (len(set(mer)) == 1) never enters akmers
   for (int s = lane(); s < c.S; s += WARP) {
@@ -1478,6 +1514,7 @@ __global__ void __launch_bounds__(32 * W, (CTAS > 0 ? CTAS : (W >= 8 ? 1 : (W ==
       atomicAdd(&P.stats[0], c.n_align);
       atomicAdd(&P.stats[1], c.n_cells);
     }
+    report_end(P.region_report, region, c.n_align);
     syncwarp();
   }
   if (W > 1) {

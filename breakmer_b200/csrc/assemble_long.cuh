@@ -54,6 +54,7 @@ __global__ void __launch_bounds__(NWL_THREADS, 1) assemble_long_kernel(AsmParams
       atomicAdd(&P.stats[0], c.n_align);
       atomicAdd(&P.stats[1], c.n_cells);
     }
+    report_end(P.region_report, region, c.n_align);
     syncwarp();
   }
   if (lane() == 0) sp.n = -1;                          // dismiss the other warps
@@ -63,23 +64,30 @@ __global__ void __launch_bounds__(NWL_THREADS, 1) assemble_long_kernel(AsmParams
 // The long modes: after assemble_kernel, build assemble_long_kernel's queue on the device.  order[n_short, n_regions) are
 // the regions routed at upload (a read above 4,095 bases, or every region with n_short = 0 for bk_compare_kmers_long;
 // assemble_kernel never saw them), most expensive first; then, in work order, every region of order[0, n_short) that
-// assemble_kernel finished with ST_CAPACITY.  *ctg_snapshot = the contig cursor at this point: the descriptors below it
-// are assemble_kernel's, and those of a rerouted region are dropped from the result.  One block.
+// assemble_kernel stopped (status not ST_OK).  *ctg_snapshot = the contig cursor at this point: the descriptors below it
+// are assemble_kernel's, and those of a rerouted region are dropped from the result.  The report's RR_FIRST_REASON of
+// every queued region is set here, before assemble_long_kernel rebinds it: routed_reason for those routed at upload
+// (the report starts zeroed, so 0 leaves it as is), the reason assemble_kernel stopped the others for (their status).  One block.
 constexpr int ROUTE_THREADS = 256;
 __global__ void __launch_bounds__(ROUTE_THREADS) route_long_kernel(const int32_t* __restrict__ order, int n_short, int n_regions,
                                                                    const int32_t* __restrict__ region_status,
                                                                    const unsigned long long* __restrict__ out_cursor,
                                                                    int32_t* __restrict__ queue, int* __restrict__ n_queue,
-                                                                   unsigned long long* __restrict__ ctg_snapshot) {
+                                                                   unsigned long long* __restrict__ ctg_snapshot,
+                                                                   int32_t* __restrict__ report, int routed_reason) {
   __shared__ int s_warp[ROUTE_THREADS / WARP];
   const int n_long = n_regions - n_short;
   const int t = threadIdx.x, wi = t / WARP;
   if (t == 0) *ctg_snapshot = out_cursor[4];
-  for (int i = t; i < n_long; i += ROUTE_THREADS) queue[i] = order[n_short + i];
+  for (int i = t; i < n_long; i += ROUTE_THREADS) {
+    const int r = order[n_short + i];
+    queue[i] = r;
+    if (routed_reason) report[(size_t)r * RR_FIELDS + RR_FIRST_REASON] = routed_reason;
+  }
   int base = n_long;
   for (int i0 = 0; i0 < n_short; i0 += ROUTE_THREADS) {       // ordered compaction, one block-wide chunk at a time
     const int i = i0 + t;
-    const bool take = i < n_short && region_status[order[i]] == ST_CAPACITY;
+    const bool take = i < n_short && region_status[order[i]] != ST_OK;
     const unsigned mk = ballot(take);
     if (lane() == 0) s_warp[wi] = popc(mk);
     __syncthreads();
@@ -88,7 +96,11 @@ __global__ void __launch_bounds__(ROUTE_THREADS) route_long_kernel(const int32_t
       before += v < wi ? s_warp[v] : 0;
       total += s_warp[v];
     }
-    if (take) queue[base + before + popc(mk & ((1u << lane()) - 1u))] = order[i];
+    if (take) {
+      const int r = order[i];
+      queue[base + before + popc(mk & ((1u << lane()) - 1u))] = r;
+      report[(size_t)r * RR_FIELDS + RR_FIRST_REASON] = region_status[r];
+    }
     base += total;
     __syncthreads();                                 // s_warp is rewritten by the next chunk
   }

@@ -100,10 +100,17 @@ BK_HD int base_code_strict(uint8_t c) {
 
 constexpr uint64_t KEY_INVALID = ~0ull;
 
-// per-region status written by device code (same values as BK_OK /
-// BK_ERR_CAPACITY in include/breakmer_b200.h)
+// per-region status written by device code: ST_OK (BK_OK in include/breakmer_b200.h), or the RR_* reason below the
+// region stopped for, which bk_batch_wait reports as BK_ERR_CAPACITY
 constexpr int ST_OK = 0;
-constexpr int ST_CAPACITY = -4;
+
+// per-region report (AsmParams::region_report): fields and reason codes, the BK_RR_* values of include/breakmer_b200.h
+enum {
+  RR_REASON = 0, RR_PASS, RR_FIRST_REASON, RR_SEEDS, RR_FIND_READS, RR_CHECK_ALIGN, RR_GROWN, RR_REJ_SUPPORT,
+  RR_REJ_LENGTH, RR_FIELDS
+};
+enum { RR_OK = 0, RR_READ_TOO_LONG, RR_CONTIG_TOO_LONG, RR_KMER_LIST_FULL, RR_TOO_MANY_CONTIGS, RR_OUTPUT_ARENA };
+enum { RR_PASS_NONE = 0, RR_PASS_BATCHED, RR_PASS_LONG };
 
 // hard limits of the packed DP cell (nw.cuh): 14-bit signed score field
 constexpr int NW_MAX_LEN = 4095;

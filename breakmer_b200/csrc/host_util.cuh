@@ -73,7 +73,9 @@ class Arena {
     }
     used_ = 0;
     total_ = 0;
+    ++resets_;
   }
+  size_t resets() const { return resets_; }   // changes whenever earlier allocations may be reused
   void release() {
     for (auto& c : chunks_) {
       if (PINNED_HOST) cudaFreeHost(c.p);
@@ -87,7 +89,7 @@ class Arena {
  private:
   struct Chunk { void* p; size_t size; };
   std::vector<Chunk> chunks_;
-  size_t used_ = 0, total_ = 0, grow_ = size_t(64) << 20;
+  size_t used_ = 0, total_ = 0, grow_ = size_t(64) << 20, resets_ = 0;
 };
 
 enum KernelFamily : int {

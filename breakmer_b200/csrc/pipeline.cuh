@@ -66,7 +66,7 @@ struct Pipeline {
   std::vector<int64_t> filt_off, filt_reg_off;
   std::vector<uint8_t> filt_flags;
   // the long assembler's mode, fixed at upload.  assemble_kernel takes the first n_short regions of the work order; in
-  // the long modes, assemble_long_kernel takes the others and those assemble_kernel stopped with ST_CAPACITY
+  // the long modes, assemble_long_kernel takes the others and those assemble_kernel stopped
   LongMode long_mode = LONG_OFF;
   int n_short = 0;                        // LONG_OFF: all; LONG_ROUTE: those without a read above NW_MAX_LEN; LONG_ALL: 0
   const uint8_t* d_routed = nullptr;      // device, per region: a read above NW_MAX_LEN (LONG_ROUTE; null when none)
@@ -115,6 +115,14 @@ struct PendingBatch {
   int32_t* h_status = nullptr;
   unsigned long long* h_cells = nullptr;
   const int64_t* h_so_off = nullptr; const int64_t* h_u_off = nullptr;
+  // the per-region report of the batch's result (bk_region_report): readable while the device arena is the one the
+  // result was made in (result_epoch == h->dev.resets())
+  bool has_result = false;
+  size_t result_epoch = 0;
+  std::vector<uint8_t> report_skipped;     // Pipeline::region_skipped of the batch
+  std::vector<int32_t> h_reason;           // the device's region_status: 0 or the RR_* reason
+  std::vector<int32_t> long_queue;         // the regions assemble_long_kernel ran (the long modes)
+  std::vector<int32_t> h_report;           // host copy, made on request
 };
 
 }  // namespace bk

@@ -357,7 +357,8 @@ void launch_assembly(bk_handle_t h, PendingBatch& B) {
     {
       TimedLaunch t(h->timers, st, KF_PREP);
       route_long_kernel<<<1, ROUTE_THREADS, 0, st>>>(A.work_order, n_short, R, A.region_status, A.out_cursor, B.LA.queue, B.n_queue,
-                                                     B.ctg_snapshot);
+                                                     B.ctg_snapshot, A.region_report,
+                                                     B.p->long_mode == LONG_ROUTE ? RR_READ_TOO_LONG : RR_OK);
     }
     TimedLaunch t(h->timers, st, KF_ASSEMBLE);
     BK_CUDA(launch_assemble_long(long_params(A, B.LA), B.LA.L, B.LA.grid, st));
@@ -613,6 +614,7 @@ void pipeline_submit(bk_handle_t h, const bk_batch_input* in, LongMode mode) {
   const size_t o_mused = zalloc(SB), o_checked = zalloc(SB * 4), o_taken = zalloc(SB * 4), o_first = zalloc(SB * 4);
   const size_t o_rused = zalloc(NUB), o_rdel = zalloc(NUB), o_rq = zalloc(NUB), o_rbuf = zalloc(NUB * 4), o_rin = zalloc(NUB * 4);
   const size_t o_work = zalloc(sizeof(int)), o_cursor = zalloc(5 * sizeof(unsigned long long)), o_stats = zalloc(32 * sizeof(unsigned long long));
+  const size_t o_report = zalloc((size_t)R * RR_FIELDS * sizeof(int32_t));
   const size_t o_route = B.route ? zalloc(2 * sizeof(int) + sizeof(unsigned long long)) : 0;   // long counter, queue length, snapshot
   uint8_t* zero_lo = h->dev.get<uint8_t>(zero_bytes);
   if (B.route) {
@@ -628,6 +630,7 @@ void pipeline_submit(bk_handle_t h, const bk_batch_input* in, LongMode mode) {
   A.work_counter = (int*)(zero_lo + o_work);
   A.out_cursor = (unsigned long long*)(zero_lo + o_cursor);
   A.stats = (unsigned long long*)(zero_lo + o_stats);
+  A.region_report = (int32_t*)(zero_lo + o_report);
   A.q_read = h->dev.get<int32_t>(NUB ? NUB : 1); A.q_seed = h->dev.get<int32_t>(NUB ? NUB : 1);
   A.l_alt = h->dev.get<int32_t>(NUB ? NUB : 1); A.l_del = h->dev.get<int32_t>(NUB ? NUB : 1);
   A.hit_u = h->dev.get<int32_t>(NUB ? NUB : 1); A.hit_pos = h->dev.get<int32_t>(NUB ? NUB : 1);
@@ -759,6 +762,10 @@ void pipeline_wait(bk_handle_t h, bk_batch_result* out) {
       out->host_wait_ms = *blocked; out->host_post_ms = total - *blocked;
     }
   } host_times{out, t_enter, &blocked_ms};
+  B.h_reason.assign(B.h_status, B.h_status + R);          // the device's status of a stopped region is the reason
+  for (int r = 0; r < R; ++r)
+    if (B.h_status[r] != ST_OK) B.h_status[r] = BK_ERR_CAPACITY;
+  B.long_queue.assign(B.route ? B.h_queue : nullptr, B.route ? B.h_queue + *B.h_n_queue : nullptr);
   if (!p.region_skipped.empty()) {
     // regions that were left out: report them, and give record indices in the caller's numbering again
     for (int r = 0; r < R; ++r) {
@@ -770,6 +777,37 @@ void pipeline_wait(bk_handle_t h, bk_batch_result* out) {
         for (int64_t e = t_rd[2 * c]; e < t_rd[2 * c] + t_rd[2 * c + 1]; ++e) h_reads[e] += shift;
     }
   }
+  B.report_skipped = p.region_skipped;                     // (the resident Pipeline may be replaced before the report is read)
+  B.result_epoch = h->dev.resets();
+  B.has_result = true;
+}
+
+// bk_region_report: the report of the last result.  The device's table holds the counters and RR_FIRST_REASON; the reason
+// (the device's region_status) and the pass (the long kernel's queue) are added here, and regions left out at upload get
+// their row here, as their region_status does in pipeline_wait
+const int32_t* region_report(bk_handle_t h) {
+  PendingBatch& B = h->pending;
+  if (B.active) fail(BK_ERR_ARG, "bk_region_report: a batch is in flight on this handle (call bk_batch_wait first)");
+  if (!B.has_result || B.result_epoch != h->dev.resets()) fail(BK_ERR_ARG, "bk_region_report: no result on this handle");
+  const int R = B.A.n_regions;
+  B.h_report.assign((size_t)(R ? R : 1) * RR_FIELDS, 0);
+  if (R) {
+    BK_CUDA(cudaMemcpyAsync(B.h_report.data(), B.A.region_report, (size_t)R * RR_FIELDS * sizeof(int32_t), cudaMemcpyDeviceToHost, h->st));
+    BK_CUDA(stream_wait(h));
+  }
+  for (int r = 0; r < R; ++r) {
+    int32_t* row = B.h_report.data() + (size_t)r * RR_FIELDS;
+    row[RR_REASON] = B.h_reason[r];
+    row[RR_PASS] = RR_PASS_BATCHED;
+  }
+  for (int32_t r : B.long_queue) B.h_report[(size_t)r * RR_FIELDS + RR_PASS] = RR_PASS_LONG;
+  for (int r = 0; r < (int)B.report_skipped.size(); ++r) {
+    if (!B.report_skipped[r]) continue;
+    int32_t* row = B.h_report.data() + (size_t)r * RR_FIELDS;
+    std::fill(row, row + RR_FIELDS, 0);
+    row[RR_REASON] = RR_READ_TOO_LONG;
+  }
+  return B.h_report.data();
 }
 
 void phase_print(bk_handle_t h, const PendingBatch& B) {

@@ -165,6 +165,7 @@ class DevicePipeline:
             if long_regions:
                 h.set_option("long_regions", 1)
         self._queue = []                               # (handle index, packed, tag) in submission order
+        self.report = False                            # pop: read every batch's per-region report
         self._next = 0
 
     def full(self):
@@ -180,10 +181,14 @@ class DevicePipeline:
         self._queue.append((j, packed, tag))
 
     def pop(self, decode=True):
-        """-> (result of the oldest batch in flight, its packed input, its tag)"""
+        """-> (result of the oldest batch in flight, its packed input, its tag).  The result's `.report` is the batch's
+        batch.region_report, read before its handle takes another batch, if `self.report` is set or a region of the
+        batch failed; else None."""
         from . import batch
         j, packed, tag = self._queue.pop(0)
-        return batch.wait(self.handles[j], packed, decode=decode), packed, tag
+        res = batch.wait(self.handles[j], packed, decode=decode)
+        res.report = batch.region_report(self.handles[j]) if (self.report or batch.any_failed(res)) else None
+        return res, packed, tag
 
     def pending(self):
         return len(self._queue)

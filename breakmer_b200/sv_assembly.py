@@ -224,10 +224,11 @@ def _clean_mers(mers, kmer_len):
     return mers
 
 
-def _assemble_calls(calls, device, long_regions):
-    """One device pass over `calls` -> (contig list or None per call, indices of the calls reported BK_ERR_CAPACITY).
-    long_regions: the pass also assembles calls with reads or contigs up to 65,535 bases (the handle's option of that
-    name, set for this call only)."""
+def _assemble_calls(calls, device, long_regions, want_report=False):
+    """One device pass over `calls` -> (contig list or None per call, indices of the calls reported BK_ERR_CAPACITY,
+    batch.region_report of the pass or None).  long_regions: the pass also assembles calls with reads or contigs up to
+    65,535 bases (the handle's option of that name, set for this call only).  The report is read when want_report or
+    when a call was not completed."""
     import numpy as np
     inputs = [_AssemblyInput("r%d" % i, c[1], c[2], c[3]) for i, c in enumerate(calls)]
     pk = batch.PackedBatch(inputs, rc_thresh=int(calls[0][3]))
@@ -236,6 +237,7 @@ def _assemble_calls(calls, device, long_regions):
     h = get_handle(device)
     with batch.long_regions([h], long_regions):
         out = batch.run(h, pk)
+        rows = batch.region_report(h) if (want_report or batch.any_failed(out)) else None
     objs = [o for inp in inputs for o in inp.objs]
     result = []
     bad = []
@@ -245,10 +247,10 @@ def _assemble_calls(calls, device, long_regions):
             result.append(None)
             continue
         result.append([contig(out, cidx, objs, int(c[2])) for cidx in range(int(out.ctg_reg_off[i]), int(out.ctg_reg_off[i + 1]))])
-    return result, bad
+    return result, bad, rows
 
 
-def init_assembly_batch(calls, device=0, on_capacity="raise"):
+def init_assembly_batch(calls, device=0, on_capacity="raise", report=None):
     """calls: [(mers, fq_recs, kmer_len, rc_thresh, read_len), ...] with one common
     kmer_len and rc_thresh -> list (per call) of contig lists.  One GPU pass.
 
@@ -258,15 +260,21 @@ def init_assembly_batch(calls, device=0, on_capacity="raise"):
                          stored in the exception's `.results`;
       "none"             their entry in the returned list is None;
       "assemble"         the same pass assembles them too (the handle's "long_regions" option: reads and contigs up
-                         to 65,535 bases); a RuntimeError as with "raise" names the calls that exceed that limit."""
+                         to 65,535 bases); a RuntimeError as with "raise" names the calls that exceed that limit.
+    The RuntimeError's `.reasons` says why each of those calls was not completed ({call index: reason name}, see
+    batch.REASONS).  `report`, a list, is extended with batch.region_report's dict of every call, in call order: why it
+    stopped, which pass assembled it, and what the assembler did."""
     if not calls:
         return []
-    result, bad = _assemble_calls(calls, device, on_capacity == "assemble")
+    result, bad, rows = _assemble_calls(calls, device, on_capacity == "assemble", report is not None)
+    if report is not None:
+        report.extend(rows)
     limit = 65535 if on_capacity == "assemble" else 4095
     if bad and on_capacity in ("raise", "assemble"):
         err = RuntimeError("init_assembly: device capacity exceeded in call(s) %s (a read or contig longer than %d bases); "
                            "the other calls completed (see .results)" % (bad, limit))
         err.results = result
+        err.reasons = {i: rows[i]["reason"] for i in bad}
         raise err
     return result
 

@@ -36,6 +36,8 @@ contig.setup writes before blat (sv_processor.py:749-782) under target.paths['co
 library's host threads (bk_write_contigs, SURVEY.md section 8.7 f.3).
 `on_capacity="assemble"` assembles targets with reads or contigs above 4,095 bases (up to 65,535) in the
 same device pass as all others (the handles' "long_regions" option).
+`report={}` is filled with what the assembler did for every target (batch.region_report: why it stopped, which pass
+assembled it, how many seeds, find_reads and check_align calls, and how many contigs were grown and rejected).
 """
 import os
 
@@ -110,12 +112,14 @@ class CapacityError(RuntimeError):
     """Some targets exceeded a device limit: a read or contig longer than 4095 bases (compare_kmers_batch's default
     on_capacity="raise"), or longer than 65,535 bases (on_capacity="assemble", where the same pass assembles everything
     up to that length).  Every other target of the batch was completed; `.targets` lists the ones that were not (their state is untouched, so the
-    reference's own compare_kmers() can still be run on them)."""
+    reference's own compare_kmers() can still be run on them), and `.reasons` says why for each of them ({name: reason},
+    the reason names of batch.REASONS: "read_too_long", "contig_too_long", "kmer_list_full", "too_many_contigs")."""
 
-    def __init__(self, names):
+    def __init__(self, names, reasons=None):
         RuntimeError.__init__(self, "compare_kmers: device capacity exceeded for target(s) %s; all other targets completed"
                               % ", ".join(names))
         self.targets = list(names)
+        self.reasons = dict(reasons or {})
 
 
 def _apply_chunk(targets, pk, res, inputs_k, objs, ingest, write_contigs, failed, ing=None):
@@ -159,6 +163,19 @@ def _apply_chunk(targets, pk, res, inputs_k, objs, ingest, write_contigs, failed
         kmers['case_only'] = {}
 
 
+def _record_report(targets, rows, failed, reasons, report):
+    """The batch.region_report rows of one device call (None: not read) -> reasons[name] of its failed targets, and
+    report[name] of all its targets when a report is wanted."""
+    if rows is None:
+        return
+    at = {t.name: i for i, t in enumerate(targets)}
+    for name in failed:
+        reasons[name] = rows[at[name]]["reason"]
+    if report is not None:
+        for t, row in zip(targets, rows):
+            report[t.name] = row
+
+
 def _pack_targets(targets, ingest, slot=0):
     """-> (packed batch, per-target k, record index -> fq_read)"""
     import numpy as np
@@ -184,7 +201,7 @@ def _pack_targets(targets, ingest, slot=0):
 
 
 def compare_kmers_batch(targets, device=0, ingest="python", write_contigs=False, devices=None, max_targets=125, inflight=4,
-                        apply_thread=False, on_capacity="raise"):
+                        apply_thread=False, on_capacity="raise", report=None):
     """target.compare_kmers() for many targets (the region loop of sv_processor.py:185-201 as one call).
 
     The targets are cut into chunks of at most max_targets, most expensive first (static cost, breakmer_b200.shard), and
@@ -204,7 +221,10 @@ def compare_kmers_batch(targets, device=0, ingest="python", write_contigs=False,
     untouched).  With on_capacity="assemble" every call runs with the handles' "long_regions" option: such targets are
     assembled in the same device pass as the others (reads and contigs up to 65,535 bases), on the device that ran their
     chunk, and their results applied like every other target's (files included); CapacityError then lists only the
-    targets beyond that limit."""
+    targets beyond that limit.  CapacityError.reasons says why each of them was not completed.
+
+    `report`, a dict, receives report[target.name] = batch.region_report's dict of the target, for every target, in every
+    form (one call, chunked, apply_thread, devices=[...])."""
     if on_capacity not in ("raise", "assemble"):
         raise ValueError("on_capacity must be 'raise' or 'assemble'")
     if not targets:
@@ -213,7 +233,7 @@ def compare_kmers_batch(targets, device=0, ingest="python", write_contigs=False,
         raise ValueError("write_contigs needs ingest='native' (the writer reads the parsed record text)")
     if ingest not in ("python", "native"):
         raise ValueError("ingest must be 'python' or 'native'")
-    failed = []
+    failed, reasons = [], {}
     devices = list(devices) if devices else [device]
     long_regions = on_capacity == "assemble"
     if len(targets) <= max_targets and len(devices) == 1:
@@ -221,11 +241,14 @@ def compare_kmers_batch(targets, device=0, ingest="python", write_contigs=False,
         h = get_handle(devices[0])
         with batch.long_regions([h], long_regions):
             res = batch.run(h, pk, decode=False)
+            rows = batch.region_report(h) if (report is not None or batch.any_failed(res)) else None
         _apply_chunk(targets, pk, res, ks, objs, ingest, write_contigs, failed)
+        _record_report(targets, rows, failed, reasons, report)
     else:
-        _sharded(targets, devices, ingest, write_contigs, max_targets, inflight, failed, apply_thread, long_regions)
+        _sharded(targets, devices, ingest, write_contigs, max_targets, inflight, failed, apply_thread, long_regions, reasons,
+                 report)
     if failed:
-        raise CapacityError(sorted(failed))
+        raise CapacityError(sorted(failed), reasons)
 
 
 _pipes = {}
@@ -241,7 +264,8 @@ def _get_pipe(dev, inflight):
     return _pipes[key]
 
 
-def _sharded(targets, devices, ingest, write_contigs, max_targets, inflight, failed, apply_thread=False, long_regions=False):
+def _sharded(targets, devices, ingest, write_contigs, max_targets, inflight, failed, apply_thread=False, long_regions=False,
+             reasons=None, report=None):
     """Chunked, pipelined (and with several devices region-sharded) pass: sv_processor.py:185-201 over `devices`."""
     import threading
     costs = [_target_cost(t) for t in targets]
@@ -269,6 +293,7 @@ def _sharded(targets, devices, ingest, write_contigs, max_targets, inflight, fai
         pipe = None
         try:
             pipe = shard.DevicePipeline(dev, inflight=inflight) if own_pipe else _get_pipe(dev, inflight)
+            pipe.report = report is not None                 # (pop reads the report of a batch with a failed region anyway)
             with batch.long_regions(pipe.handles, long_regions):
                 # (the writer the applying thread uses: made here so that it is cached under the calling thread's key)
                 apply_ing = _get_ingest("apply") if (apply_thread and ingest == "native") else None
@@ -280,6 +305,7 @@ def _sharded(targets, devices, ingest, write_contigs, max_targets, inflight, fai
                     _apply_chunk(chunk, pk, res, ks, objs, ingest, write_contigs, mine, apply_ing)
                     with lock:
                         failed.extend(mine)
+                        _record_report(chunk, getattr(res, "report", None), mine, reasons, report)
 
                 if apply_thread:
                     # this thread parses and submits; a second one takes the results in submission order and applies them.

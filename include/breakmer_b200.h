@@ -160,7 +160,7 @@ typedef struct bk_batch_result {
   const int64_t* ctg_reads_off; const int32_t* ctg_reads;
   const int64_t* ctg_kmers_off; const uint64_t* ctg_kmer_mer; const int32_t* ctg_kmer_pos;
   const int32_t* ctg_kmer_lth;  const int32_t* ctg_kmer_dist; const int32_t* ctg_kmer_order;
-  const int32_t* region_status;      /* 0 or BK_ERR_CAPACITY per region */
+  const int32_t* region_status;      /* 0 or BK_ERR_CAPACITY per region (the cause: bk_region_report) */
   /* work counters of this call (for roofline arithmetic) */
   int64_t n_check_align;             /* contig.check_align calls (each = two olc.nw) */
   int64_t n_dp_cells;                /* sum over those of len(contig)*len(read) (one sweep each).  With the
@@ -230,6 +230,58 @@ int bk_ref_cache_clear(bk_handle_t h);
  * with.  It costs device memory per call (scratch of the long assembler, about 11 MB per CTA for at least 4 CTAs)
  * and two small launches; with 0 nothing extra is allocated or launched. */
 int bk_set_option(bk_handle_t h, const char* name, int64_t value);
+
+/* ---- per-region report: why a region's assembly stopped and what the assembler did ----------------------------
+ * One row of BK_RR_FIELDS int32 per region, in the order of the call's regions:
+ *   BK_RR_REASON        why the region has no result (region_status BK_ERR_CAPACITY), BK_RR_OK (0) when it has one:
+ *                       BK_RR_READ_TOO_LONG     a read above the mode's limit (4095 bases, 65535 in the long modes):
+ *                                               the region was left out at upload
+ *                       BK_RR_CONTIG_TOO_LONG   a contig would grow past the assembler's limit
+ *                       BK_RR_KMER_LIST_FULL    a contig holds more k-mer tuples than 2 x that limit
+ *                       BK_RR_TOO_MANY_CONTIGS  the region started more contigs than the assembler can tag
+ *                                               (2^20 in the batched assembler, 2^16 in the long one)
+ *   BK_RR_PASS          which assembler produced the result: BK_RR_PASS_NONE (0, left out at upload),
+ *                       BK_RR_PASS_BATCHED (1, the batched assembler), BK_RR_PASS_LONG (2, the long assembler)
+ *   BK_RR_FIRST_REASON  for a region the long assembler took over under the "long_regions" option: why the batched
+ *                       assembler did not keep it -- BK_RR_READ_TOO_LONG (a read above 4095 bases, routed at upload),
+ *                       one of the codes above, or BK_RR_OUTPUT_ARENA (its contigs did not fit the output arena).
+ *                       0 for every other region, and for every region of bk_compare_kmers_long.
+ *   BK_RR_SEEDS         seeds taken (akmers.has_mers iterations, sv_assembly.py:43-45)
+ *   BK_RR_FIND_READS    find_reads calls
+ *   BK_RR_CHECK_ALIGN   contig.check_align calls
+ *   BK_RR_GROWN         contigs taken from buffer.contigs, grown and tested for acceptance (sv_assembly.py:50-59)
+ *   BK_RR_REJ_SUPPORT   of those, rejected because their total read support is below rc_thresh
+ *   BK_RR_REJ_LENGTH    of those, rejected because they are not longer than read_len (support tested first)
+ * The counters are those of the pass that produced the result (BK_RR_PASS).  For a region with BK_RR_REASON 0,
+ * BK_RR_GROWN = its contigs in the result + BK_RR_REJ_SUPPORT + BK_RR_REJ_LENGTH. */
+#define BK_RR_REASON 0
+#define BK_RR_PASS 1
+#define BK_RR_FIRST_REASON 2
+#define BK_RR_SEEDS 3
+#define BK_RR_FIND_READS 4
+#define BK_RR_CHECK_ALIGN 5
+#define BK_RR_GROWN 6
+#define BK_RR_REJ_SUPPORT 7
+#define BK_RR_REJ_LENGTH 8
+#define BK_RR_FIELDS 9
+
+#define BK_RR_OK 0
+#define BK_RR_READ_TOO_LONG 1
+#define BK_RR_CONTIG_TOO_LONG 2
+#define BK_RR_KMER_LIST_FULL 3
+#define BK_RR_TOO_MANY_CONTIGS 4
+#define BK_RR_OUTPUT_ARENA 5
+
+#define BK_RR_PASS_NONE 0
+#define BK_RR_PASS_BATCHED 1
+#define BK_RR_PASS_LONG 2
+
+/* The per-region report of the last result on the handle (bk_compare_kmers_batch, bk_compare_kmers_long,
+ * bk_compare_kmers_resident, bk_batch_wait): n_regions rows of *n_fields int32, row-major, library-owned,
+ * valid until the next call on the handle.  Copied from the device on request (nothing is copied when it
+ * is not asked for).  BK_ERR_ARG while a batch is in flight or before any result. */
+int bk_region_report(bk_handle_t h, const int32_t** table, int32_t* n_fields);
+
 int bk_compare_kmers_resident(bk_handle_t h, bk_batch_result* out);
 int bk_kernel_times(bk_handle_t h, const char** names, const double** ms, const int64_t** launches, int32_t* n);
 int bk_kernel_times_reset(bk_handle_t h, int enable);
