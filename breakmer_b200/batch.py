@@ -263,6 +263,12 @@ def any_failed(res):
     return n > 0 and bool(np.ctypeslib.as_array(res.region_status, shape=(n,)).any())
 
 
+def region_report_if(handle, res, wanted):
+    """region_report(handle) if `wanted` or a region of `res`, the handle's last result, failed; else None.  A default
+    call reads nothing more, and the reason of a failed region is always known."""
+    return region_report(handle) if (wanted or any_failed(res)) else None
+
+
 def submit(handle, packed=None):
     """bk_batch_submit: enqueue the device pass of `packed` (None: the batch uploaded with `upload`) and return.
     `packed` must stay alive until `wait` has returned."""

@@ -13,12 +13,14 @@ Two ways to run it:
     (call c on rank c % N) or handed out by `CallQueue` -- an atomic counter in the
     torch.distributed key-value store, host side, no device traffic -- so that a rank whose calls
     turn out slow takes fewer of them; `gather_by_name` collects the per-region results on rank 0;
-  * one process, several devices: `run_sharded(regions, devices=[0, 1, ...])` -- one host
-    thread per device pulls chunks of regions from a shared queue (largest first) and keeps
-    `inflight` batches on its device with bk_batch_submit / bk_batch_wait.  This is what
-    `sv_processor.compare_kmers_batch(targets, devices=[...])` uses.
+  * one process, several devices: `run_sharded(regions, devices=[0, 1, ...])` and
+    `sv_processor.compare_kmers_batch(targets, devices=[...])` -- `plan_chunks` cuts the regions
+    into chunks of similar static cost, and `drive_chunks` runs one host thread per device that
+    pulls chunks from a shared queue (largest first) and keeps `inflight` batches on its device
+    with bk_batch_submit / bk_batch_wait.
 """
 import hashlib
+import queue
 import threading
 
 import numpy as np
@@ -187,7 +189,7 @@ class DevicePipeline:
         from . import batch
         j, packed, tag = self._queue.pop(0)
         res = batch.wait(self.handles[j], packed, decode=decode)
-        res.report = batch.region_report(self.handles[j]) if (self.report or batch.any_failed(res)) else None
+        res.report = batch.region_report_if(self.handles[j], res, self.report)
         return res, packed, tag
 
     def pending(self):
@@ -199,61 +201,94 @@ class DevicePipeline:
         self.handles = []
 
 
-def run_sharded(regions, devices=(0,), max_regions=2048, inflight=3, costs=None, pack=None, on_result=None, long_regions=False):
-    """The region loop of sv_processor.py:185-201 over several GPUs of one box, single process.
+def plan_chunks(costs, n_devices, max_per_chunk, key=None):
+    """Chunks of similar static cost: consecutive runs of the indices ordered most expensive first (ties by index), at
+    least one chunk per device and at most max_per_chunk indices per chunk.  Each chunk is sorted by `key` (None: by
+    index)."""
+    n = len(costs)
+    if not n:
+        return []
+    order = sorted(range(n), key=lambda i: (-costs[i], i))
+    per = -(-n // max(n_devices, -(-n // max_per_chunk)))
+    return [sorted(order[a:a + per], key=key) for a in range(0, n, per)]
 
-    regions     region-like objects (see batch.PackedBatch)
-    devices     CUDA device ordinals; one host thread and `inflight` handles per device
-    pack        callable(list of regions) -> PackedBatch (default batch.PackedBatch)
-    on_result   callable(indices, BatchOutput, PackedBatch) called from the worker threads, once per chunk
-    long_regions  assemble regions with reads or contigs up to 65,535 bases in the same pass (DevicePipeline)
 
-    Chunks of at most max_regions regions are handed out dynamically, most expensive first (static `region_cost`),
-    so a device that drew cheap chunks simply takes more of them.  Returns {region name: (BatchOutput, index in it)}
-    ordered by target name (the host-side gather)."""
+def drive_chunks(chunks, devices, inflight, pack, consume, pipe=None, decode=True, long_regions=False, report=False,
+                 apply_thread=False):
+    """Run `chunks` (lists of indices) on `devices`, each device taking the next chunk when it has room for it.
+    pack(indices, slot) -> (packed, tag) parses a chunk into parse buffer `slot`; consume(result, packed, tag) takes the
+    finished batches (pipe.pop(decode)), per device in submission order.  `pipe`: an open pipeline of devices[0], driven
+    on the calling thread and left open; without it every device gets a thread and an `inflight`-handle DevicePipeline of
+    its own, closed at the end.  long_regions and report set the handles' option and DevicePipeline.report for the call.
+
+    Without apply_thread a device's thread pops the oldest batch of a full pipeline before it parses the next chunk, and
+    one parse slot per handle rotates.  With apply_thread a second thread pops and consumes while the first parses ahead,
+    so one more slot rotates, and a handle is free again only once its chunk has been consumed (the result arrays live in
+    the handle's arena).  The first error of any thread is re-raised on the calling thread after every thread stopped."""
     from . import batch
-    pack = pack or batch.PackedBatch
-    costs = list(costs) if costs is not None else [region_cost(r) for r in regions]
-    order = sorted(range(len(regions)), key=lambda i: (-costs[i], i))
-    # chunks of similar cost: consecutive runs of the cost-sorted order, restored to input order inside a chunk
-    n_chunks = max(len(devices), (len(regions) + max_regions - 1) // max_regions) if regions else 0
-    per = (len(regions) + n_chunks - 1) // n_chunks if n_chunks else 0
-    chunks = [sorted(order[a:a + per]) for a in range(0, len(order), per)] if per else []
+    todo = iter(chunks)
     lock = threading.Lock()
-    cursor = [0]
-    results = {}
-    errors = []
 
     def take():
         with lock:
-            if cursor[0] >= len(chunks):
-                return None
-            c = chunks[cursor[0]]
-            cursor[0] += 1
-            return c
+            return next(todo, None)
+
+    def run(pipe):
+        def drain_one():
+            consume(*pipe.pop(decode=decode))
+
+        n_handles = len(pipe.handles)
+        free = threading.Semaphore(n_handles)
+        posted = queue.SimpleQueue()                     # one True per submitted batch, then False
+        apply_errors = []
+
+        def applier():
+            try:
+                while posted.get():
+                    drain_one()
+                    free.release()
+            except Exception as e:                       # noqa: BLE001 -- re-raised on the submitting thread
+                apply_errors.append(e)
+                free.release()
+
+        pipe.report = report
+        with batch.long_regions(pipe.handles, long_regions):
+            if apply_thread:
+                helper = threading.Thread(target=applier)
+                helper.start()
+            try:
+                n = 0
+                while not apply_errors and (idx := take()) is not None:
+                    if not apply_thread and pipe.full():
+                        drain_one()
+                    packed, tag = pack(idx, n % (n_handles + 1 if apply_thread else n_handles))
+                    if apply_thread:
+                        free.acquire()
+                        if apply_errors:
+                            break
+                    pipe.submit(packed, tag)
+                    n += 1
+                    if apply_thread:
+                        posted.put(True)
+                while not apply_thread and pipe.pending():
+                    drain_one()
+            finally:
+                if apply_thread:
+                    posted.put(False)
+                    helper.join()
+        if apply_errors:
+            raise apply_errors[0]
+
+    if pipe is not None:
+        run(pipe)
+        return
+    errors = []
 
     def worker(dev):
         pipe = None
         try:
-            pipe = DevicePipeline(dev, inflight=inflight, long_regions=long_regions)
-
-            def drain_one():
-                out, pk, idx = pipe.pop()
-                if on_result is not None:
-                    on_result(idx, out, pk)
-                with lock:
-                    for j, i in enumerate(idx):
-                        results[pk.names[j]] = (out, j)
-
-            while True:
-                idx = take()
-                if idx is None:
-                    break
-                if pipe.full():
-                    drain_one()
-                pipe.submit(pack([regions[i] for i in idx]), idx)
-            while pipe.pending():
-                drain_one()
+            pipe = DevicePipeline(dev, inflight=inflight)
+            run(pipe)
         except Exception as e:                           # noqa: BLE001 -- re-raised on the calling thread
             errors.append(e)
         finally:
@@ -267,4 +302,33 @@ def run_sharded(regions, devices=(0,), max_regions=2048, inflight=3, costs=None,
         t.join()
     if errors:
         raise errors[0]
+
+
+def run_sharded(regions, devices=(0,), max_regions=2048, inflight=3, costs=None, pack=None, on_result=None, long_regions=False):
+    """The region loop of sv_processor.py:185-201 over several GPUs of one box, single process.
+
+    regions     region-like objects (see batch.PackedBatch)
+    devices     CUDA device ordinals; one host thread and `inflight` handles per device
+    pack        callable(list of regions) -> PackedBatch (default batch.PackedBatch)
+    on_result   callable(indices, BatchOutput, PackedBatch) called from the worker threads, once per chunk
+    long_regions  assemble regions with reads or contigs up to 65,535 bases in the same pass
+
+    Chunks of at most max_regions regions (plan_chunks on the static `region_cost`, regions in input order inside a
+    chunk) are handed out dynamically, most expensive first (drive_chunks).  Returns {region name: (BatchOutput, index
+    in it)} ordered by target name (the host-side gather)."""
+    from . import batch
+    pack = pack or batch.PackedBatch
+    costs = list(costs) if costs is not None else [region_cost(r) for r in regions]
+    lock = threading.Lock()
+    results = {}
+
+    def consume(out, pk, idx):
+        if on_result is not None:
+            on_result(idx, out, pk)
+        with lock:
+            for j in range(len(idx)):
+                results[pk.names[j]] = (out, j)
+
+    drive_chunks(plan_chunks(costs, len(devices), max_regions), devices, inflight,
+                 lambda idx, slot: (pack([regions[i] for i in idx]), idx), consume, long_regions=long_regions)
     return dict(sorted(results.items()))

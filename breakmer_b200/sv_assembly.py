@@ -237,7 +237,7 @@ def _assemble_calls(calls, device, long_regions, want_report=False):
     h = get_handle(device)
     with batch.long_regions([h], long_regions):
         out = batch.run(h, pk)
-        rows = batch.region_report(h) if (want_report or batch.any_failed(out)) else None
+        rows = batch.region_report_if(h, out, want_report)
     objs = [o for inp in inputs for o in inp.objs]
     result = []
     bad = []

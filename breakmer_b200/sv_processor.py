@@ -241,7 +241,7 @@ def compare_kmers_batch(targets, device=0, ingest="python", write_contigs=False,
         h = get_handle(devices[0])
         with batch.long_regions([h], long_regions):
             res = batch.run(h, pk, decode=False)
-            rows = batch.region_report(h) if (report is not None or batch.any_failed(res)) else None
+            rows = batch.region_report_if(h, res, report is not None)
         _apply_chunk(targets, pk, res, ks, objs, ingest, write_contigs, failed)
         _record_report(targets, rows, failed, reasons, report)
     else:
@@ -268,127 +268,36 @@ def _sharded(targets, devices, ingest, write_contigs, max_targets, inflight, fai
              reasons=None, report=None):
     """Chunked, pipelined (and with several devices region-sharded) pass: sv_processor.py:185-201 over `devices`."""
     import threading
-    costs = [_target_cost(t) for t in targets]
-    order = sorted(range(len(targets)), key=lambda i: (-costs[i], i))
-    n_chunks = max(len(devices), (len(targets) + max_targets - 1) // max_targets)
-    per = (len(targets) + n_chunks - 1) // n_chunks
-    by_name = sorted(range(len(targets)), key=lambda i: targets[i].name)           # sv_processor.py:175-176
-    rank_of = {i: r for r, i in enumerate(by_name)}
-    chunks = [sorted(order[a:a + per], key=lambda i: rank_of[i]) for a in range(0, len(order), per)]
+    from . import shard
     lock = threading.Lock()
-    cursor = [0]
-    errors = []
 
-    def take():
+    def pack(idx, slot):
+        chunk = [targets[i] for i in idx]
+        pk, ks, objs = _pack_targets(chunk, ingest, slot=slot)
+        # the applying thread's writer: made here so that it is cached under the submitting thread's key
+        apply_ing = _get_ingest("apply") if (apply_thread and ingest == "native") else None
+        return pk, (chunk, ks, objs, apply_ing)
+
+    def consume(res, pk, tag):
+        chunk, ks, objs, apply_ing = tag
+        mine = []
+        _apply_chunk(chunk, pk, res, ks, objs, ingest, write_contigs, mine, apply_ing)
         with lock:
-            if cursor[0] >= len(chunks):
-                return None
-            c = chunks[cursor[0]]
-            cursor[0] += 1
-            return c
+            failed.extend(mine)
+            _record_report(chunk, getattr(res, "report", None), mine, reasons, report)
 
-    def worker(dev, own_pipe):
-        from . import shard
-        n_sub = 0
-        pipe = None
-        try:
-            pipe = shard.DevicePipeline(dev, inflight=inflight) if own_pipe else _get_pipe(dev, inflight)
-            pipe.report = report is not None                 # (pop reads the report of a batch with a failed region anyway)
-            with batch.long_regions(pipe.handles, long_regions):
-                # (the writer the applying thread uses: made here so that it is cached under the calling thread's key)
-                apply_ing = _get_ingest("apply") if (apply_thread and ingest == "native") else None
-
-                def drain_one():
-                    res, pk, tag = pipe.pop(decode=False)
-                    chunk, ks, objs = tag
-                    mine = []
-                    _apply_chunk(chunk, pk, res, ks, objs, ingest, write_contigs, mine, apply_ing)
-                    with lock:
-                        failed.extend(mine)
-                        _record_report(chunk, getattr(res, "report", None), mine, reasons, report)
-
-                if apply_thread:
-                    # this thread parses and submits; a second one takes the results in submission order and applies them.
-                    # A handle is free again only when its chunk has been applied (the result arrays live in its arena).
-                    free = threading.Semaphore(inflight)
-                    submitted = []                           # grows by append only; the applier follows it by index
-                    more = threading.Condition()
-                    state = {"done": False}
-
-                    def applier():
-                        at = 0
-                        try:
-                            while True:
-                                with more:
-                                    while at >= len(submitted) and not state["done"]:
-                                        more.wait()
-                                    if at >= len(submitted):
-                                        return
-                                at += 1
-                                drain_one()
-                                free.release()
-                        except Exception as e:               # noqa: BLE001 -- re-raised on the calling thread
-                            errors.append(e)
-                            state["failed"] = True
-                            free.release()
-
-                    helper = threading.Thread(target=applier)
-                    helper.start()
-                    try:
-                        while not state.get("failed"):
-                            idx = take()
-                            if idx is None:
-                                break
-                            chunk = [targets[i] for i in idx]
-                            pk, ks, objs = _pack_targets(chunk, ingest, slot=n_sub % (inflight + 1))
-                            free.acquire()
-                            if state.get("failed"):
-                                break
-                            n_sub += 1
-                            pipe.submit(pk, (chunk, ks, objs))
-                            with more:
-                                submitted.append(n_sub)
-                                more.notify()
-                    finally:
-                        with more:
-                            state["done"] = True
-                            more.notify()
-                        helper.join()
-                    if state.get("failed"):
-                        raise errors.pop()
-                    return
-                while True:
-                    idx = take()
-                    if idx is None:
-                        break
-                    chunk = [targets[i] for i in idx]
-                    if pipe.full():
-                        drain_one()
-                    # (a native ingest buffer is reused call to call: `inflight` of them rotate under the batches in flight)
-                    pk, ks, objs = _pack_targets(chunk, ingest, slot=n_sub % inflight)
-                    n_sub += 1
-                    pipe.submit(pk, (chunk, ks, objs))
-                while pipe.pending():
-                    drain_one()
-        except Exception as e:                           # noqa: BLE001 -- re-raised on the calling thread
-            errors.append(e)
-            if pipe is not None and not own_pipe:        # a cached pipeline with batches in flight is not reusable
-                _pipes.pop((threading.get_ident(), dev, inflight), None)
-                pipe.close()
-        finally:
-            if pipe is not None and own_pipe:
-                pipe.close()
-
-    if len(devices) == 1:
-        worker(devices[0], False)                        # one device: the calling thread drives it (handles are kept)
-    else:
-        threads = [threading.Thread(target=worker, args=(d, True)) for d in devices]
-        for t in threads:
-            t.start()
-        for t in threads:
-            t.join()
-    if errors:
-        raise errors[0]
+    chunks = shard.plan_chunks([_target_cost(t) for t in targets], len(devices), max_targets,
+                               key=lambda i: (targets[i].name, i))               # sv_processor.py:175-176
+    # one device: the calling thread drives it, and its handles keep their arenas from call to call
+    pipe = _get_pipe(devices[0], inflight) if len(devices) == 1 else None
+    try:
+        shard.drive_chunks(chunks, devices, inflight, pack, consume, pipe, decode=False, long_regions=long_regions,
+                           report=report is not None, apply_thread=apply_thread)
+    except Exception:
+        if pipe is not None:                             # a pipeline with batches in flight is not reusable
+            _pipes.pop((threading.get_ident(), devices[0], inflight), None)
+            pipe.close()
+        raise
 
 
 def _target_cost(trgt):

@@ -1,12 +1,14 @@
-"""Host logic of sv_processor.compare_kmers_batch's chunked pass (no device: the pipeline, the parser and the result
-application are replaced by recording fakes).  What is under test is the scheduling: every target applied exactly once,
-never more chunks un-applied than there are handles, errors of either thread reach the caller without a hang."""
+"""Host logic of sv_processor.compare_kmers_batch's chunked pass and of shard.run_sharded (no device: the pipeline, the
+parser and the result application are replaced by recording fakes).  What is under test is the scheduling: every target
+applied exactly once, never more chunks un-applied than there are handles, errors of either thread reach the caller
+without a hang."""
+import itertools
 import threading
 import time
 
 import pytest
 
-from breakmer_b200 import sv_processor
+from breakmer_b200 import shard, sv_processor
 
 
 class _T:
@@ -46,9 +48,13 @@ class _FakePipe:
         self.closed = True
 
 
+def _new_log():
+    return {"lock": threading.Lock(), "submitted": 0, "applied": 0, "max_unapplied": 0, "order": [], "threads": set(),
+            "packed": 0, "slots": []}
+
+
 def _install(monkeypatch, inflight, fail_apply_at=None, fail_pack_at=None):
-    log = {"lock": threading.Lock(), "submitted": 0, "applied": 0, "max_unapplied": 0, "order": [], "threads": set(),
-           "packed": 0, "slots": []}
+    log = _new_log()
     pipe = _FakePipe(inflight, log)
     monkeypatch.setattr(sv_processor, "_get_pipe", lambda dev, n: pipe)
     monkeypatch.setattr(sv_processor, "_get_ingest", lambda slot=0: "ingest-%s" % slot)
@@ -108,3 +114,72 @@ def test_errors_of_either_side_reach_the_caller(monkeypatch, apply_thread):
     with pytest.raises(ValueError, match="pack failed"):
         sv_processor.compare_kmers_batch(targets, ingest="native", max_targets=5, apply_thread=apply_thread)
     assert pipe.closed
+
+
+class _Packed:
+    def __init__(self, regions):
+        self.names = [r.name for r in regions]
+
+
+def _install_pipes(monkeypatch):
+    """shard.DevicePipeline -> a _FakePipe with a log of its own per worker thread; -> (every pipe made, applied() to
+    call from the thread that consumed a chunk)"""
+    pipes = []
+    mine = threading.local()
+
+    def make(dev, inflight, **options):
+        mine.pipe = _FakePipe(inflight, _new_log())
+        pipes.append(mine.pipe)
+        return mine.pipe
+
+    def applied():
+        with mine.pipe.log["lock"]:
+            mine.pipe.log["applied"] += 1
+
+    monkeypatch.setattr(shard, "DevicePipeline", make)
+    return pipes, applied
+
+
+@pytest.mark.parametrize("n,n_devices,max_regions,inflight", [(50, 1, 7, 3), (50, 3, 7, 2), (23, 2, 5, 1), (3, 4, 5, 2)])
+def test_run_sharded_returns_every_region_once(monkeypatch, n, n_devices, max_regions, inflight):
+    pipes, applied = _install_pipes(monkeypatch)
+    regions = [_T(i, 0) for i in range(n)][::-1]                 # names against input order
+    chunks = []
+
+    def on_result(idx, out, pk):
+        assert out == ("res", pk) and pk.names == [regions[i].name for i in idx]
+        assert threading.get_ident() != here
+        applied()
+        chunks.append(idx)
+
+    here = threading.get_ident()
+    got = shard.run_sharded(regions, devices=list(range(n_devices)), max_regions=max_regions, inflight=inflight,
+                            costs=[(i * 37) % 11 for i in range(n)], pack=_Packed, on_result=on_result)
+    assert list(got) == sorted(r.name for r in regions)
+    assert all(out[1].names[j] == name for name, (out, j) in got.items())
+    assert sorted(i for idx in chunks for i in idx) == list(range(n))
+    assert all(idx == sorted(idx) and len(idx) <= max_regions for idx in chunks)
+    assert len(chunks) >= min(n, n_devices)
+    assert len(pipes) == n_devices and all(p.closed and p.pending() == 0 for p in pipes)
+
+
+@pytest.mark.parametrize("fail", ["pack", "consume"])
+def test_run_sharded_errors_reach_the_caller(monkeypatch, fail):
+    pipes, applied = _install_pipes(monkeypatch)
+    regions = [_T(i, 3) for i in range(40)]
+    calls = itertools.count(1)
+
+    def pack(rs):
+        if fail == "pack" and next(calls) == 4:
+            raise ValueError("pack failed")
+        return _Packed(rs)
+
+    def on_result(idx, out, pk):
+        if fail == "consume" and next(calls) == 2:
+            raise RuntimeError("consume failed")
+        applied()
+
+    with pytest.raises(ValueError if fail == "pack" else RuntimeError, match=fail + " failed"):
+        shard.run_sharded(regions, devices=[0, 1], max_regions=5, inflight=2, costs=[1.0] * 40, pack=pack,
+                          on_result=on_result)
+    assert len(pipes) == 2 and all(p.closed for p in pipes)
