@@ -116,6 +116,7 @@ def load():
     lib.bk_ref_cache_build.argtypes = [H, c_void_p, c_void_p, c_int32, c_int32]
     lib.bk_ref_cache_clear.argtypes = [H]
     lib.bk_region_report.argtypes = [H, POINTER(POINTER(c_int32)), POINTER(c_int32)]
+    lib.bk_rejected_contigs.argtypes = [H, POINTER(POINTER(c_int64)), POINTER(POINTER(c_int32)), POINTER(c_int64)]
     lib.bk_ingest_create.argtypes = [c_int, c_int, POINTER(H)]
     lib.bk_ingest_destroy.argtypes = [H]
     lib.bk_ingest_last_error.argtypes = [H]
@@ -133,7 +134,7 @@ def load():
     for name in ("bk_create", "bk_destroy", "bk_nw_batch", "bk_dedup_reads", "bk_count_kmers", "bk_sample_only",
                  "bk_compare_kmers_batch", "bk_compare_kmers_long", "bk_batch_submit", "bk_batch_wait", "bk_batch_upload",
                  "bk_compare_kmers_resident", "bk_kernel_times", "bk_kernel_times_reset", "bk_set_option", "bk_ref_cache_build",
-                 "bk_ref_cache_clear", "bk_region_report"):
+                 "bk_ref_cache_clear", "bk_region_report", "bk_rejected_contigs"):
         getattr(lib, name).restype = c_int
     _lib = lib
     return lib
@@ -143,6 +144,7 @@ EXPORTED_SYMBOLS = (
     "bk_version", "bk_device_count", "bk_create", "bk_destroy", "bk_last_error", "bk_nw_batch", "bk_dedup_reads",
     "bk_count_kmers", "bk_sample_only", "bk_compare_kmers_batch", "bk_compare_kmers_long", "bk_batch_submit", "bk_batch_wait", "bk_batch_upload", "bk_compare_kmers_resident", "bk_kernel_times",
     "bk_kernel_times_reset", "bk_set_option", "bk_ref_cache_build", "bk_ref_cache_clear", "bk_region_report",
+    "bk_rejected_contigs",
     "bk_ingest_create", "bk_ingest_destroy", "bk_ingest_last_error", "bk_ingest_buffers", "bk_ingest_files",
     "bk_write_contigs", "bk_write_sample_kmers")
 
@@ -287,6 +289,19 @@ class Handle:
         if n == 0:
             return np.zeros((0, nf.value), np.int32)
         return np.ctypeslib.as_array(table, shape=(int(n), nf.value)).copy()
+
+    def rejected_contigs(self):
+        """bk_rejected_contigs: the rejected contigs of the handle's last result (a batch uploaded with the
+        "rejected_contigs" option) as copies (reg_off int64[n_regions + 1], reason int32[n]): rejected contig j of region
+        r has j in [reg_off[r], reg_off[r + 1]) and its payload at index n_contigs + j of the result's tables.  Read it
+        before the handle's next call."""
+        reg_off, reason, n = POINTER(c_int64)(), POINTER(c_int32)(), c_int64()
+        self._check(self.lib.bk_rejected_contigs(self.h, byref(reg_off), byref(reason), byref(n)))
+        if self.result_regions is None:
+            raise BreakmerError(BK_ERR_ARG, "rejected_contigs: no result of batch.run / batch.wait on this handle")
+        off = np.ctypeslib.as_array(reg_off, shape=(int(self.result_regions) + 1,)).copy()
+        why = np.ctypeslib.as_array(reason, shape=(n.value,)).copy() if n.value else np.zeros(0, np.int32)
+        return off, why
 
     # ---- timers -------------------------------------------------------------------------
     def kernel_times_reset(self, enable=True):

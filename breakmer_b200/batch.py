@@ -116,11 +116,14 @@ def _arr(ptr, n, dtype):
 
 
 class BatchOutput:
-    """Copies of the library-owned result arrays of one call."""
+    """Copies of the library-owned result arrays of one call.  `rejected`: the call's rejected_tables, or None; with them
+    the contig tables also hold the rejected contigs, after the n_contigs accepted ones."""
 
-    def __init__(self, res, packed):
+    def __init__(self, res, packed, rejected=None):
         R = res.n_regions
         C = int(res.n_contigs)
+        self.rej_reg_off, self.rej_reason = rejected if rejected is not None else (None, None)
+        n_all = C + (len(self.rej_reason) if rejected is not None else 0)
         self.k = packed.k
         self._kmer_str = None
         self.n_regions = R
@@ -135,14 +138,14 @@ class BatchOutput:
         self.uniq_rec = _arr(res.uniq_rec, NU, np.int32)
         self.uniq_mult = _arr(res.uniq_mult, NU, np.uint32)
         self.ctg_reg_off = _arr(res.ctg_reg_off, R + 1, np.int64)
-        self.seq_off = _arr(res.ctg_seq_off, 2 * C, np.int64).reshape(C, 2)
-        self.cnt_off = _arr(res.ctg_cnt_off, 2 * C, np.int64).reshape(C, 2)
-        self.reads_off = _arr(res.ctg_reads_off, 2 * C, np.int64).reshape(C, 2)
-        self.kmers_off = _arr(res.ctg_kmers_off, 2 * C, np.int64).reshape(C, 2)
-        n_seq = int((self.seq_off[:, 0] + self.seq_off[:, 1]).max()) if C else 0
-        n_cnt = int((self.cnt_off[:, 0] + self.cnt_off[:, 1]).max()) if C else 0
-        n_rd = int((self.reads_off[:, 0] + self.reads_off[:, 1]).max()) if C else 0
-        n_km = int((self.kmers_off[:, 0] + self.kmers_off[:, 1]).max()) if C else 0
+        self.seq_off = _arr(res.ctg_seq_off, 2 * n_all, np.int64).reshape(n_all, 2)
+        self.cnt_off = _arr(res.ctg_cnt_off, 2 * n_all, np.int64).reshape(n_all, 2)
+        self.reads_off = _arr(res.ctg_reads_off, 2 * n_all, np.int64).reshape(n_all, 2)
+        self.kmers_off = _arr(res.ctg_kmers_off, 2 * n_all, np.int64).reshape(n_all, 2)
+        n_seq = int((self.seq_off[:, 0] + self.seq_off[:, 1]).max()) if n_all else 0
+        n_cnt = int((self.cnt_off[:, 0] + self.cnt_off[:, 1]).max()) if n_all else 0
+        n_rd = int((self.reads_off[:, 0] + self.reads_off[:, 1]).max()) if n_all else 0
+        n_km = int((self.kmers_off[:, 0] + self.kmers_off[:, 1]).max()) if n_all else 0
         self.seq = _arr(ctypes.cast(res.ctg_seq, ctypes.POINTER(ctypes.c_uint8)), n_seq, np.uint8)
         self.kmer_locs = _arr(res.ctg_kmer_locs, n_seq, np.int32)
         self.indel_only = _arr(res.ctg_indel_only, n_cnt, np.int32)
@@ -173,29 +176,57 @@ class BatchOutput:
             self._kmer_str = _lib.codes_to_mers(self.kmer_mer, self.k)
         return self._kmer_str
 
+    def _record(self, c, with_reads):
+        so, sl = self.seq_off[c]
+        co, cl = self.cnt_off[c]
+        ro, nr = self.reads_off[c]
+        ko, nk = self.kmers_off[c]
+        ks = self._kmer_strings()
+        kmers = [list(t) for t in zip(ks[ko:ko + nk], self.kmer_pos[ko:ko + nk].tolist(), self.kmer_lth[ko:ko + nk].tolist(),
+                                      self.kmer_dist[ko:ko + nk].tolist(),
+                                      [ORDER_NAMES[o] for o in self.kmer_order[ko:ko + nk].tolist()])]
+        return {
+            "seq": self.seq[so:so + sl].tobytes().decode(),
+            "indel_only": self.indel_only[co:co + cl].tolist(),
+            "others": self.others[co:co + cl].tolist(),
+            "reads": sorted(self.read_ids[int(i)] for i in self.reads[ro:ro + nr]) if with_reads else None,
+            "kmers": kmers,
+            "kmer_locs": self.kmer_locs[so:so + sl].tolist(),
+        }
+
     def contig_records(self, r, with_reads=True):
         """Contigs of region r in acceptance order, in the canonical comparable form
         (same shape as oracle.assembler_py.contig_record).  with_reads=False leaves "reads" out (callers that map
         ctg_reads to their own read objects do not need the sorted id list)."""
-        out = []
-        for c in range(int(self.ctg_reg_off[r]), int(self.ctg_reg_off[r + 1])):
-            so, sl = self.seq_off[c]
-            co, cl = self.cnt_off[c]
-            ro, nr = self.reads_off[c]
-            ko, nk = self.kmers_off[c]
-            ks = self._kmer_strings()
-            kmers = [list(t) for t in zip(ks[ko:ko + nk], self.kmer_pos[ko:ko + nk].tolist(), self.kmer_lth[ko:ko + nk].tolist(),
-                                          self.kmer_dist[ko:ko + nk].tolist(),
-                                          [ORDER_NAMES[o] for o in self.kmer_order[ko:ko + nk].tolist()])]
-            out.append({
-                "seq": self.seq[so:so + sl].tobytes().decode(),
-                "indel_only": self.indel_only[co:co + cl].tolist(),
-                "others": self.others[co:co + cl].tolist(),
-                "reads": sorted(self.read_ids[int(i)] for i in self.reads[ro:ro + nr]) if with_reads else None,
-                "kmers": kmers,
-                "kmer_locs": self.kmer_locs[so:so + sl].tolist(),
-            })
-        return out
+        return [self._record(c, with_reads) for c in range(int(self.ctg_reg_off[r]), int(self.ctg_reg_off[r + 1]))]
+
+    def rejected_indices(self, r):
+        """-> [(reason name, contig index into the tables), ...]: the rejected contigs of region r in growth order
+        (REJECT_REASONS); ValueError for a result without the rejected tables"""
+        if self.rej_reg_off is None:
+            raise ValueError("rejected contigs: the result was made without the \"rejected_contigs\" option")
+        a, b = int(self.rej_reg_off[r]), int(self.rej_reg_off[r + 1])
+        return [(REJECT_REASONS[why], self.n_contigs + j) for j, why in zip(range(a, b), self.rej_reason[a:b].tolist())]
+
+    def rejected_records(self, r, with_reads=True):
+        """[(reason, record), ...]: the contigs of region r the acceptance test dropped, in growth order, reason
+        "support" or "length", record in the contig_records form"""
+        return [(why, self._record(c, with_reads)) for why, c in self.rejected_indices(r)]
+
+
+# bk_rejected_contigs (include/breakmer_b200.h): reason names of BK_REJ_SUPPORT (1) and BK_REJ_LENGTH (2)
+REJECT_REASONS = (None, "support", "length")
+
+
+def rejected_tables(handle):
+    """Handle.rejected_contigs() of the handle's last result, or None when that result holds no rejected contigs (its
+    batch was uploaded with the "rejected_contigs" option off).  Read it before the handle's next call."""
+    try:
+        return handle.rejected_contigs()
+    except _lib.BreakmerError as e:
+        if e.code != _lib.BK_ERR_ARG:
+            raise
+        return None
 
 
 def run(handle, packed, resident=False, decode=True, long=False):
@@ -215,22 +246,31 @@ def run(handle, packed, resident=False, decode=True, long=False):
     handle.result_regions = res.n_regions
     if not decode:
         return res
-    return BatchOutput(res, packed)
+    return BatchOutput(res, packed, rejected_tables(handle))
 
 
 @contextlib.contextmanager
-def long_regions(handles, on=True):
-    """The handles' "long_regions" option for the duration of a call (on=False: untouched), then 0 (the default) again,
-    so that later calls on handles the caller shares still report long regions.  Closed handles are skipped."""
+def options(handles, **on):
+    """The handles' 0 | 1 options named with a true value (e.g. long_regions=True, rejected_contigs=True) set to 1 for
+    the duration of a call, then 0 (the default) again, so that later calls on handles the caller shares get the default
+    behaviour.  Options given a false value are left untouched.  Closed handles are skipped."""
+    names = [name for name, value in on.items() if value]
+
     def set_all(value):
-        for h in handles if on else ():
+        for h in handles if names else ():
             if h.h:
-                h.set_option("long_regions", value)
+                for name in names:
+                    h.set_option(name, value)
     set_all(1)
     try:
         yield
     finally:
         set_all(0)
+
+
+def long_regions(handles, on=True):
+    """options(handles, long_regions=on)"""
+    return options(handles, long_regions=on)
 
 
 # bk_region_report (include/breakmer_b200.h): the BK_RR_* fields in column order, and the names of the reason codes
@@ -286,7 +326,7 @@ def wait(handle, packed=None, decode=True):
     handle.result_regions = res.n_regions
     if not decode:
         return res
-    return BatchOutput(res, packed)
+    return BatchOutput(res, packed, rejected_tables(handle))
 
 
 def upload(handle, packed):

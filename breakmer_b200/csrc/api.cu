@@ -27,6 +27,7 @@ struct bk_handle_s {
   int sm_count = 148;
   int spec_width = 0;      // assembler speculation width (bk_set_option); 0 = choose per batch
   int long_regions = 0;    // bk_set_option "long_regions": the batched entries also assemble regions up to 65,535 bases
+  int rejected_contigs = 0;  // bk_set_option "rejected_contigs": results also hold the contigs the acceptance test drops
   cudaEvent_t sync_ev = nullptr;   // blocking-sync event (BK_BLOCKING_SYNC=1)
   bool spin_sync = true;
   Arena<false> dev;        // per-call device scratch
@@ -622,6 +623,9 @@ int bk_set_option(bk_handle_t h, const char* name, int64_t value) {
     } else if (strcmp(name, "long_regions") == 0) {
       if (value != 0 && value != 1) fail(BK_ERR_ARG, "long_regions must be 0 or 1");
       h->long_regions = (int)value;
+    } else if (strcmp(name, "rejected_contigs") == 0) {
+      if (value != 0 && value != 1) fail(BK_ERR_ARG, "rejected_contigs must be 0 or 1");
+      h->rejected_contigs = (int)value;
     } else {
       fail(BK_ERR_ARG, "bk_set_option: unknown option %s", name);
     }
@@ -644,6 +648,16 @@ int bk_region_report(bk_handle_t h, const int32_t** table, int32_t* n_fields) {
     if (!table || !n_fields) fail(BK_ERR_ARG, "bk_region_report: null argument");
     *table = region_report(h);
     *n_fields = RR_FIELDS;
+  });
+}
+
+static_assert(REJ_SUPPORT == BK_REJ_SUPPORT && REJ_LENGTH == BK_REJ_LENGTH,
+              "rejection reasons of common.cuh and include/breakmer_b200.h differ");
+
+int bk_rejected_contigs(bk_handle_t h, const int64_t** reg_off, const int32_t** reason, int64_t* n) {
+  return guarded(h, [&] {
+    if (!reg_off || !reason || !n) fail(BK_ERR_ARG, "bk_rejected_contigs: null argument");
+    rejected_contigs(h, reg_off, reason, n);
   });
 }
 

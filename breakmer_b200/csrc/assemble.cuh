@@ -107,6 +107,7 @@ struct AsmParams {
   int n_regions;
   int k;
   int rc_thresh;
+  int keep_rejected;               // 1: contigs that fail the acceptance test are emitted too (bk_rejected_contigs)
   int read_cap;                    // bytes of one staged-read buffer in shared memory: >= longest read + 2, multiple of 16
   // reads: raw records + unique-read table (fq_recs, utils.py:239-244, Q28)
   const uint8_t* rbases;
@@ -167,10 +168,11 @@ struct AsmParams {
   int32_t* o_io; int32_t* o_ot;
   int32_t* o_reads;
   uint64_t* o_kmer_mer; int32_t* o_kmer_pos; int32_t* o_kmer_meta;
-  int64_t* o_desc;                 // per contig 10 x int64: region, ordinal, seq_off, seq_len, cnt_off, cnt_len,
-                                   //                        reads_off, n_reads, kmers_off, n_kmers
+  int64_t* o_desc;                 // per contig 10 x int64: region, ordinal | reason << 32, seq_off, seq_len, cnt_off,
+                                   // cnt_len, reads_off, n_reads, kmers_off, n_kmers.  The ordinal counts the region's
+                                   // emitted contigs of both kinds (growth order); reason is REJ_NONE for an accepted one
   int32_t* region_status;          // per region: its status (ST_OK or the RR_* reason it stopped for)
-  int32_t* region_ncontigs;
+  int32_t* region_ncontigs;        // per region: contigs emitted (rejected ones included)
   unsigned long long* region_cells;  // per region: sum over its check_align calls of len(contig) * len(read)
   int32_t* region_report;          // per region: RR_FIELDS ints (common.cuh, bk_region_report), or null: no report
   unsigned long long* stats;       // [0] check_align calls, [1] DP cells, [2] find_reads, [3] seeds, [8..] phase cycles
@@ -1086,9 +1088,9 @@ BK_DEV void add_used_mer(RegionCtxT<T>& c, int s) {
   syncwarp();
 }
 
-// ---- set_kmer_locs (:434-438, Q25) + emit the accepted contig -------------------------------------------
+// ---- set_kmer_locs (:434-438, Q25) + emit the contig (accepted, or rejected for `reason` under keep_rejected) ----------
 template <class T>
-BK_DEV void emit_contig(RegionCtxT<T>& c) {
+BK_DEV void emit_contig(RegionCtxT<T>& c, int reason) {
   BK_PH_BEGIN
   const AsmParams& P = *c.P;
   const int k = c.k, len = c.clen;
@@ -1170,7 +1172,7 @@ BK_DEV void emit_contig(RegionCtxT<T>& c) {
   }
   if (lane() == 0) {
     int64_t* d = P.o_desc + o_ct * 10;
-    d[0] = c.region; d[1] = c.n_out; d[2] = (int64_t)o_seq; d[3] = len; d[4] = (int64_t)o_cnt; d[5] = c.klen;
+    d[0] = c.region; d[1] = (int64_t)c.n_out | ((int64_t)reason << 32); d[2] = (int64_t)o_seq; d[3] = len; d[4] = (int64_t)o_cnt; d[5] = c.klen;
     d[6] = (int64_t)o_rd; d[7] = n_reads; d[8] = (int64_t)o_km; d[9] = c.nK;
   }
   c.n_out += 1;
@@ -1295,14 +1297,19 @@ BK_DEV int total_reads(const RegionCtxT<T>& c) {                         // :178
   return warp_max_i(a) + warp_max_i(b);
 }
 
-// after grow: accept or drop (:53-59, Q21)
+// after grow: accept or drop (:53-59, Q21; support is tested first).  Under keep_rejected a dropped contig is emitted
+// as well, with its reason: the reason is decided first so that emit_contig keeps one call site (its code is large and
+// the controller's instruction footprint is what its speed depends on, DESIGN 4.2)
 template <class T>
 BK_DEV void finish_contig(RegionCtxT<T>& c, int rc_thresh, int read_len) {
   if (c.status != ST_OK) return;
   report_add(RR_GROWN, 1);
-  if (total_reads(c) < rc_thresh) { report_add(RR_REJ_SUPPORT, 1); return; }
-  if (c.clen <= read_len) { report_add(RR_REJ_LENGTH, 1); return; }
-  emit_contig(c);
+  const int reason = total_reads(c) < rc_thresh ? REJ_SUPPORT : (c.clen <= read_len ? REJ_LENGTH : REJ_NONE);
+  if (reason != REJ_NONE) {
+    report_add(RR_REJ_SUPPORT - REJ_SUPPORT + reason, 1);
+    if (!c.P->keep_rejected) return;
+  }
+  emit_contig(c, reason);
 }
 
 // ---- akmers.has_mers + mers.items()[0] (:43-45, :318-322; seed order Q7) ----------------------------------------

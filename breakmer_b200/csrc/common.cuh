@@ -111,6 +111,10 @@ enum {
 };
 enum { RR_OK = 0, RR_READ_TOO_LONG, RR_CONTIG_TOO_LONG, RR_KMER_LIST_FULL, RR_TOO_MANY_CONTIGS, RR_OUTPUT_ARENA };
 enum { RR_PASS_NONE = 0, RR_PASS_BATCHED, RR_PASS_LONG };
+// why a grown contig failed the acceptance test (AsmParams::keep_rejected, bk_rejected_contigs): the BK_REJ_* values;
+// RR_REJ_SUPPORT - REJ_SUPPORT + reason is its report counter
+enum { REJ_NONE = 0, REJ_SUPPORT, REJ_LENGTH };
+static_assert(RR_REJ_LENGTH == RR_REJ_SUPPORT + REJ_LENGTH - REJ_SUPPORT, "report counters follow the rejection reasons");
 
 // hard limits of the packed DP cell (nw.cuh): 14-bit signed score field
 constexpr int NW_MAX_LEN = 4095;

@@ -68,6 +68,7 @@ struct Pipeline {
   // the long assembler's mode, fixed at upload.  assemble_kernel takes the first n_short regions of the work order; in
   // the long modes, assemble_long_kernel takes the others and those assemble_kernel stopped
   LongMode long_mode = LONG_OFF;
+  bool keep_rejected = false;             // the "rejected_contigs" option, fixed at upload like long_mode
   int n_short = 0;                        // LONG_OFF: all; LONG_ROUTE: those without a read above NW_MAX_LEN; LONG_ALL: 0
   const uint8_t* d_routed = nullptr;      // device, per region: a read above NW_MAX_LEN (LONG_ROUTE; null when none)
   int max_short_read_len = 0;             // longest read of the other regions (sizes assemble_kernel's read buffers)
@@ -123,6 +124,11 @@ struct PendingBatch {
   std::vector<int32_t> h_reason;           // the device's region_status: 0 or the RR_* reason
   std::vector<int32_t> long_queue;         // the regions assemble_long_kernel ran (the long modes)
   std::vector<int32_t> h_report;           // host copy, made on request
+  // the rejected contigs of the result (bk_rejected_contigs; keep_rejected: the batch was uploaded with the option on):
+  // per region offsets into them and their reasons, growth order; their payload is at n_contigs + j of the ctg_* tables
+  bool keep_rejected = false;
+  std::vector<int64_t> rej_reg_off;
+  std::vector<int32_t> rej_reason;
 };
 
 }  // namespace bk

@@ -76,6 +76,7 @@ void upload_record_set(bk_handle_t h, Arena<false>& A, const char* bases, const 
 void pipeline_upload_into(bk_handle_t h, Arena<false>& A, const bk_batch_input* in, Pipeline& p, LongMode mode) {
   p = Pipeline();
   p.long_mode = mode;
+  p.keep_rejected = h->rejected_contigs != 0;
   const int max_len = mode == LONG_OFF ? NW_MAX_LEN : ASM_LONG_MAX_LEN;
   if (in->n_regions < 0 || in->n_regions > 65535) fail(BK_ERR_ARG, "batch: n_regions must be in 0..65535 per call");
   if (in->k < 2 || in->k > 31) fail(BK_ERR_ARG, "batch: k must be in 2..31");
@@ -567,7 +568,7 @@ void pipeline_submit(bk_handle_t h, const bk_batch_input* in, LongMode mode) {
   // ---- 5. assembly ----------------------------------------------------------------------------------------
   AsmParams& A = B.A;
   memset(&A, 0, sizeof A);
-  A.n_regions = R; A.k = k; A.rc_thresh = p.rc_thresh;
+  A.n_regions = R; A.k = k; A.rc_thresh = p.rc_thresh; A.keep_rejected = p.keep_rejected ? 1 : 0;
   A.rbases = p.reads.bases; A.roff = p.reads.off;
   A.u_off = u_off; A.u_rec = u_rec; A.u_mult = u_mult; A.u_io = u_io; A.u_len = u_len; A.read_len = p.read_len;
   A.rk_off = rk_off; A.rk_s = rk_s; A.rk_pos = rk_pos;
@@ -709,8 +710,8 @@ void pipeline_wait(bk_handle_t h, bk_batch_result* out) {
   BK_CUDA(cudaEventElapsedTime(&ms, h->ev0, h->ev1));
   out->gpu_ms = ms;
 
-  // contigs left the device in completion order; the table below puts them in
-  // (region, acceptance order) -- payload arrays stay where they are
+  // contigs left the device in completion order; the tables below put them in (region, growth order) -- payload arrays
+  // stay where they are.  The accepted contigs come first; rejected ones (keep_rejected) follow them, at n_contigs ..
   std::vector<int64_t> idx(n_desc);
   std::iota(idx.begin(), idx.end(), 0);
   if (B.route) {
@@ -724,27 +725,44 @@ void pipeline_wait(bk_handle_t h, bk_batch_result* out) {
                 return rerouted[r] && (c < snap || B.h_status[r] != ST_OK);
               }), idx.end());
   }
-  const int64_t n_ctg = (int64_t)idx.size();
+  auto reason_of = [&](int64_t c) { return (int32_t)(h_desc[c * 10 + 1] >> 32); };
+  if (p.keep_rejected)                                     // a region that stopped has no rejected contigs
+    idx.erase(std::remove_if(idx.begin(), idx.end(), [&](int64_t c) {
+                return reason_of(c) != REJ_NONE && B.h_status[h_desc[c * 10]] != ST_OK;
+              }), idx.end());
+  const auto first_rej = std::stable_partition(idx.begin(), idx.end(), [&](int64_t c) { return reason_of(c) == REJ_NONE; });
+  const int64_t n_ctg = first_rej - idx.begin(), n_all = (int64_t)idx.size();
   out->n_contigs = n_ctg;
-  std::sort(idx.begin(), idx.end(), [&](int64_t a, int64_t b) {
+  auto growth_order = [&](int64_t a, int64_t b) {
     const int64_t* da = h_desc + a * 10; const int64_t* db = h_desc + b * 10;
-    return da[0] != db[0] ? da[0] < db[0] : da[1] < db[1];
-  });
+    return da[0] != db[0] ? da[0] < db[0] : (uint32_t)da[1] < (uint32_t)db[1];
+  };
+  std::sort(idx.begin(), first_rej, growth_order);
+  std::sort(first_rej, idx.end(), growth_order);
   int64_t* t_reg = h->pin.get<int64_t>(R + 1);
-  int64_t* t_seq = h->pin.get<int64_t>(2 * n_ctg + 2);
-  int64_t* t_cnt = h->pin.get<int64_t>(2 * n_ctg + 2);
-  int64_t* t_rd = h->pin.get<int64_t>(2 * n_ctg + 2);
-  int64_t* t_km = h->pin.get<int64_t>(2 * n_ctg + 2);
+  int64_t* t_seq = h->pin.get<int64_t>(2 * n_all + 2);
+  int64_t* t_cnt = h->pin.get<int64_t>(2 * n_all + 2);
+  int64_t* t_rd = h->pin.get<int64_t>(2 * n_all + 2);
+  int64_t* t_km = h->pin.get<int64_t>(2 * n_all + 2);
   for (int r = 0; r <= R; ++r) t_reg[r] = 0;
-  for (int64_t c = 0; c < n_ctg; ++c) {
+  B.keep_rejected = p.keep_rejected;
+  B.rej_reg_off.assign(p.keep_rejected ? R + 1 : 0, 0);
+  B.rej_reason.clear();
+  for (int64_t c = 0; c < n_all; ++c) {
     const int64_t* d = h_desc + idx[c] * 10;
-    t_reg[d[0] + 1] += 1;
+    if (c < n_ctg) {
+      t_reg[d[0] + 1] += 1;
+    } else {
+      B.rej_reg_off[d[0] + 1] += 1;
+      B.rej_reason.push_back(reason_of(idx[c]));
+    }
     t_seq[2 * c] = d[2]; t_seq[2 * c + 1] = d[3];
     t_cnt[2 * c] = d[4]; t_cnt[2 * c + 1] = d[5];
     t_rd[2 * c] = d[6]; t_rd[2 * c + 1] = d[7];
     t_km[2 * c] = d[8]; t_km[2 * c + 1] = d[9];
   }
   for (int r = 0; r < R; ++r) t_reg[r + 1] += t_reg[r];
+  for (int r = 0; r < (int)B.rej_reg_off.size() - 1; ++r) B.rej_reg_off[r + 1] += B.rej_reg_off[r];
   out->ctg_reg_off = t_reg;
   out->ctg_seq_off = t_seq; out->ctg_cnt_off = t_cnt; out->ctg_reads_off = t_rd; out->ctg_kmers_off = t_km;
   // split the packed tuple meta word into the three fields of the 5-tuple
@@ -773,8 +791,12 @@ void pipeline_wait(bk_handle_t h, bk_batch_result* out) {
       const int32_t shift = (int32_t)p.rec_shift[r];
       if (!shift) continue;
       for (int64_t u = B.h_u_off[r]; u < B.h_u_off[r + 1]; ++u) h_urec[u] += shift;
-      for (int64_t c = t_reg[r]; c < t_reg[r + 1]; ++c)
-        for (int64_t e = t_rd[2 * c]; e < t_rd[2 * c] + t_rd[2 * c + 1]; ++e) h_reads[e] += shift;
+      auto shift_reads = [&](int64_t c0, int64_t c1) {
+        for (int64_t c = c0; c < c1; ++c)
+          for (int64_t e = t_rd[2 * c]; e < t_rd[2 * c] + t_rd[2 * c + 1]; ++e) h_reads[e] += shift;
+      };
+      shift_reads(t_reg[r], t_reg[r + 1]);
+      if (p.keep_rejected) shift_reads(n_ctg + B.rej_reg_off[r], n_ctg + B.rej_reg_off[r + 1]);
     }
   }
   B.report_skipped = p.region_skipped;                     // (the resident Pipeline may be replaced before the report is read)
@@ -808,6 +830,17 @@ const int32_t* region_report(bk_handle_t h) {
     row[RR_REASON] = RR_READ_TOO_LONG;
   }
   return B.h_report.data();
+}
+
+// bk_rejected_contigs: the rejected contigs of the last result, as pipeline_wait split them off
+void rejected_contigs(bk_handle_t h, const int64_t** reg_off, const int32_t** reason, int64_t* n) {
+  PendingBatch& B = h->pending;
+  if (B.active) fail(BK_ERR_ARG, "bk_rejected_contigs: a batch is in flight on this handle (call bk_batch_wait first)");
+  if (!B.has_result || B.result_epoch != h->dev.resets()) fail(BK_ERR_ARG, "bk_rejected_contigs: no result on this handle");
+  if (!B.keep_rejected) fail(BK_ERR_ARG, "bk_rejected_contigs: the last result was made with the \"rejected_contigs\" option off");
+  *reg_off = B.rej_reg_off.data();
+  *reason = B.rej_reason.empty() ? nullptr : B.rej_reason.data();
+  *n = (int64_t)B.rej_reason.size();
 }
 
 void phase_print(bk_handle_t h, const PendingBatch& B) {

@@ -154,9 +154,10 @@ def digest_of_digests(by_name):
 class DevicePipeline:
     """`inflight` handles of one device driven by ONE host thread: submit keeps up to `inflight` batches queued on the
     device (bk_batch_submit), results come back in submission order (bk_batch_wait).  long_regions=True sets the
-    handles' "long_regions" option: regions with reads or contigs up to 65,535 bases are assembled in the same pass."""
+    handles' "long_regions" option: regions with reads or contigs up to 65,535 bases are assembled in the same pass.
+    rejected_contigs=True sets the option of that name: results also hold the contigs the acceptance test drops."""
 
-    def __init__(self, device, inflight=3, spec_width=0, long_regions=False):
+    def __init__(self, device, inflight=3, spec_width=0, long_regions=False, rejected_contigs=False):
         from . import _lib
         self.device = device
         self.handles = [_lib.Handle(device) for _ in range(max(1, inflight))]
@@ -166,6 +167,8 @@ class DevicePipeline:
                 h.set_option("spec_width", spec_width)
             if long_regions:
                 h.set_option("long_regions", 1)
+            if rejected_contigs:
+                h.set_option("rejected_contigs", 1)
         self._queue = []                               # (handle index, packed, tag) in submission order
         self.report = False                            # pop: read every batch's per-region report
         self._next = 0
@@ -185,11 +188,14 @@ class DevicePipeline:
     def pop(self, decode=True):
         """-> (result of the oldest batch in flight, its packed input, its tag).  The result's `.report` is the batch's
         batch.region_report, read before its handle takes another batch, if `self.report` is set or a region of the
-        batch failed; else None."""
+        batch failed; else None.  With decode=False its `.rejected` is the batch's batch.rejected_tables (None unless the
+        batch was submitted with the "rejected_contigs" option); a decoded result holds them already."""
         from . import batch
         j, packed, tag = self._queue.pop(0)
         res = batch.wait(self.handles[j], packed, decode=decode)
         res.report = batch.region_report_if(self.handles[j], res, self.report)
+        if not decode:
+            res.rejected = batch.rejected_tables(self.handles[j])
         return res, packed, tag
 
     def pending(self):
@@ -214,12 +220,13 @@ def plan_chunks(costs, n_devices, max_per_chunk, key=None):
 
 
 def drive_chunks(chunks, devices, inflight, pack, consume, pipe=None, decode=True, long_regions=False, report=False,
-                 apply_thread=False):
+                 apply_thread=False, rejected_contigs=False):
     """Run `chunks` (lists of indices) on `devices`, each device taking the next chunk when it has room for it.
     pack(indices, slot) -> (packed, tag) parses a chunk into parse buffer `slot`; consume(result, packed, tag) takes the
     finished batches (pipe.pop(decode)), per device in submission order.  `pipe`: an open pipeline of devices[0], driven
     on the calling thread and left open; without it every device gets a thread and an `inflight`-handle DevicePipeline of
-    its own, closed at the end.  long_regions and report set the handles' option and DevicePipeline.report for the call.
+    its own, closed at the end.  long_regions, rejected_contigs and report set the handles' options and
+    DevicePipeline.report for the call.
 
     Without apply_thread a device's thread pops the oldest batch of a full pipeline before it parses the next chunk, and
     one parse slot per handle rotates.  With apply_thread a second thread pops and consumes while the first parses ahead,
@@ -252,7 +259,7 @@ def drive_chunks(chunks, devices, inflight, pack, consume, pipe=None, decode=Tru
                 free.release()
 
         pipe.report = report
-        with batch.long_regions(pipe.handles, long_regions):
+        with batch.options(pipe.handles, long_regions=long_regions, rejected_contigs=rejected_contigs):
             if apply_thread:
                 helper = threading.Thread(target=applier)
                 helper.start()

@@ -66,7 +66,12 @@ class _lazy(object):
 class contig:
     """What the rest of BreaKmer reads from an sv_assembly.contig (SURVEY.md section 3.5).  The Python lists, tuples and
     fq_read objects are built from the batch's result arrays on FIRST ACCESS of each attribute: resolve_sv touches few of
-    them per contig, and building all of them eagerly costs 12x the device time of the batch."""
+    them per contig, and building all of them eagerly costs 12x the device time of the batch.
+
+    `rejected_for` is None for a contig the assembler kept, and "support" or "length" for one it grew and then dropped in
+    its acceptance test (sv_assembly.py:53-59; the rejected= lists of init_assembly_batch and compare_kmers_batch)."""
+
+    rejected_for = None
 
     def __init__(self, out, cidx, objs, kmer_len, rec=None):
         self._out = out
@@ -224,18 +229,30 @@ def _clean_mers(mers, kmer_len):
     return mers
 
 
-def _assemble_calls(calls, device, long_regions, want_report=False):
+def rejected_contigs(out, r, objs, kmer_len):
+    """The contigs of region r of a BatchOutput that the acceptance test dropped, in growth order, as `contig` objects with
+    `.rejected_for` set"""
+    res = []
+    for why, c in out.rejected_indices(r):
+        ct = contig(out, c, objs, kmer_len)
+        ct.rejected_for = why
+        res.append(ct)
+    return res
+
+
+def _assemble_calls(calls, device, long_regions, want_report=False, want_rejected=False):
     """One device pass over `calls` -> (contig list or None per call, indices of the calls reported BK_ERR_CAPACITY,
-    batch.region_report of the pass or None).  long_regions: the pass also assembles calls with reads or contigs up to
-    65,535 bases (the handle's option of that name, set for this call only).  The report is read when want_report or
-    when a call was not completed."""
+    batch.region_report of the pass or None, rejected contig list per call or None).  long_regions: the pass also
+    assembles calls with reads or contigs up to 65,535 bases (the handle's option of that name, set for this call only);
+    want_rejected sets the "rejected_contigs" option the same way.  The report is read when want_report or when a call was
+    not completed."""
     import numpy as np
     inputs = [_AssemblyInput("r%d" % i, c[1], c[2], c[3]) for i, c in enumerate(calls)]
     pk = batch.PackedBatch(inputs, rc_thresh=int(calls[0][3]))
     pk.set_mers([_clean_mers(c[0], int(c[2])) for c in calls])
     pk.read_len = np.array([int(c[4]) for c in calls] + [0], dtype=np.int32)
     h = get_handle(device)
-    with batch.long_regions([h], long_regions):
+    with batch.options([h], long_regions=long_regions, rejected_contigs=want_rejected):
         out = batch.run(h, pk)
         rows = batch.region_report_if(h, out, want_report)
     objs = [o for inp in inputs for o in inp.objs]
@@ -247,10 +264,11 @@ def _assemble_calls(calls, device, long_regions, want_report=False):
             result.append(None)
             continue
         result.append([contig(out, cidx, objs, int(c[2])) for cidx in range(int(out.ctg_reg_off[i]), int(out.ctg_reg_off[i + 1]))])
-    return result, bad, rows
+    rejected = [rejected_contigs(out, i, objs, int(c[2])) for i, c in enumerate(calls)] if want_rejected else None
+    return result, bad, rows, rejected
 
 
-def init_assembly_batch(calls, device=0, on_capacity="raise", report=None):
+def init_assembly_batch(calls, device=0, on_capacity="raise", report=None, rejected=None):
     """calls: [(mers, fq_recs, kmer_len, rc_thresh, read_len), ...] with one common
     kmer_len and rc_thresh -> list (per call) of contig lists.  One GPU pass.
 
@@ -263,12 +281,17 @@ def init_assembly_batch(calls, device=0, on_capacity="raise", report=None):
                          to 65,535 bases); a RuntimeError as with "raise" names the calls that exceed that limit.
     The RuntimeError's `.reasons` says why each of those calls was not completed ({call index: reason name}, see
     batch.REASONS).  `report`, a list, is extended with batch.region_report's dict of every call, in call order: why it
-    stopped, which pass assembled it, and what the assembler did."""
+    stopped, which pass assembled it, and what the assembler did.  `rejected`, a list, is extended with one list per call,
+    in call order, of the contigs the assembler grew and then dropped in its acceptance test (total read support below
+    rc_thresh, or not longer than read_len), in growth order, as `contig` objects with `.rejected_for` "support" or
+    "length" (the handle's "rejected_contigs" option, set for this call only); a call not completed has none."""
     if not calls:
         return []
-    result, bad, rows = _assemble_calls(calls, device, on_capacity == "assemble", report is not None)
+    result, bad, rows, rej = _assemble_calls(calls, device, on_capacity == "assemble", report is not None, rejected is not None)
     if report is not None:
         report.extend(rows)
+    if rejected is not None:
+        rejected.extend(rej)
     limit = 65535 if on_capacity == "assemble" else 4095
     if bad and on_capacity in ("raise", "assemble"):
         err = RuntimeError("init_assembly: device capacity exceeded in call(s) %s (a read or contig longer than %d bases); "

@@ -38,11 +38,13 @@ library's host threads (bk_write_contigs, SURVEY.md section 8.7 f.3).
 same device pass as all others (the handles' "long_regions" option).
 `report={}` is filled with what the assembler did for every target (batch.region_report: why it stopped, which pass
 assembled it, how many seeds, find_reads and check_align calls, and how many contigs were grown and rejected).
+`rejected={}` is filled with the contigs themselves that the assembler grew and then rejected, per target (the handles'
+"rejected_contigs" option).
 """
 import os
 
 from . import batch, get_handle, utils
-from .sv_assembly import contig, contig_list
+from .sv_assembly import contig, contig_list, rejected_contigs
 
 
 class _TargetInput:
@@ -123,7 +125,8 @@ class CapacityError(RuntimeError):
 
 
 def _apply_chunk(targets, pk, res, inputs_k, objs, ingest, write_contigs, failed, ing=None):
-    """Results of one device call -> the state target.compare_kmers leaves behind, for the targets of that call."""
+    """Results of one device call -> the state target.compare_kmers leaves behind, for the targets of that call.  Returns
+    the call's BatchOutput, which holds the rejected contigs when res.rejected (the call's batch.rejected_tables) does."""
     import numpy as np
     n = len(targets)
     status = np.ctypeslib.as_array(res.region_status, shape=(max(n, 1),))[:n].tolist()
@@ -139,7 +142,7 @@ def _apply_chunk(targets, pk, res, inputs_k, objs, ingest, write_contigs, failed
                               [p[:-4] + "_merged.out" if st == 0 else None for p, st in zip(sk_paths, status)])
         # the "<mer>\t<count>" files of the completed targets in one multi-threaded sweep (bk_write_sample_kmers)
         ing.write_sample_kmers(res, pk.k, sk_paths if all_ok else [p if st == 0 else None for p, st in zip(sk_paths, status)])
-    out = batch.BatchOutput(res, pk)
+    out = batch.BatchOutput(res, pk, getattr(res, "rejected", None))
     ctg_reg_off = out.ctg_reg_off.tolist()
     so_off = out.so_off.tolist()
     for i, trgt in enumerate(targets):
@@ -161,6 +164,13 @@ def _apply_chunk(targets, pk, res, inputs_k, objs, ingest, write_contigs, failed
         kmers['clusters'] = contig_list(out, ctg_reg_off[i], ctg_reg_off[i + 1], objs, inputs_k[i])
         trgt.cleaned_read_recs = None
         kmers['case_only'] = {}
+    return out
+
+
+def _record_rejected(targets, out, objs, inputs_k, rejected):
+    """rejected[name] = the rejected contigs of every target of one device call (out: its BatchOutput)"""
+    for i, trgt in enumerate(targets):
+        rejected[trgt.name] = rejected_contigs(out, i, objs, inputs_k[i])
 
 
 def _record_report(targets, rows, failed, reasons, report):
@@ -201,7 +211,7 @@ def _pack_targets(targets, ingest, slot=0):
 
 
 def compare_kmers_batch(targets, device=0, ingest="python", write_contigs=False, devices=None, max_targets=125, inflight=4,
-                        apply_thread=False, on_capacity="raise", report=None):
+                        apply_thread=False, on_capacity="raise", report=None, rejected=None):
     """target.compare_kmers() for many targets (the region loop of sv_processor.py:185-201 as one call).
 
     The targets are cut into chunks of at most max_targets, most expensive first (static cost, breakmer_b200.shard), and
@@ -224,7 +234,13 @@ def compare_kmers_batch(targets, device=0, ingest="python", write_contigs=False,
     targets beyond that limit.  CapacityError.reasons says why each of them was not completed.
 
     `report`, a dict, receives report[target.name] = batch.region_report's dict of the target, for every target, in every
-    form (one call, chunked, apply_thread, devices=[...])."""
+    form (one call, chunked, apply_thread, devices=[...]).
+
+    `rejected`, a dict, receives rejected[target.name] = the contigs the assembler grew for the target and then dropped
+    in its acceptance test (sv_assembly.py:53-59: total read support below the min sr_thresh, or not longer than
+    read_len), in growth order, as sv_assembly.contig objects with `.rejected_for` "support" or "length", for every
+    target (an empty list for one not completed), in every form.  The handles' "rejected_contigs" option is set for the
+    call only; the accepted contigs, the target state and the files are the same as without it."""
     if on_capacity not in ("raise", "assemble"):
         raise ValueError("on_capacity must be 'raise' or 'assemble'")
     if not targets:
@@ -239,14 +255,18 @@ def compare_kmers_batch(targets, device=0, ingest="python", write_contigs=False,
     if len(targets) <= max_targets and len(devices) == 1:
         pk, ks, objs = _pack_targets(targets, ingest)
         h = get_handle(devices[0])
-        with batch.long_regions([h], long_regions):
+        with batch.options([h], long_regions=long_regions, rejected_contigs=rejected is not None):
             res = batch.run(h, pk, decode=False)
             rows = batch.region_report_if(h, res, report is not None)
-        _apply_chunk(targets, pk, res, ks, objs, ingest, write_contigs, failed)
+            if rejected is not None:
+                res.rejected = batch.rejected_tables(h)
+        out = _apply_chunk(targets, pk, res, ks, objs, ingest, write_contigs, failed)
+        if rejected is not None:
+            _record_rejected(targets, out, objs, ks, rejected)
         _record_report(targets, rows, failed, reasons, report)
     else:
         _sharded(targets, devices, ingest, write_contigs, max_targets, inflight, failed, apply_thread, long_regions, reasons,
-                 report)
+                 report, rejected)
     if failed:
         raise CapacityError(sorted(failed), reasons)
 
@@ -265,7 +285,7 @@ def _get_pipe(dev, inflight):
 
 
 def _sharded(targets, devices, ingest, write_contigs, max_targets, inflight, failed, apply_thread=False, long_regions=False,
-             reasons=None, report=None):
+             reasons=None, report=None, rejected=None):
     """Chunked, pipelined (and with several devices region-sharded) pass: sv_processor.py:185-201 over `devices`."""
     import threading
     from . import shard
@@ -281,10 +301,12 @@ def _sharded(targets, devices, ingest, write_contigs, max_targets, inflight, fai
     def consume(res, pk, tag):
         chunk, ks, objs, apply_ing = tag
         mine = []
-        _apply_chunk(chunk, pk, res, ks, objs, ingest, write_contigs, mine, apply_ing)
+        out = _apply_chunk(chunk, pk, res, ks, objs, ingest, write_contigs, mine, apply_ing)
         with lock:
             failed.extend(mine)
             _record_report(chunk, getattr(res, "report", None), mine, reasons, report)
+            if rejected is not None:
+                _record_rejected(chunk, out, objs, ks, rejected)
 
     chunks = shard.plan_chunks([_target_cost(t) for t in targets], len(devices), max_targets,
                                key=lambda i: (targets[i].name, i))               # sv_processor.py:175-176
@@ -292,7 +314,7 @@ def _sharded(targets, devices, ingest, write_contigs, max_targets, inflight, fai
     pipe = _get_pipe(devices[0], inflight) if len(devices) == 1 else None
     try:
         shard.drive_chunks(chunks, devices, inflight, pack, consume, pipe, decode=False, long_regions=long_regions,
-                           report=report is not None, apply_thread=apply_thread)
+                           report=report is not None, apply_thread=apply_thread, rejected_contigs=rejected is not None)
     except Exception:
         if pipe is not None:                             # a pipeline with batches in flight is not reusable
             _pipes.pop((threading.get_ident(), devices[0], inflight), None)

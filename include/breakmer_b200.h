@@ -146,6 +146,8 @@ typedef struct bk_batch_input {
  *                  of each unique read in contig.reads
  *   k-mer tuples   ctg_kmer_mer/pos/lth/dist/order  via ctg_kmers_off ; order
  *                  0='for' 1='rev' 2='mid' (sv_assembly.py:130,142)
+ * With the "rejected_contigs" option the ctg_*_off tables also hold, after the n_contigs
+ * accepted contigs, those the acceptance test dropped (bk_rejected_contigs).
  * Unique reads (fq_recs keys, insertion order): region r owns
  * [uniq_reg_off[r], uniq_reg_off[r+1]); uniq_rec = representative record index,
  * uniq_mult = len(fq_recs[seq]). */
@@ -228,7 +230,16 @@ int bk_ref_cache_clear(bk_handle_t h);
  * attempt never appear.  The option is read when the inputs are uploaded (bk_batch_submit with inputs,
  * bk_compare_kmers_batch, bk_batch_upload): a batch in flight or already uploaded keeps the mode it was uploaded
  * with.  It costs device memory per call (scratch of the long assembler, about 11 MB per CTA for at least 4 CTAs)
- * and two small launches; with 0 nothing extra is allocated or launched. */
+ * and two small launches; with 0 nothing extra is allocated or launched.
+ * "rejected_contigs" = 0 | 1 adds to a result the contigs the assembler grows completely and then drops in its
+ * acceptance test (sv_assembly.py:53-59): total read support below rc_thresh, or not longer than read_len.  0
+ * (default): a result holds the accepted contigs only.  1: the rejected contigs are written out exactly as accepted
+ * ones are and follow them in the ctg_*_off tables, at indices n_contigs and up; bk_rejected_contigs tells which
+ * region and reason each one has.  Accepted contigs, n_contigs, ctg_reg_off and the files of bk_write_contigs /
+ * bk_write_sample_kmers are the same either way.  A contig only set up (its first read already used) is never grown or
+ * tested, so it is not one of them, and a region reported as BK_ERR_CAPACITY has none.  Read when the inputs are
+ * uploaded, as "long_regions" is; bk_compare_kmers_long honours it too.  The rejected contigs take room in the
+ * output arena like accepted ones. */
 int bk_set_option(bk_handle_t h, const char* name, int64_t value);
 
 /* ---- per-region report: why a region's assembly stopped and what the assembler did ----------------------------
@@ -281,6 +292,19 @@ int bk_set_option(bk_handle_t h, const char* name, int64_t value);
  * valid until the next call on the handle.  Copied from the device on request (nothing is copied when it
  * is not asked for).  BK_ERR_ARG while a batch is in flight or before any result. */
 int bk_region_report(bk_handle_t h, const int32_t** table, int32_t* n_fields);
+
+/* ---- rejected contigs of the last result (the "rejected_contigs" option) ------------------------------------------
+ * Rejected contig j of region r has j in [reg_off[r], reg_off[r+1]) (n_regions + 1 offsets), in the order the
+ * assembler grew them, and reason[j] = BK_REJ_SUPPORT (its total read support is below rc_thresh, tested first) or
+ * BK_REJ_LENGTH (it is not longer than read_len).  Its sequence, kmer_locs, count vectors, reads and k-mer tuples are
+ * those of contig n_contigs + j of the result's ctg_*_off tables.  For every region with a result,
+ * reg_off[r+1] - reg_off[r] = BK_RR_REJ_SUPPORT + BK_RR_REJ_LENGTH of bk_region_report.  *n = reg_off[n_regions].
+ * The arrays are library-owned host memory, valid until the next call on the handle.  BK_ERR_ARG while a batch is in
+ * flight, before any result, after another call reused the result's memory, and for a result of a batch uploaded with
+ * the option off. */
+#define BK_REJ_SUPPORT 1
+#define BK_REJ_LENGTH 2
+int bk_rejected_contigs(bk_handle_t h, const int64_t** reg_off, const int32_t** reason, int64_t* n);
 
 int bk_compare_kmers_resident(bk_handle_t h, bk_batch_result* out);
 int bk_kernel_times(bk_handle_t h, const char** names, const double** ms, const int64_t** launches, int32_t* n);
