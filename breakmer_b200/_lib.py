@@ -117,6 +117,9 @@ def load():
     lib.bk_ref_cache_clear.argtypes = [H]
     lib.bk_region_report.argtypes = [H, POINTER(POINTER(c_int32)), POINTER(c_int32)]
     lib.bk_rejected_contigs.argtypes = [H, POINTER(POINTER(c_int64)), POINTER(POINTER(c_int32)), POINTER(c_int64)]
+    lib.bk_kmer_report.argtypes = [H, POINTER(POINTER(c_int32)), POINTER(c_int32)]
+    lib.bk_normal_kmers.argtypes = [H, POINTER(POINTER(c_int64)), POINTER(POINTER(c_uint64)), POINTER(POINTER(c_uint32)),
+                                    POINTER(c_int64)]
     lib.bk_ingest_create.argtypes = [c_int, c_int, POINTER(H)]
     lib.bk_ingest_destroy.argtypes = [H]
     lib.bk_ingest_last_error.argtypes = [H]
@@ -134,7 +137,7 @@ def load():
     for name in ("bk_create", "bk_destroy", "bk_nw_batch", "bk_dedup_reads", "bk_count_kmers", "bk_sample_only",
                  "bk_compare_kmers_batch", "bk_compare_kmers_long", "bk_batch_submit", "bk_batch_wait", "bk_batch_upload",
                  "bk_compare_kmers_resident", "bk_kernel_times", "bk_kernel_times_reset", "bk_set_option", "bk_ref_cache_build",
-                 "bk_ref_cache_clear", "bk_region_report", "bk_rejected_contigs"):
+                 "bk_ref_cache_clear", "bk_region_report", "bk_rejected_contigs", "bk_kmer_report", "bk_normal_kmers"):
         getattr(lib, name).restype = c_int
     _lib = lib
     return lib
@@ -144,7 +147,7 @@ EXPORTED_SYMBOLS = (
     "bk_version", "bk_device_count", "bk_create", "bk_destroy", "bk_last_error", "bk_nw_batch", "bk_dedup_reads",
     "bk_count_kmers", "bk_sample_only", "bk_compare_kmers_batch", "bk_compare_kmers_long", "bk_batch_submit", "bk_batch_wait", "bk_batch_upload", "bk_compare_kmers_resident", "bk_kernel_times",
     "bk_kernel_times_reset", "bk_set_option", "bk_ref_cache_build", "bk_ref_cache_clear", "bk_region_report",
-    "bk_rejected_contigs",
+    "bk_rejected_contigs", "bk_kmer_report", "bk_normal_kmers",
     "bk_ingest_create", "bk_ingest_destroy", "bk_ingest_last_error", "bk_ingest_buffers", "bk_ingest_files",
     "bk_write_contigs", "bk_write_sample_kmers")
 
@@ -302,6 +305,32 @@ class Handle:
         off = np.ctypeslib.as_array(reg_off, shape=(int(self.result_regions) + 1,)).copy()
         why = np.ctypeslib.as_array(reason, shape=(n.value,)).copy() if n.value else np.zeros(0, np.int32)
         return off, why
+
+    def kmer_report(self):
+        """bk_kmer_report: where the soft-clip k-mers of every region of the handle's last result went, as an
+        (n_regions, BK_KR_FIELDS) int32 copy (batch.KMER_REPORT_FIELDS).  Read it before the handle's next call."""
+        table, nf = POINTER(c_int32)(), c_int32()
+        self._check(self.lib.bk_kmer_report(self.h, byref(table), byref(nf)))
+        n = self.result_regions
+        if n is None:
+            raise BreakmerError(BK_ERR_ARG, "kmer_report: no result of batch.run / batch.wait on this handle")
+        if n == 0:
+            return np.zeros((0, nf.value), np.int32)
+        return np.ctypeslib.as_array(table, shape=(int(n), nf.value)).copy()
+
+    def normal_kmers(self):
+        """bk_normal_kmers: the k-mers the normal sample removed from the handle's last result (a batch uploaded with the
+        "normal_kmers" option) as copies (reg_off int64[n_regions + 1], mers uint64[n], counts uint32[n]), ascending per
+        region, with their case counts.  Read it before the handle's next call."""
+        reg_off, mers, counts, n = POINTER(c_int64)(), POINTER(c_uint64)(), POINTER(c_uint32)(), c_int64()
+        self._check(self.lib.bk_normal_kmers(self.h, byref(reg_off), byref(mers), byref(counts), byref(n)))
+        if self.result_regions is None:
+            raise BreakmerError(BK_ERR_ARG, "normal_kmers: no result of batch.run / batch.wait on this handle")
+        off = np.ctypeslib.as_array(reg_off, shape=(int(self.result_regions) + 1,)).copy()
+        if not n.value:
+            return off, np.zeros(0, np.uint64), np.zeros(0, np.uint32)
+        return (off, np.ctypeslib.as_array(mers, shape=(n.value,)).copy(),
+                np.ctypeslib.as_array(counts, shape=(n.value,)).copy())
 
     # ---- timers -------------------------------------------------------------------------
     def kernel_times_reset(self, enable=True):

@@ -117,10 +117,12 @@ def _arr(ptr, n, dtype):
 
 class BatchOutput:
     """Copies of the library-owned result arrays of one call.  `rejected`: the call's rejected_tables, or None; with them
-    the contig tables also hold the rejected contigs, after the n_contigs accepted ones."""
+    the contig tables also hold the rejected contigs, after the n_contigs accepted ones.  `normal`: the call's
+    normal_kmer_tables, or None."""
 
-    def __init__(self, res, packed, rejected=None):
+    def __init__(self, res, packed, rejected=None, normal=None):
         R = res.n_regions
+        self.normal = normal                  # the call's normal_kmer_tables, or None
         C = int(res.n_contigs)
         self.rej_reg_off, self.rej_reason = rejected if rejected is not None else (None, None)
         n_all = C + (len(self.rej_reason) if rejected is not None else 0)
@@ -170,6 +172,15 @@ class BatchOutput:
     def sample_only(self, r):
         a, b = int(self.so_off[r]), int(self.so_off[r + 1])
         return dict(zip(_lib.codes_to_mers(self.so_mers[a:b], self.k), self.so_counts[a:b].tolist()))
+
+    def normal_kmers(self, r):
+        """{mer: case count} of the k-mers the normal sample removed from region r (the shape of sample_only(r)); ValueError
+        for a result made without the "normal_kmers" option"""
+        if self.normal is None:
+            raise ValueError("normal k-mers: the result was made without the \"normal_kmers\" option")
+        off, mers, counts = self.normal
+        a, b = int(off[r]), int(off[r + 1])
+        return dict(zip(_lib.codes_to_mers(mers[a:b], self.k), counts[a:b].tolist()))
 
     def _kmer_strings(self):
         if self._kmer_str is None:                      # all contig k-mers of the batch decoded at once
@@ -229,6 +240,17 @@ def rejected_tables(handle):
         return None
 
 
+def normal_kmer_tables(handle):
+    """Handle.normal_kmers() of the handle's last result, or None when that result was made without them (its batch was
+    uploaded with the "normal_kmers" option off, or had no k-mer stage).  Read it before the handle's next call."""
+    try:
+        return handle.normal_kmers()
+    except _lib.BreakmerError as e:
+        if e.code != _lib.BK_ERR_ARG:
+            raise
+        return None
+
+
 def run(handle, packed, resident=False, decode=True, long=False):
     """bk_compare_kmers_batch (or the resident variant after `upload`).  long=True: bk_compare_kmers_long, for regions
     with reads or contigs above MAX_LEN (up to LONG_MAX_LEN) bases, which the batched call reports as BK_ERR_CAPACITY."""
@@ -246,12 +268,13 @@ def run(handle, packed, resident=False, decode=True, long=False):
     handle.result_regions = res.n_regions
     if not decode:
         return res
-    return BatchOutput(res, packed, rejected_tables(handle))
+    return BatchOutput(res, packed, rejected_tables(handle), normal_kmer_tables(handle))
 
 
 @contextlib.contextmanager
 def options(handles, **on):
-    """The handles' 0 | 1 options named with a true value (e.g. long_regions=True, rejected_contigs=True) set to 1 for
+    """The handles' 0 | 1 options named with a true value (e.g. long_regions=True, rejected_contigs=True,
+    normal_kmers=True) set to 1 for
     the duration of a call, then 0 (the default) again, so that later calls on handles the caller shares get the default
     behaviour.  Options given a false value are left untouched.  Closed handles are skipped."""
     names = [name for name, value in on.items() if value]
@@ -295,6 +318,17 @@ def region_report(handle):
     return out
 
 
+# bk_kmer_report (include/breakmer_b200.h): the BK_KR_* fields in column order
+KMER_REPORT_FIELDS = ("soft_clip", "not_in_reads", "in_reference", "in_normal", "sample_only")
+
+
+def kmer_report(handle):
+    """Where the soft-clip k-mers of each region of the handle's last result (run / wait) went (bk_kmer_report): one
+    dict per region with the KMER_REPORT_FIELDS as keys, counts of distinct k-mers; soft_clip = not_in_reads +
+    in_reference + in_normal + sample_only.  Read it before the handle's next call."""
+    return [dict(zip(KMER_REPORT_FIELDS, row)) for row in handle.kmer_report().tolist()]
+
+
 def any_failed(res):
     """True if some region of a result (BatchOutput, or the BatchResult of decode=False) has a nonzero status."""
     if isinstance(res, BatchOutput):
@@ -326,7 +360,7 @@ def wait(handle, packed=None, decode=True):
     handle.result_regions = res.n_regions
     if not decode:
         return res
-    return BatchOutput(res, packed, rejected_tables(handle))
+    return BatchOutput(res, packed, rejected_tables(handle), normal_kmer_tables(handle))
 
 
 def upload(handle, packed):

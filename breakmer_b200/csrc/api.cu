@@ -28,6 +28,7 @@ struct bk_handle_s {
   int spec_width = 0;      // assembler speculation width (bk_set_option); 0 = choose per batch
   int long_regions = 0;    // bk_set_option "long_regions": the batched entries also assemble regions up to 65,535 bases
   int rejected_contigs = 0;  // bk_set_option "rejected_contigs": results also hold the contigs the acceptance test drops
+  int normal_kmers = 0;    // bk_set_option "normal_kmers": results also hold the k-mers the normal sample removed
   cudaEvent_t sync_ev = nullptr;   // blocking-sync event (BK_BLOCKING_SYNC=1)
   bool spin_sync = true;
   Arena<false> dev;        // per-call device scratch
@@ -626,6 +627,9 @@ int bk_set_option(bk_handle_t h, const char* name, int64_t value) {
     } else if (strcmp(name, "rejected_contigs") == 0) {
       if (value != 0 && value != 1) fail(BK_ERR_ARG, "rejected_contigs must be 0 or 1");
       h->rejected_contigs = (int)value;
+    } else if (strcmp(name, "normal_kmers") == 0) {
+      if (value != 0 && value != 1) fail(BK_ERR_ARG, "normal_kmers must be 0 or 1");
+      h->normal_kmers = (int)value;
     } else {
       fail(BK_ERR_ARG, "bk_set_option: unknown option %s", name);
     }
@@ -658,6 +662,25 @@ int bk_rejected_contigs(bk_handle_t h, const int64_t** reg_off, const int32_t** 
   return guarded(h, [&] {
     if (!reg_off || !reason || !n) fail(BK_ERR_ARG, "bk_rejected_contigs: null argument");
     rejected_contigs(h, reg_off, reason, n);
+  });
+}
+
+static_assert(KR_SOFT_CLIP == BK_KR_SOFT_CLIP && KR_NOT_IN_READS == BK_KR_NOT_IN_READS && KR_IN_REFERENCE == BK_KR_IN_REFERENCE &&
+                  KR_IN_NORMAL == BK_KR_IN_NORMAL && KR_SAMPLE_ONLY == BK_KR_SAMPLE_ONLY && KR_FIELDS == BK_KR_FIELDS,
+              "k-mer report fields of region_kmers.cuh and include/breakmer_b200.h differ");
+
+int bk_kmer_report(bk_handle_t h, const int32_t** table, int32_t* n_fields) {
+  return guarded(h, [&] {
+    if (!table || !n_fields) fail(BK_ERR_ARG, "bk_kmer_report: null argument");
+    *table = kmer_report(h);
+    *n_fields = KR_FIELDS;
+  });
+}
+
+int bk_normal_kmers(bk_handle_t h, const int64_t** reg_off, const uint64_t** mers, const uint32_t** counts, int64_t* n) {
+  return guarded(h, [&] {
+    if (!reg_off || !mers || !counts || !n) fail(BK_ERR_ARG, "bk_normal_kmers: null argument");
+    normal_kmers(h, reg_off, mers, counts, n);
   });
 }
 

@@ -69,6 +69,7 @@ struct Pipeline {
   // the long modes, assemble_long_kernel takes the others and those assemble_kernel stopped
   LongMode long_mode = LONG_OFF;
   bool keep_rejected = false;             // the "rejected_contigs" option, fixed at upload like long_mode
+  bool keep_normal = false;               // the "normal_kmers" option, fixed at upload like long_mode
   int n_short = 0;                        // LONG_OFF: all; LONG_ROUTE: those without a read above NW_MAX_LEN; LONG_ALL: 0
   const uint8_t* d_routed = nullptr;      // device, per region: a read above NW_MAX_LEN (LONG_ROUTE; null when none)
   int max_short_read_len = 0;             // longest read of the other regions (sizes assemble_kernel's read buffers)
@@ -129,6 +130,16 @@ struct PendingBatch {
   bool keep_rejected = false;
   std::vector<int64_t> rej_reg_off;
   std::vector<int32_t> rej_reason;
+  // the k-mer stage's report and, with the "normal_kmers" option (keep_normal), the k-mers the normal sample removed
+  // (bk_kmer_report, bk_normal_kmers): device tables of the result, copied on request.  kmer_stage: the batch ran the
+  // k-mer stage (have_mers = 0); kmer_report null: no region reached region_kmer_kernel (every row is 0)
+  bool kmer_stage = false, keep_normal = false;
+  const int32_t* kmer_report = nullptr;
+  const int64_t* nm_off = nullptr; const uint64_t* nm_mer = nullptr; const uint32_t* nm_cnt = nullptr;
+  std::vector<int32_t> h_kmer_report;      // host copies, made on request
+  std::vector<int64_t> h_nm_off;
+  std::vector<uint64_t> h_nm_mer;
+  std::vector<uint32_t> h_nm_cnt;
 };
 
 }  // namespace bk

@@ -77,6 +77,7 @@ void pipeline_upload_into(bk_handle_t h, Arena<false>& A, const bk_batch_input* 
   p = Pipeline();
   p.long_mode = mode;
   p.keep_rejected = h->rejected_contigs != 0;
+  p.keep_normal = h->normal_kmers != 0;
   const int max_len = mode == LONG_OFF ? NW_MAX_LEN : ASM_LONG_MAX_LEN;
   if (in->n_regions < 0 || in->n_regions > 65535) fail(BK_ERR_ARG, "batch: n_regions must be in 0..65535 per call");
   if (in->k < 2 || in->k > 31) fail(BK_ERR_ARG, "batch: k must be in 2..31");
@@ -399,9 +400,9 @@ void pipeline_submit(bk_handle_t h, const bk_batch_input* in, LongMode mode) {
   const int k = p.k;
   if (p.reads.n_bases >= (int64_t(1) << 31) || p.n_in_mers >= (int64_t(1) << 31))
     fail(BK_ERR_CAPACITY, "batch: more than 2^31 read bases or k-mers in one call; use fewer regions per call");
-  uint32_t* d_counts = dev_zero<uint32_t>(h, 4);         // [0] unique reads, [1] sample-only k-mers, [2] postings
+  uint32_t* d_counts = dev_zero<uint32_t>(h, 4);   // [0] unique reads, [1] sample-only k-mers, [2] postings, [3] normal k-mers
   B.d_counts = d_counts;
-  uint32_t* d_NU = d_counts, *d_S = d_counts + 1, *d_npost = d_counts + 2;
+  uint32_t* d_NU = d_counts, *d_S = d_counts + 1, *d_npost = d_counts + 2, *d_N = d_counts + 3;
 
   // field widths of the packed sort keys, from bounds the input offsets give (no device round trip)
   const int s_bits = std::max(1, bits_for((uint64_t)std::max<int64_t>(1, p.max_reg_mers)));
@@ -469,9 +470,12 @@ void pipeline_submit(bk_handle_t h, const bk_batch_input* in, LongMode mode) {
     uint64_t* all_m = h->dev.get<uint64_t>(SB ? SB : 1);
     uint32_t* all_c = h->dev.get<uint32_t>(SB ? SB : 1);
     uint32_t* seg_counts = dev_zero<uint32_t>(h, (size_t)R + 1);
-    if (R > 0 && SB > 0) {
+    B.kmer_stage = true;
+    B.keep_normal = p.keep_normal;
+    int64_t* nm_off = p.keep_normal ? h->dev.get<int64_t>(R + 1) : nullptr;
+    if (R > 0 && p.sc.n_bases > 0) {
       // one CTA per region: shared-memory hash table of its soft-clip k-mers, reads counted into it, reference and
-      // normal windows streamed past it (region_kmers.cuh)
+      // normal windows streamed past it (region_kmers.cuh).  It runs without reads too: the report counts the candidates.
       RegionKmerParams K{};
       K.n_regions = R; K.k = k;
       auto view = [](const RecordSet& rs) { return RkSet{rs.n_bases > 0 ? rs.bases : nullptr, rs.koff, rs.d_reg_base, rs.d_reg_krec}; };
@@ -483,6 +487,12 @@ void pipeline_submit(bk_handle_t h, const bk_batch_input* in, LongMode mode) {
       K.gcnt = h->dev.get<uint32_t>(p.rk_gtab_slots ? p.rk_gtab_slots : 1);
       K.st_mer = h->dev.get<uint64_t>(p.sc.n_bases); K.st_cnt = h->dev.get<uint32_t>(p.sc.n_bases);
       K.seg_counts = seg_counts;
+      K.kmer_report = h->dev.get<int32_t>((size_t)R * KR_FIELDS);
+      B.kmer_report = K.kmer_report;
+      if (p.keep_normal) {                                 // a second staging slice, sorted and compacted the same way
+        K.nm_mer = h->dev.get<uint64_t>(p.sc.n_bases); K.nm_cnt = h->dev.get<uint32_t>(p.sc.n_bases);
+        K.nm_counts = h->dev.get<uint32_t>((size_t)R + 1);
+      }
       const size_t smem = (size_t)K.smem_cap * 12 + RK_TILE + 64;
       const int per_sm = std::max<int>(1, (int)((220 * 1024) / (smem + 1024)));
       const int grid_k = (int)std::min<int64_t>(R, (int64_t)h->sm_count * std::min(per_sm, 4) * 2);
@@ -493,22 +503,39 @@ void pipeline_submit(bk_handle_t h, const bk_batch_input* in, LongMode mode) {
         region_kmer_kernel<<<grid_k, RK_THREADS, smem, st>>>(K);
         BK_CUDA(cudaGetLastError());
       }
-      uint32_t* seg_excl = h->dev.get<uint32_t>(R + 1);
-      uint32_t* stmp = h->dev.get<uint32_t>(scan_tmp_elems(R));
-      {
-        TimedLaunch t(h->timers, st, KF_SCAN, 4);
-        exclusive_scan_u32(seg_counts, seg_excl, R, stmp, d_S, st);
-        widen_scan_kernel<<<nblk(R + 1, 256), 256, 0, st>>>(seg_excl, d_S, R, so_off);
+      // the per-region counts -> offsets, and the staged k-mers -> dense arrays at those offsets
+      auto compact = [&](const uint32_t* counts, uint32_t* d_total, int64_t* off, const uint64_t* st_m, const uint32_t* st_c,
+                         uint64_t* m, uint32_t* c) {
+        if (SB == 0) {                                     // no reads in the batch: no region has any
+          BK_CUDA(cudaMemsetAsync(off, 0, (R + 1) * sizeof(int64_t), st));
+          return;
+        }
+        uint32_t* excl = h->dev.get<uint32_t>(R + 1);
+        uint32_t* stmp = h->dev.get<uint32_t>(scan_tmp_elems(R));
+        {
+          TimedLaunch t(h->timers, st, KF_SCAN, 4);
+          exclusive_scan_u32(counts, excl, R, stmp, d_total, st);
+          widen_scan_kernel<<<nblk(R + 1, 256), 256, 0, st>>>(excl, d_total, R, off);
+        }
+        {
+          TimedLaunch t(h->timers, st, KF_REGION_KMERS);
+          region_compact_kernel<<<(unsigned)std::min<int64_t>(R, (int64_t)h->sm_count * 16), 256, 0, st>>>(st_m, st_c, p.sc.d_reg_base, off, R,
+                                                                                                         m, c);
+        }
+        BK_CUDA(cudaGetLastError());
+      };
+      compact(seg_counts, d_S, so_off, K.st_mer, K.st_cnt, all_m, all_c);
+      if (p.keep_normal) {
+        uint64_t* nm_m = h->dev.get<uint64_t>(SB ? SB : 1);   // (every one is a k-mer of the reads, as a sample-only one is)
+        uint32_t* nm_c = h->dev.get<uint32_t>(SB ? SB : 1);
+        compact(K.nm_counts, d_N, nm_off, K.nm_mer, K.nm_cnt, nm_m, nm_c);
+        B.nm_mer = nm_m; B.nm_cnt = nm_c;
       }
-      {
-        TimedLaunch t(h->timers, st, KF_REGION_KMERS);
-        region_compact_kernel<<<(unsigned)std::min<int64_t>(R, (int64_t)h->sm_count * 16), 256, 0, st>>>(K.st_mer, K.st_cnt, p.sc.d_reg_base, so_off, R,
-                                                                                                       all_m, all_c);
-      }
-      BK_CUDA(cudaGetLastError());
     } else {
       BK_CUDA(cudaMemsetAsync(so_off, 0, (R + 1) * sizeof(int64_t), st));
+      if (p.keep_normal) BK_CUDA(cudaMemsetAsync(nm_off, 0, (R + 1) * sizeof(int64_t), st));
     }
+    B.nm_off = nm_off;
     so_mer = all_m; so_cnt = all_c;
   }
 
@@ -841,6 +868,53 @@ void rejected_contigs(bk_handle_t h, const int64_t** reg_off, const int32_t** re
   *reg_off = B.rej_reg_off.data();
   *reason = B.rej_reason.empty() ? nullptr : B.rej_reason.data();
   *n = (int64_t)B.rej_reason.size();
+}
+
+// the refusals bk_kmer_report and bk_normal_kmers share: a batch in flight, no result (or its memory reused), a result
+// without a k-mer stage (have_mers)
+void check_kmer_stage_result(bk_handle_t h, const char* what) {
+  const PendingBatch& B = h->pending;
+  if (B.active) fail(BK_ERR_ARG, "%s: a batch is in flight on this handle (call bk_batch_wait first)", what);
+  if (!B.has_result || B.result_epoch != h->dev.resets()) fail(BK_ERR_ARG, "%s: no result on this handle", what);
+  if (!B.kmer_stage) fail(BK_ERR_ARG, "%s: the last result was given its sample-only k-mers (have_mers): no k-mer stage ran", what);
+}
+
+// bk_kmer_report: the k-mer stage's report of the last result; regions left out at upload get an all-zero row
+const int32_t* kmer_report(bk_handle_t h) {
+  check_kmer_stage_result(h, "bk_kmer_report");
+  PendingBatch& B = h->pending;
+  const int R = B.A.n_regions;
+  B.h_kmer_report.assign((size_t)(R ? R : 1) * KR_FIELDS, 0);
+  if (R && B.kmer_report) {
+    BK_CUDA(cudaMemcpyAsync(B.h_kmer_report.data(), B.kmer_report, (size_t)R * KR_FIELDS * sizeof(int32_t), cudaMemcpyDeviceToHost, h->st));
+    BK_CUDA(stream_wait(h));
+  }
+  for (int r = 0; r < (int)B.report_skipped.size(); ++r)
+    if (B.report_skipped[r]) std::fill_n(B.h_kmer_report.data() + (size_t)r * KR_FIELDS, KR_FIELDS, 0);
+  return B.h_kmer_report.data();
+}
+
+// bk_normal_kmers: the k-mers the normal sample removed from the last result (the "normal_kmers" option)
+void normal_kmers(bk_handle_t h, const int64_t** reg_off, const uint64_t** mers, const uint32_t** counts, int64_t* n) {
+  check_kmer_stage_result(h, "bk_normal_kmers");
+  PendingBatch& B = h->pending;
+  if (!B.keep_normal) fail(BK_ERR_ARG, "bk_normal_kmers: the last result was made with the \"normal_kmers\" option off");
+  const int R = B.A.n_regions;
+  B.h_nm_off.assign((size_t)R + 1, 0);
+  BK_CUDA(cudaMemcpyAsync(B.h_nm_off.data(), B.nm_off, ((size_t)R + 1) * sizeof(int64_t), cudaMemcpyDeviceToHost, h->st));
+  BK_CUDA(stream_wait(h));
+  const int64_t total = B.h_nm_off[R];
+  B.h_nm_mer.assign((size_t)(total ? total : 1), 0);
+  B.h_nm_cnt.assign((size_t)(total ? total : 1), 0);
+  if (total) {
+    BK_CUDA(cudaMemcpyAsync(B.h_nm_mer.data(), B.nm_mer, (size_t)total * sizeof(uint64_t), cudaMemcpyDeviceToHost, h->st));
+    BK_CUDA(cudaMemcpyAsync(B.h_nm_cnt.data(), B.nm_cnt, (size_t)total * sizeof(uint32_t), cudaMemcpyDeviceToHost, h->st));
+    BK_CUDA(stream_wait(h));
+  }
+  *reg_off = B.h_nm_off.data();
+  *mers = B.h_nm_mer.data();
+  *counts = B.h_nm_cnt.data();
+  *n = total;
 }
 
 void phase_print(bk_handle_t h, const PendingBatch& B) {

@@ -155,9 +155,10 @@ class DevicePipeline:
     """`inflight` handles of one device driven by ONE host thread: submit keeps up to `inflight` batches queued on the
     device (bk_batch_submit), results come back in submission order (bk_batch_wait).  long_regions=True sets the
     handles' "long_regions" option: regions with reads or contigs up to 65,535 bases are assembled in the same pass.
-    rejected_contigs=True sets the option of that name: results also hold the contigs the acceptance test drops."""
+    rejected_contigs=True sets the option of that name: results also hold the contigs the acceptance test drops.
+    normal_kmers=True sets the option of that name: results also hold the k-mers the normal sample removed."""
 
-    def __init__(self, device, inflight=3, spec_width=0, long_regions=False, rejected_contigs=False):
+    def __init__(self, device, inflight=3, spec_width=0, long_regions=False, rejected_contigs=False, normal_kmers=False):
         from . import _lib
         self.device = device
         self.handles = [_lib.Handle(device) for _ in range(max(1, inflight))]
@@ -169,8 +170,11 @@ class DevicePipeline:
                 h.set_option("long_regions", 1)
             if rejected_contigs:
                 h.set_option("rejected_contigs", 1)
+            if normal_kmers:
+                h.set_option("normal_kmers", 1)
         self._queue = []                               # (handle index, packed, tag) in submission order
         self.report = False                            # pop: read every batch's per-region report
+        self.kmer_report = False                       # pop: read every batch's k-mer stage report
         self._next = 0
 
     def full(self):
@@ -189,13 +193,17 @@ class DevicePipeline:
         """-> (result of the oldest batch in flight, its packed input, its tag).  The result's `.report` is the batch's
         batch.region_report, read before its handle takes another batch, if `self.report` is set or a region of the
         batch failed; else None.  With decode=False its `.rejected` is the batch's batch.rejected_tables (None unless the
-        batch was submitted with the "rejected_contigs" option); a decoded result holds them already."""
+        batch was submitted with the "rejected_contigs" option); a decoded result holds them already.  So is `.normal`
+        the batch's batch.normal_kmer_tables.  `.kmer_report` is the batch's batch.kmer_report if `self.kmer_report` is
+        set, else None."""
         from . import batch
         j, packed, tag = self._queue.pop(0)
         res = batch.wait(self.handles[j], packed, decode=decode)
         res.report = batch.region_report_if(self.handles[j], res, self.report)
+        res.kmer_report = batch.kmer_report(self.handles[j]) if self.kmer_report else None
         if not decode:
             res.rejected = batch.rejected_tables(self.handles[j])
+            res.normal = batch.normal_kmer_tables(self.handles[j])
         return res, packed, tag
 
     def pending(self):
@@ -220,13 +228,13 @@ def plan_chunks(costs, n_devices, max_per_chunk, key=None):
 
 
 def drive_chunks(chunks, devices, inflight, pack, consume, pipe=None, decode=True, long_regions=False, report=False,
-                 apply_thread=False, rejected_contigs=False):
+                 apply_thread=False, rejected_contigs=False, kmer_report=False, normal_kmers=False):
     """Run `chunks` (lists of indices) on `devices`, each device taking the next chunk when it has room for it.
     pack(indices, slot) -> (packed, tag) parses a chunk into parse buffer `slot`; consume(result, packed, tag) takes the
     finished batches (pipe.pop(decode)), per device in submission order.  `pipe`: an open pipeline of devices[0], driven
     on the calling thread and left open; without it every device gets a thread and an `inflight`-handle DevicePipeline of
-    its own, closed at the end.  long_regions, rejected_contigs and report set the handles' options and
-    DevicePipeline.report for the call.
+    its own, closed at the end.  long_regions, rejected_contigs and normal_kmers set the handles' options, report and
+    kmer_report DevicePipeline.report and .kmer_report, for the call.
 
     Without apply_thread a device's thread pops the oldest batch of a full pipeline before it parses the next chunk, and
     one parse slot per handle rotates.  With apply_thread a second thread pops and consumes while the first parses ahead,
@@ -259,7 +267,9 @@ def drive_chunks(chunks, devices, inflight, pack, consume, pipe=None, decode=Tru
                 free.release()
 
         pipe.report = report
-        with batch.options(pipe.handles, long_regions=long_regions, rejected_contigs=rejected_contigs):
+        pipe.kmer_report = kmer_report
+        with batch.options(pipe.handles, long_regions=long_regions, rejected_contigs=rejected_contigs,
+                           normal_kmers=normal_kmers):
             if apply_thread:
                 helper = threading.Thread(target=applier)
                 helper.start()

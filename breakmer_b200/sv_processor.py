@@ -40,6 +40,8 @@ same device pass as all others (the handles' "long_regions" option).
 assembled it, how many seeds, find_reads and check_align calls, and how many contigs were grown and rejected).
 `rejected={}` is filled with the contigs themselves that the assembler grew and then rejected, per target (the handles'
 "rejected_contigs" option).
+`kmer_report={}` is filled with where every target's soft-clip k-mers went in the k-mer stage (batch.kmer_report), and
+`normal_kmers={}` with the k-mers the normal sample removed from each target (the handles' "normal_kmers" option).
 """
 import os
 
@@ -142,7 +144,7 @@ def _apply_chunk(targets, pk, res, inputs_k, objs, ingest, write_contigs, failed
                               [p[:-4] + "_merged.out" if st == 0 else None for p, st in zip(sk_paths, status)])
         # the "<mer>\t<count>" files of the completed targets in one multi-threaded sweep (bk_write_sample_kmers)
         ing.write_sample_kmers(res, pk.k, sk_paths if all_ok else [p if st == 0 else None for p, st in zip(sk_paths, status)])
-    out = batch.BatchOutput(res, pk, getattr(res, "rejected", None))
+    out = batch.BatchOutput(res, pk, getattr(res, "rejected", None), getattr(res, "normal", None))
     ctg_reg_off = out.ctg_reg_off.tolist()
     so_off = out.so_off.tolist()
     for i, trgt in enumerate(targets):
@@ -171,6 +173,16 @@ def _record_rejected(targets, out, objs, inputs_k, rejected):
     """rejected[name] = the rejected contigs of every target of one device call (out: its BatchOutput)"""
     for i, trgt in enumerate(targets):
         rejected[trgt.name] = rejected_contigs(out, i, objs, inputs_k[i])
+
+
+def _record_kmer_stage(targets, out, rows, kmer_report, normal_kmers):
+    """kmer_report[name] and normal_kmers[name] of every target of one device call (out: its BatchOutput, rows: its
+    batch.kmer_report), for the dicts that are wanted"""
+    for i, trgt in enumerate(targets):
+        if kmer_report is not None:
+            kmer_report[trgt.name] = rows[i]
+        if normal_kmers is not None:
+            normal_kmers[trgt.name] = out.normal_kmers(i)
 
 
 def _record_report(targets, rows, failed, reasons, report):
@@ -211,7 +223,8 @@ def _pack_targets(targets, ingest, slot=0):
 
 
 def compare_kmers_batch(targets, device=0, ingest="python", write_contigs=False, devices=None, max_targets=125, inflight=4,
-                        apply_thread=False, on_capacity="raise", report=None, rejected=None):
+                        apply_thread=False, on_capacity="raise", report=None, rejected=None, kmer_report=None,
+                        normal_kmers=None):
     """target.compare_kmers() for many targets (the region loop of sv_processor.py:185-201 as one call).
 
     The targets are cut into chunks of at most max_targets, most expensive first (static cost, breakmer_b200.shard), and
@@ -240,7 +253,14 @@ def compare_kmers_batch(targets, device=0, ingest="python", write_contigs=False,
     in its acceptance test (sv_assembly.py:53-59: total read support below the min sr_thresh, or not longer than
     read_len), in growth order, as sv_assembly.contig objects with `.rejected_for` "support" or "length", for every
     target (an empty list for one not completed), in every form.  The handles' "rejected_contigs" option is set for the
-    call only; the accepted contigs, the target state and the files are the same as without it."""
+    call only; the accepted contigs, the target state and the files are the same as without it.
+
+    `kmer_report`, a dict, receives kmer_report[target.name] = batch.kmer_report's dict of the target: how many distinct
+    soft-clip k-mers it had, and how many of them the reads lacked, the reference held, the normal sample held, and were
+    left as sample-only k-mers.  `normal_kmers`, a dict, receives normal_kmers[target.name] = {mer: case count} of the
+    k-mers the normal sample removed (files['normal_fq']; empty without one), the entries the sample-only file would
+    have held without the normal sample.  Both are filled for every target, in every form; the handles' "normal_kmers"
+    option is set for the call only, and the target state and the files are the same as without it."""
     if on_capacity not in ("raise", "assemble"):
         raise ValueError("on_capacity must be 'raise' or 'assemble'")
     if not targets:
@@ -255,18 +275,23 @@ def compare_kmers_batch(targets, device=0, ingest="python", write_contigs=False,
     if len(targets) <= max_targets and len(devices) == 1:
         pk, ks, objs = _pack_targets(targets, ingest)
         h = get_handle(devices[0])
-        with batch.options([h], long_regions=long_regions, rejected_contigs=rejected is not None):
+        with batch.options([h], long_regions=long_regions, rejected_contigs=rejected is not None,
+                           normal_kmers=normal_kmers is not None):
             res = batch.run(h, pk, decode=False)
             rows = batch.region_report_if(h, res, report is not None)
             if rejected is not None:
                 res.rejected = batch.rejected_tables(h)
+            if normal_kmers is not None:
+                res.normal = batch.normal_kmer_tables(h)
+            kr_rows = batch.kmer_report(h) if kmer_report is not None else None
         out = _apply_chunk(targets, pk, res, ks, objs, ingest, write_contigs, failed)
         if rejected is not None:
             _record_rejected(targets, out, objs, ks, rejected)
+        _record_kmer_stage(targets, out, kr_rows, kmer_report, normal_kmers)
         _record_report(targets, rows, failed, reasons, report)
     else:
         _sharded(targets, devices, ingest, write_contigs, max_targets, inflight, failed, apply_thread, long_regions, reasons,
-                 report, rejected)
+                 report, rejected, kmer_report, normal_kmers)
     if failed:
         raise CapacityError(sorted(failed), reasons)
 
@@ -285,7 +310,7 @@ def _get_pipe(dev, inflight):
 
 
 def _sharded(targets, devices, ingest, write_contigs, max_targets, inflight, failed, apply_thread=False, long_regions=False,
-             reasons=None, report=None, rejected=None):
+             reasons=None, report=None, rejected=None, kmer_report=None, normal_kmers=None):
     """Chunked, pipelined (and with several devices region-sharded) pass: sv_processor.py:185-201 over `devices`."""
     import threading
     from . import shard
@@ -307,6 +332,7 @@ def _sharded(targets, devices, ingest, write_contigs, max_targets, inflight, fai
             _record_report(chunk, getattr(res, "report", None), mine, reasons, report)
             if rejected is not None:
                 _record_rejected(chunk, out, objs, ks, rejected)
+            _record_kmer_stage(chunk, out, getattr(res, "kmer_report", None), kmer_report, normal_kmers)
 
     chunks = shard.plan_chunks([_target_cost(t) for t in targets], len(devices), max_targets,
                                key=lambda i: (targets[i].name, i))               # sv_processor.py:175-176
@@ -314,7 +340,8 @@ def _sharded(targets, devices, ingest, write_contigs, max_targets, inflight, fai
     pipe = _get_pipe(devices[0], inflight) if len(devices) == 1 else None
     try:
         shard.drive_chunks(chunks, devices, inflight, pack, consume, pipe, decode=False, long_regions=long_regions,
-                           report=report is not None, apply_thread=apply_thread, rejected_contigs=rejected is not None)
+                           report=report is not None, apply_thread=apply_thread, rejected_contigs=rejected is not None,
+                           kmer_report=kmer_report is not None, normal_kmers=normal_kmers is not None)
     except Exception:
         if pipe is not None:                             # a pipeline with batches in flight is not reusable
             _pipes.pop((threading.get_ident(), devices[0], inflight), None)

@@ -239,7 +239,10 @@ int bk_ref_cache_clear(bk_handle_t h);
  * bk_write_sample_kmers are the same either way.  A contig only set up (its first read already used) is never grown or
  * tested, so it is not one of them, and a region reported as BK_ERR_CAPACITY has none.  Read when the inputs are
  * uploaded, as "long_regions" is; bk_compare_kmers_long honours it too.  The rejected contigs take room in the
- * output arena like accepted ones. */
+ * output arena like accepted ones.
+ * "normal_kmers" = 0 | 1: 1 makes the k-mer stage also return the k-mers the normal sample removed (bk_normal_kmers).
+ * Read when the inputs are uploaded, as "long_regions" is; bk_compare_kmers_long honours it too.  The result is the
+ * same either way; with 0 nothing extra is allocated, launched or copied. */
 int bk_set_option(bk_handle_t h, const char* name, int64_t value);
 
 /* ---- per-region report: why a region's assembly stopped and what the assembler did ----------------------------
@@ -305,6 +308,36 @@ int bk_region_report(bk_handle_t h, const int32_t** table, int32_t* n_fields);
 #define BK_REJ_SUPPORT 1
 #define BK_REJ_LENGTH 2
 int bk_rejected_contigs(bk_handle_t h, const int64_t** reg_off, const int32_t** reason, int64_t* n);
+
+/* ---- per-region report of the k-mer stage: where the soft-clip k-mers went ------------------------------------------
+ * One row of BK_KR_FIELDS int32 per region, in the order of the call's regions.  Counts of distinct k-mers, in the
+ * order of the reference's set operations ((case & case_sc) - ref, then the normal sample's k-mers):
+ *   BK_KR_SOFT_CLIP      valid soft-clip k-mers: the candidates
+ *   BK_KR_NOT_IN_READS   of those, the ones no read holds (dropped by case & case_sc)
+ *   BK_KR_IN_REFERENCE   of the others, the ones the reference window holds on either strand (or the handle's
+ *                        reference k-mer cache)
+ *   BK_KR_IN_NORMAL      of the rest, the ones the normal sample holds (0 without a normal sample)
+ *   BK_KR_SAMPLE_ONLY    the sample-only k-mers: so_off[r+1] - so_off[r]
+ * BK_KR_SOFT_CLIP = BK_KR_NOT_IN_READS + BK_KR_IN_REFERENCE + BK_KR_IN_NORMAL + BK_KR_SAMPLE_ONLY.  A region without
+ * soft-clip bases, and a region left out at upload (bk_region_report says why), has an all-zero row.  The table is
+ * library-owned, valid until the next call on the handle, and copied from the device only when asked for.  BK_ERR_ARG
+ * while a batch is in flight, before any result, after another call reused the result's memory, and for a result whose
+ * k-mer stage did not run (have_mers = 1). */
+#define BK_KR_SOFT_CLIP 0
+#define BK_KR_NOT_IN_READS 1
+#define BK_KR_IN_REFERENCE 2
+#define BK_KR_IN_NORMAL 3
+#define BK_KR_SAMPLE_ONLY 4
+#define BK_KR_FIELDS 5
+int bk_kmer_report(bk_handle_t h, const int32_t** table, int32_t* n_fields);
+
+/* ---- the k-mers the normal sample removed (the "normal_kmers" option) ---------------------------------------------
+ * Region r owns [reg_off[r], reg_off[r+1]) of mers / counts (n_regions + 1 offsets; *n = reg_off[n_regions]): the
+ * k-mers counted in BK_KR_IN_NORMAL, in ascending 2-bit order (A<C<G<T), each with its case count -- the entries the
+ * sample-only table would hold had no normal sample been given.  The arrays are library-owned host memory, valid until
+ * the next call on the handle.  BK_ERR_ARG in the cases bk_kmer_report refuses, and for a result of a batch uploaded
+ * with the option off. */
+int bk_normal_kmers(bk_handle_t h, const int64_t** reg_off, const uint64_t** mers, const uint32_t** counts, int64_t* n);
 
 int bk_compare_kmers_resident(bk_handle_t h, bk_batch_result* out);
 int bk_kernel_times(bk_handle_t h, const char** names, const double** ms, const int64_t** launches, int32_t* n);
